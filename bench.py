@@ -3,7 +3,7 @@
 (BASELINE.json config 3) in Mrays/s, on N B200s of one node.  --scene / --spp / --width / --height select the other configs
 (cornell_box: config 2; synthetic_<N> at 256 spp: config 4; 3840x2160 at 16384 spp: config 5).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--spp S] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--spp S] [--impl ours|reference] [--dump-outputs DIR]
   (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 A "step" = one complete render of the configuration: every pixel, `spp` samples, up to 5 path segments per sample
@@ -23,6 +23,8 @@ selects that one) and the float4 accumulation buffers are summed with ONE NCCL r
             on the same GPU, same scene / resolution / spp; time = its own "ms GPU time"; rays = its own count
             (oracle/_ref/ref_gpu).  The reference has no CPU renderer; its __host__ __device__ math built with g++
             (oracle/_ref/libref_host.so) is timed on the box's cores as `cpu_baseline` in both arms.
+  --dump-outputs DIR   after the timed steps, write what the last one computed as DIR/*.npy (see dump_outputs): the same
+            arguments give the same inputs, so two builds can be compared output for output.
 """
 import os
 
@@ -89,6 +91,24 @@ BYTES_NODE = 64.0            # our two-box node record (the reference: 2 x 32 B 
 BYTES_PRIM = 64.0            # our primitive record (the reference: 96 B Hittable)
 BYTES_MAT = 48.0             # material record, once per shade
 BYTES_PIXEL = 16.0           # float4 accumulate, once per pixel per render
+
+DUMP_BYTES = 64 << 20        # --dump-outputs budget
+DUMP_SAMPLE = 1 << 21        # pixels kept of an image over that budget
+
+
+def dump_outputs(out_dir, hdr_mean, rays):
+    """--dump-outputs: the last timed render as its caller receives it - the per-sample mean radiance, float32 (H, W, 3), as
+    hdr_mean.npy - and the rays it traced (whole job) as rays.npy, float64.  An image over DUMP_BYTES is written as a fixed sample
+    of DUMP_SAMPLE pixels (seed 0, the same from run to run): hdr_mean.npy (N, 3) with their row-major indices in
+    pixel_index.npy (float64 holding exact integers)."""
+    os.makedirs(out_dir, exist_ok=True)
+    if hdr_mean.nbytes > DUMP_BYTES:
+        h, w, c = hdr_mean.shape
+        pix = np.sort(np.random.default_rng(0).choice(h * w, DUMP_SAMPLE, replace=False))
+        hdr_mean = hdr_mean.reshape(h * w, c)[pix]
+        np.save(os.path.join(out_dir, "pixel_index.npy"), pix.astype(np.float64))
+    np.save(os.path.join(out_dir, "hdr_mean.npy"), np.ascontiguousarray(hdr_mean, np.float32))
+    np.save(os.path.join(out_dir, "rays.npy"), np.array([rays], np.float64))
 
 
 def clock_sampler(stop, out, index):
@@ -227,7 +247,12 @@ def main():
     ap.add_argument("--no-e2e-cli", action="store_true", help="skip the fresh-process e2e (in-process figure only)")
     ap.add_argument("--partition", default="pixels", choices=["pixels", "samples"],
                     help="N > 1: what is split over the GPUs (pathtracercuda_b200/distributed.py); the single reduce is the same")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's image and ray count to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.spp < 1:
+        ap.error("--steps and --spp must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the timed path of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -305,6 +330,9 @@ def main():
     wall = time.perf_counter() - t0
     stop.set()
     th.join(timeout=2)
+    # the last timed step's image (rank 0 holds the whole job's sum after the reduce), before the e2e runs below render into the
+    # same buffer; pixels outside a rank's share are zero on the other ranks, so only rank 0's copy is the caller's image
+    last_hdr = (accum[..., :3].cpu().numpy() / np.float32(args.spp)) if args.dump_outputs and rank == 0 else None
 
     ms_t = torch.tensor(ms_steps, dtype=torch.float64, device=f"cuda:{local}")
     rays_t = torch.tensor(rays_steps, dtype=torch.float64, device=f"cuda:{local}")
@@ -444,6 +472,8 @@ def main():
         }
         if not args.no_cpu_baseline and world == 1:
             line["cpu_baseline"] = cpu_baseline()
+        if last_hdr is not None:
+            dump_outputs(args.dump_outputs, last_hdr, float(rays_t[-1]))
         print(json.dumps(line))
     if dist:
         dist.barrier()
