@@ -208,6 +208,13 @@ const float *pt_get_hdr_sum(pt_context *ctx);
  *                    heuristic) of that draw and the BSDF's own.  The same integral as the reference's estimator (paths of at
  *                    most max_bounces segments, sky light through a miss) - the image converges to the same picture, with less
  *                    variance per sample under a sky with a sun; one more ray per vertex.  Default 0 (trace.cu:115-134).
+ *  "light_is"        1: every scattering vertex also draws one point on an emissive object (pt_light_distribution picks the object,
+ *                    the point is uniform over its surface) and traces a shadow ray to it; the light of the emitters is estimated by
+ *                    multiple importance sampling (balance heuristic) of that point and the BSDF's own direction.  The same integral as
+ *                    the reference's estimator (emission added where a path segment hits an emitter) - the image converges to the same
+ *                    picture, with less variance per sample in scenes lit by small emitters; one more ray per vertex.  A scene without
+ *                    emitters renders as without the option.  Not combinable with "env_is", the parity aids or a non-default "variant"
+ *                    (pt_render returns PT_E_INVALID).  Default 0 (trace.cu:136-151).
  *  "tex_unit"        1 (default): texture taps through CUDA texture objects, as the reference (Pathtracer.cpp:259-288);
  *                    0: fp32 bilinear filter in software over the packed texels */
 int pt_set_option(pt_context *ctx, const char *key, double value);
@@ -259,6 +266,13 @@ void pt_free(void *p);
  * P(cell) x cells / (2 pi^2), so that the solid-angle pdf of a direction in the cell is density / sin(theta).  Host only.
  * Call with alias = density = NULL for the grid size; returns the cell count or a negative error. */
 int pt_env_distribution(uint32_t width, uint32_t height, int is_hdr, const void *rgba, uint32_t *cols, uint32_t *rows, uint32_t *alias, float *density);
+
+/* The emitter table option "light_is" samples (no counterpart in the reference, which finds an emitter only when a BSDF-sampled ray
+ * hits it): every object with a non-zero emissive channel is one emitter, in the order of `objects`; selection weight = mean emissive x
+ * world surface area (exact for disks, quads and cubes under any transform, the uniform-scale value for the curved shapes).  Writes per
+ * emitter its index in `objects`, its selection probability and its alias-table entry (2 words: float bits of the acceptance threshold,
+ * alias emitter).  Host only.  Call with NULL buffers for the count; returns the emitter count (0 when nothing emits) or a negative error. */
+int pt_light_distribution(size_t count, const pt_object_desc *objects, uint32_t *scene_index, float *probability, uint32_t *alias);
 
 const char *pt_last_error(void);
 const char *pt_version(void);

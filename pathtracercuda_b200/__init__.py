@@ -8,8 +8,8 @@ device raises.
 """
 from .abi import (ASSETS, MATERIALS, REPO_ROOT, SHAPES, CameraDesc, MaterialDesc, ObjectDesc, Stats, make_camera,
                   make_object, object_array, parse_scene_py)
-from .api import LIB_PATH, Pathtracer, PtError, camera_rotate, camera_translate, env_distribution, load_library, parse_scene_file, read_image, write_hdr, write_png
+from .api import LIB_PATH, Pathtracer, PtError, camera_rotate, camera_translate, env_distribution, light_distribution, load_library, parse_scene_file, read_image, write_hdr, write_png
 
-__all__ = ["Pathtracer", "PtError", "camera_rotate", "camera_translate", "load_library", "env_distribution", "parse_scene_file", "read_image", "write_hdr", "write_png", "LIB_PATH",
+__all__ = ["Pathtracer", "PtError", "camera_rotate", "camera_translate", "load_library", "env_distribution", "light_distribution", "parse_scene_file", "read_image", "write_hdr", "write_png", "LIB_PATH",
            "make_object", "make_camera", "object_array", "parse_scene_py", "ObjectDesc", "MaterialDesc", "CameraDesc", "Stats",
            "SHAPES", "MATERIALS", "ASSETS", "REPO_ROOT"]

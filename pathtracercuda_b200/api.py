@@ -55,6 +55,7 @@ def load_library():
         "pt_write_png": (i32, [cp, u32, u32, vp]),
         "pt_write_hdr": (i32, [cp, u32, u32, vp]),
         "pt_env_distribution": (i32, [u32, u32, i32, vp, vp, vp, vp, vp]),
+        "pt_light_distribution": (i32, [sz, vp, vp, vp, vp]),
         "pt_read_image": (i32, [cp, vp, vp, vp, vp]),
         "pt_free": (None, [vp]),
         "pt_last_error": (cp, []),
@@ -73,7 +74,7 @@ def load_library():
 EXPORTS = ["pt_create", "pt_create_multi", "pt_get_multi_info", "pt_destroy", "pt_set_scene", "pt_set_scene_xform", "pt_render_vectors", "pt_load_texture", "pt_load_texture_mem", "pt_set_skybox", "pt_render",
            "pt_get_timing_ms", "pt_get_hdr", "pt_get_hdr_mean", "pt_get_hdr_sum", "pt_get_ldr", "pt_set_option", "pt_get_stats", "pt_camera_rotate", "pt_camera_translate", "pt_primary_pass",
            "pt_trace_rays", "pt_get_first_hit", "pt_accum_device_ptr", "pt_set_accum_device_ptr", "pt_load_scene_file", "pt_parse_scene_file",
-           "pt_write_png", "pt_write_hdr", "pt_env_distribution", "pt_read_image", "pt_free", "pt_last_error", "pt_version"]
+           "pt_write_png", "pt_write_hdr", "pt_env_distribution", "pt_light_distribution", "pt_read_image", "pt_free", "pt_last_error", "pt_version"]
 
 
 def _err(L):
@@ -130,6 +131,19 @@ def env_distribution(img):
     table, dens = np.zeros(2 * n, np.uint32), np.zeros(n, np.float32)
     L.pt_env_distribution(img.shape[1], img.shape[0], int(is_hdr), _p(img), None, None, _p(table), _p(dens))
     return cols.value, rows.value, table[0::2].copy().view(np.float32), table[1::2].copy(), dens
+
+
+def light_distribution(objects):
+    """pt_light_distribution: (scene_index, probability, q, alias) of the emitter table option "light_is" samples; host only"""
+    L = load_library()
+    arr = object_array(objects)
+    n = L.pt_light_distribution(len(objects), C.byref(arr), None, None, None)
+    if n < 0:
+        raise PtError(f"pt_light_distribution failed ({n}): {_err(L)}")
+    idx, prob, table = np.zeros(n, np.uint32), np.zeros(n, np.float32), np.zeros(2 * n, np.uint32)
+    if n:
+        L.pt_light_distribution(len(objects), C.byref(arr), _p(idx), _p(prob), _p(table))
+    return idx, prob, table[0::2].copy().view(np.float32), table[1::2].copy()
 
 
 def write_png(path, rgba):

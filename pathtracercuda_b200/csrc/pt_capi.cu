@@ -4,6 +4,7 @@
 #include "../../include/pt_b200.h"
 #include "image_io.h"
 #include "env_sampling.h"
+#include "light_sampling.h"
 #include "scene_compile.h"
 #include "scene_loader.h"
 #include "trace_kernels.h"
@@ -51,6 +52,10 @@ struct pt_context
 	void *envAlias = nullptr;
 	float *envDensity = nullptr;
 	uint32_t envCols = 0, envRows = 0;
+	// option "light_is": the emitter table of the current scene (light_sampling.h), built with the compiled scene
+	bool lightIS = false;
+	float4 *lightRecs = nullptr;
+	uint32_t lightCount = 0;
 	float *centreUV = nullptr; // option "jitter" = 0: pixel-centre coordinates (RenderParams::centreU / centreV), made on first use
 	// scene
 	float4 *sceneBlob = nullptr;
@@ -276,6 +281,7 @@ void pt_destroy(pt_context *c)
 	if (c->centreUV) cudaFree(c->centreUV);
 	if (c->envAlias) cudaFree(c->envAlias);
 	if (c->envDensity) cudaFree(c->envDensity);
+	if (c->lightRecs) cudaFree(c->lightRecs);
 	if (c->texDev) cudaFree(c->texDev);
 	if (c->sceneBlob) cudaFree(c->sceneBlob); // (the material table lives in the same allocation)
 	for (void *p : c->texMem) cudaFree(p);
@@ -287,12 +293,20 @@ void pt_destroy(pt_context *c)
 	delete c;
 }
 
-// upload a compiled scene to one device (replaces the previous one)
-static int uploadScene(pt_context *c, const CompiledScene &cs)
+// upload a compiled scene and its emitter table to one device (replaces the previous ones)
+static int uploadScene(pt_context *c, const CompiledScene &cs, const LightTable &lt)
 {
 	CK(cudaSetDevice(c->device));
 	CK(cudaStreamSynchronize(c->stream));
 	if (c->sceneBlob) { CK(cudaFree(c->sceneBlob)); c->sceneBlob = nullptr; }
+	if (c->lightRecs) { CK(cudaFree(c->lightRecs)); c->lightRecs = nullptr; }
+	c->lightCount = 0;
+	if (!lt.recs.empty())
+	{
+		CK(cudaMalloc(&c->lightRecs, lt.recs.size() * sizeof(LightRec)));
+		CK(cudaMemcpyAsync(c->lightRecs, lt.recs.data(), lt.recs.size() * sizeof(LightRec), cudaMemcpyHostToDevice, c->stream));
+		c->lightCount = uint32_t(lt.recs.size());
+	}
 	c->mats = nullptr;
 	// one allocation, nodes | primitives | materials: a scene that fits is staged in shared memory whole, by one bulk copy
 	const size_t nodeBytes = cs.nodes.size() * sizeof(Node), primBytes = cs.prims.size() * sizeof(Prim), matBytes = cs.mats.size() * sizeof(Mat);
@@ -326,9 +340,11 @@ int pt_set_scene(pt_context *c, size_t count, const pt_object_desc *objects)
 	CompiledScene cs;
 	std::string err;
 	if (!compileScene(count, objects, c->maxLeaf, cs, err, c->maxGlobal, nullptr, c->bvhBuilder)) return setError(PT_E_LIMIT, "pt_set_scene: " + err);
-	// the BVH is built ONCE on the host; a multi-GPU context replicates the compiled scene on every device
-	int r = uploadScene(c, cs);
-	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs);
+	LightTable lt;
+	buildLightTable(cs, lt);
+	// the BVH (and the emitter table) is built ONCE on the host; a multi-GPU context replicates the compiled scene on every device
+	int r = uploadScene(c, cs, lt);
+	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs, lt);
 	return r;
 	PT_CATCH(PT_E_LIMIT)
 }
@@ -359,8 +375,10 @@ int pt_set_scene_xform(pt_context *c, size_t count, const pt_object_xform_desc *
 	CompiledScene cs;
 	std::string err;
 	if (!compileScene(count, descs.data(), c->maxLeaf, cs, err, c->maxGlobal, xf.data(), c->bvhBuilder)) return setError(PT_E_LIMIT, "pt_set_scene_xform: " + err);
-	int r = uploadScene(c, cs);
-	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs);
+	LightTable lt;
+	buildLightTable(cs, lt);
+	int r = uploadScene(c, cs, lt);
+	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs, lt);
 	return r;
 	PT_CATCH(PT_E_LIMIT)
 }
@@ -595,6 +613,20 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		if (p.aids && !(v == 0 || v == 4 || v == 12))
 			return setError(PT_E_INVALID, "pt_render: the parity aids (jitter = 0, first_hit = 1) are built into the default kernels only (variant 0, 4 or 12)");
 		if (p.aids && c->launch.envIS) return setError(PT_E_INVALID, "pt_render: the parity aids and env_is cannot be combined");
+		c->launch.lightIS = 0;
+		if (c->lightIS)
+		{
+			if (c->envIS) return setError(PT_E_INVALID, "pt_render: light_is and env_is cannot be combined (one sampled light source per kernel)");
+			if (c->noJitter || c->firstHit) return setError(PT_E_INVALID, "pt_render: light_is and the parity aids (jitter = 0, first_hit = 1) cannot be combined");
+			if (!(v == 0 || v == 4 || v == 12)) return setError(PT_E_INVALID, "pt_render: light_is is built into the default kernels only (variant 0, 4 or 12)");
+			// a scene without emitters renders with the plain kernel: the same bits as without the option
+			if (c->lightCount != 0)
+			{
+				p.lights.recs = c->lightRecs;
+				p.lights.count = c->lightCount;
+				c->launch.lightIS = 1;
+			}
+		}
 		c->launch.stackLevels = int(c->bvhDepth) + 2;
 		CK(cudaEventRecord(c->evStart, c->stream)); // (all allocations are behind us: the events bracket the device work alone)
 		// pixel partition: the pixels of the other ranks hold zeros, so that the sum over ranks is the image
@@ -908,6 +940,7 @@ static int setOptionOne(pt_context *c, const char *key, double value)
 	else if (k == "smem_stack") c->launch.smemStack = int(value);
 	else if (k == "jitter") c->noJitter = value == 0;
 	else if (k == "env_is") c->envIS = value != 0;
+	else if (k == "light_is") c->lightIS = value != 0;
 	else if (k == "first_hit")
 	{
 		c->firstHit = value != 0;
@@ -1131,6 +1164,29 @@ int pt_env_distribution(uint32_t width, uint32_t height, int is_hdr, const void 
 	if (alias) memcpy(alias, d.alias.data(), d.alias.size() * 4);
 	if (density) memcpy(density, d.density.data(), d.density.size() * 4);
 	return int(d.density.size());
+	PT_CATCH(PT_E_LIMIT)
+}
+
+int pt_light_distribution(size_t count, const pt_object_desc *objects, uint32_t *scene_index, float *probability, uint32_t *alias)
+{
+	PT_TRY
+	if (count == 0 || !objects) return setError(PT_E_INVALID, "pt_light_distribution: bad arguments");
+	CompiledScene cs;
+	std::string err;
+	if (!compileScene(count, objects, 4, cs, err)) return setError(PT_E_LIMIT, "pt_light_distribution: " + err);
+	LightTable lt;
+	buildLightTable(cs, lt);
+	for (size_t k = 0; k < lt.recs.size(); ++k)
+	{
+		if (scene_index) scene_index[k] = lt.sceneIndex[k];
+		if (probability) probability[k] = lt.probability[k];
+		if (alias)
+		{
+			memcpy(&alias[2 * k], &lt.recs[k].aliasQ, 4);
+			alias[2 * k + 1] = lt.recs[k].alias;
+		}
+	}
+	return int(lt.recs.size());
 	PT_CATCH(PT_E_LIMIT)
 }
 

@@ -32,7 +32,9 @@ namespace ptb
 // AIDS: the parity aids (options "jitter" = 0, "first_hit" = 1) are compiled into a twin instantiation as well: in the kernel
 // that is benchmarked their two never-taken branches cost 1.5 % (measured: 6.5 of 435 ms; profiles/r02c_microvariants_run22.txt).
 // The twin is the same template with the same arguments; tests/test_gpu_baseline_sizes.py checks that both render the same bits.
-template <bool SMEM, bool COUNT, int TRAV, bool SHARE, bool SPLIT = false, bool SSTACK = false, bool ENVIS = false, bool AIDS = false>
+// LIGHTIS (option "light_is"): every scattering vertex also samples a point on an emitter (light_sampling.h), combined with the BSDF
+// sample by multiple importance sampling - a twin instantiation as well
+template <bool SMEM, bool COUNT, int TRAV, bool SHARE, bool SPLIT = false, bool SSTACK = false, bool ENVIS = false, bool AIDS = false, bool LIGHTIS = false>
 __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_constant__ RenderParams p)
 {
 	extern __shared__ __align__(128) float4 smemScene[];
@@ -82,7 +84,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 	V3 ro = camO, rd = mk(0.0f, 0.0f, 1.0f), thr = mk(1.0f, 1.0f, 1.0f), L = mk(0.0f, 0.0f, 0.0f);
 	uint32_t bounce = 0, rz = 0, rw = 0, sampleIdx = 0;
 	uint32_t rays = 0, nodeVisits = 0, primTests = 0, shades = 0, misses = 0;
-	float lastPdf = 0.0f;   // ENVIS: pdf with which the BSDF sampled the direction the lane is tracing (weights the sky at a miss)
+	float lastPdf = 0.0f;   // ENVIS / LIGHTIS: pdf with which the BSDF sampled the direction the lane is tracing (weights the sky at a miss, an emitter at a hit)
 	uint32_t wNext = p.spp; // SHARE: next sample of the warp's pixel to hand out (warp-uniform)
 	unsigned long long passStat[6] = { 0, 0, 0, 0, 0, 0 }; // COUNT + SPLIT (lane 0): camera passes, lanes, clocks; scattered passes, lanes, clocks
 	unsigned long long travClk[2] = { 0, 0 };               // COUNT + SPLIT: clocks up to the end of the traversal, camera / scattered passes
@@ -319,7 +321,21 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				// ---- shade / sample (trace.cu:136-151) ----
 				const float4 *mp = matTable + h.prim * 3;
 				const float4 m1 = sv.ld(mp + 1);
-				if constexpr (SHARE) color = color + thr * mk(m1.x, m1.y, m1.z); // getEmitted, Material.inl:62-65
+				if constexpr (LIGHTIS)
+				{
+					// a scattered ray that hits an emitter: the point could also have come from the light sample of the vertex it left
+					// (balance heuristic; the camera ray's hit has no such rival and keeps weight 1).  Mat::pad[0] = emitter index + 1
+					V3 emitted = mk(m1.x, m1.y, m1.z);
+					const uint32_t emitter = __float_as_uint(sv.ld(mp + 2).z);
+					if (bounce != 0u && emitter != 0u)
+					{
+						const float pl = lightPdfHit<SMEM>(p.lights, sv, emitter - 1u, h.prim, ro, rd, h.t);
+						emitted = (lastPdf * rcpApprox(lastPdf + pl)) * emitted;
+					}
+					if constexpr (SHARE) color = color + thr * emitted;
+					else L = L + thr * emitted;
+				}
+				else if constexpr (SHARE) color = color + thr * mk(m1.x, m1.y, m1.z); // getEmitted, Material.inl:62-65
 				else L = L + thr * mk(m1.x, m1.y, m1.z);
 				terminate = true;
 				// The last segment of a path only contributes what it hits: the direction the reference still samples there
@@ -376,6 +392,42 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							++rays;
 							uint32_t nv = 0, pt = 0;
 							const Hit hs = closestHitWW<SMEM, false, false, kHotExact, SSTACK, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr);
+							if (hs.prim < 0)
+							{
+								if constexpr (SHARE) color = color + contrib;
+								else L = L + contrib;
+							}
+						}
+					}
+					else if constexpr (LIGHTIS)
+					{
+						const Frame fr = makeFrame(s.n);
+						const V3 Vv = toTangent(fr, -rd);
+						// one point on an emitter (its own Philox stream: fourth counter word 2, slot = bounce - the draws of the path
+						// itself are those of a render without "light_is"), the f and pdf the BSDF sample would have had for its
+						// direction, and a shadow ray that stops short of it: Le x f x cos / (pdf_light + pdf_bsdf) if nothing is in the way
+						const uint4 q = philox4x32_10_keyed(pixel, sampleIdx, bounce, 2u, p.philoxKeys);
+						V3 wl;
+						float dist, pl;
+						int lprim;
+						const bool onLight = sampleLight<SMEM>(p.lights, sv, q, s.p, wl, dist, pl, lprim);
+						const V3 sl = toTangent(fr, wl);
+						V3 attL;
+						float pbL;
+						V3 contrib = mk(0.0f, 0.0f, 0.0f);
+						const bool lit = onLight && sl.z > 0.0f && evalMaterial(mtype, base, m0.w, m1.w, Vv, sl, attL, pbL);
+						if (lit)
+						{
+							const float4 le = sv.ld(matTable + lprim * 3 + 1);
+							contrib = thr * ((sl.z * rcpApprox(pl + pbL)) * attL) * mk(le.x, le.y, le.z);
+						}
+						scattered = sampleMaterial(mtype, base, m0.w, m1.w, fr, Vv, rnd0, rnd1, wi, weight, &lastPdf);
+						if (lit)
+						{
+							++rays;
+							uint32_t nv = 0, pt = 0;
+							const Hit hs = closestHitWW<SMEM, false, false, kHotExact, SSTACK, true, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr,
+							                                                                             dist * (1.0f - 1e-4f));
 							if (hs.prim < 0)
 							{
 								if constexpr (SHARE) color = color + contrib;
@@ -560,8 +612,8 @@ int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t s
 	// default: one pixel per warp (camera passes / scattered passes) for renders long enough to amortise the drain at the end of
 	// every pixel (the last paths of a pixel run with the other lanes idle: ~half a path per spp/32 samples), one pixel per lane otherwise
 	if (variant == 0) variant = p.spp >= 64 ? 12 : 4; // measured crossover on generated_scene: 32 spp 15.0 vs 15.2, 64 spp 15.7 vs 15.2, 128 spp 17.8 vs 15.2 Grays/s
-	if ((cfg.envIS || p.aids) && variant != 12 && variant != 4) return -1; // "env_is" and the parity aids are built into the two default kernels only
-	if (cfg.envIS && p.aids) return -1;                                    // (and not into one twin together)
+	if ((cfg.envIS || cfg.lightIS || p.aids) && variant != 12 && variant != 4) return -1; // "env_is", "light_is" and the parity aids are built into the two default kernels only
+	if (int(cfg.envIS != 0) + int(cfg.lightIS != 0) + int(p.aids != 0) > 1) return -1;   // (and not into one twin together)
 	const bool stackVariant = variant == 12 || variant == 4; // the two default kernels have shared-memory-stack instantiations
 	const size_t stackBytes = size_t(cfg.stackLevels) * kStackStride;
 	// what goes into shared memory: the scene when it fits (a scene larger than the opt-in limit stays in L2/HBM), the traversal
@@ -571,7 +623,7 @@ int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t s
 #define PT_PICK(KERN, ...)                                                                                                        \
 	(smem ? (cfg.countWork ? launchKernel(KERN<true, true __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<true, false __VA_ARGS__>, p, cfg, sb, stream)) \
 	      : (cfg.countWork ? launchKernel(KERN<false, true __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<false, false __VA_ARGS__>, p, cfg, sb, stream)))
-	// (the "env_is" twins exist without work counters only)
+	// (the "env_is" / "light_is" twins exist without work counters only)
 #define PT_PICK_NOCOUNT(KERN, ...) (smem ? launchKernel(KERN<true, false __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<false, false __VA_ARGS__>, p, cfg, sb, stream))
 	for (int attempt = 0; attempt < 3; ++attempt)
 	{
@@ -589,12 +641,14 @@ int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t s
 		case 12: // one pixel per warp, camera passes and scattered passes alternate
 			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, true, true, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, true, true, false, false, true);
 			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, true, true, true, true) : PT_PICK_NOCOUNT(traceKernel, , 1, true, true, false, true);
+			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, true, true, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, true, true, false, false, false, true);
 			else n = sstack ? PT_PICK(traceKernel, , 1, true, true, true) : PT_PICK(traceKernel, , 1, true, true);
 			break;
 		case 13: n = PT_PICK(traceKernel, , 2, true, true); break; // 12 + leaf parking
 		default: // 4: one pixel per lane, while-while traversal
 			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, false, false, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, false, false, false, false, true);
 			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, false, false, true, true) : PT_PICK_NOCOUNT(traceKernel, , 1, false, false, false, true);
+			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, false, false, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, false, false, false, false, false, true);
 			else n = sstack ? PT_PICK(traceKernel, , 1, false, false, true) : PT_PICK(traceKernel, , 1, false);
 			break;
 		}

@@ -20,6 +20,13 @@ struct EnvDev
 	uint32_t cols = 0, rows = 0;
 };
 
+// option "light_is": the emitter table (light_sampling.h LightRec, 64 bytes each), on the read-only path
+struct LightDev
+{
+	const float4 *recs = nullptr; // 4 quads per emitter
+	uint32_t count = 0;
+};
+
 struct SceneDev
 {
 	const float4 *sceneBlob = nullptr; // [nodes | prims | materials], 16-byte records, one allocation (bulk-copied to smem)
@@ -64,6 +71,9 @@ struct RenderParams
 	float alpha = 1.0f;             // what the kernel writes to the accumulation buffer's fourth channel (trace.cu:198 writes 1); a multi-GPU
 	                                // sample partition lets only its first device write 1, so that the summed alpha is 1 as on one GPU
 	uint32_t stackOffset = 0;       // SSTACK kernels: byte offset of the shared-memory traversal stack in dynamic shared memory
+	// (launch parameters added from here on go at the END: the constant-bank offsets of the fields above stay where the existing
+	// kernels read them)
+	LightDev lights; // set (count != 0) when the launch samples the emitters directly (option "light_is")
 };
 
 constexpr uint32_t kAidPixelCentre = 1u, kAidFirstHit = 2u;
@@ -82,6 +92,7 @@ struct LaunchConfig
 	int strataK = 0;     // experiments: log2 of the cell count (0 = the rule of pt_render: at least 32 samples per cell, at most 128 cells)
 	int smemStack = -1;  // traversal stack in shared memory (TravStack<true>): 1 on, 0 off, -1 = on when it fits beside the scene
 	int envIS = 0;       // next-event estimation of the sky with multiple importance sampling (RenderParams::scene.env; one-pixel-per-warp kernel)
+	int lightIS = 0;     // next-event estimation of the emitters with multiple importance sampling (RenderParams::lights; variants 4 / 12)
 	int stackLevels = 0; // BVH depth + 2: levels the shared-memory stack needs (set by pt_render from the compiled scene)
 	size_t maxSmemOptin = 0;
 };
