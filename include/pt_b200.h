@@ -189,7 +189,8 @@ const float *pt_get_hdr_sum(pt_context *ctx);
  *                    Karras' radix tree, one primitive per leaf - built by all cores in a tenth of the time, traversal ~2 % slower
  *                    (measured on 10 k ... 1 M objects); 2 (default): LBVH from 2^19 objects, SAH below (set before the scene)
  *  "max_global"      how many scene-spanning primitives are hoisted out of the BVH (default 8; set before the scene)
- *  "variant"         trace kernel variant, 0 = default (see csrc/trace_kernels.h LaunchConfig)
+ *  "variant"         trace kernel: 0 (default) = 12 from 64 spp, 4 below; 4 = one pixel per lane; 12 = one pixel per warp, with
+ *                    separate passes for camera rays and scattered rays.  Any other value returns PT_E_INVALID
  *  "beam"            pixel beams for camera rays (one-pixel-per-warp kernels): 1 on, 0 off, -1 auto (default: on from 128 spp)
  *  "regen_low"       one-pixel-per-warp kernels: idle lanes wait until this many can start new samples together (0 = default)
  *  "stratify"        one-pixel-per-warp kernels: stratify the two randoms of the FIRST scattering direction over the samples of a
@@ -201,7 +202,7 @@ const float *pt_get_hdr_sum(pt_context *ctx);
  *  "first_hit"       1: pt_render also records, per pixel, the scene index and t of the closest hit of the camera ray AS FOUND BY
  *                    THE RENDER KERNEL ITSELF (pt_get_first_hit); with "jitter" = 0 this is the primary-pass gate on the
  *                    production traversal (beams, MUFU reciprocals and all).  Both aids are compiled into a twin instantiation
- *                    of the default kernels (variant 0 / 4 / 12) - same template, same arguments - which renders the same bits
+ *                    of each trace kernel - same template, same arguments - which renders the same bits
  *                    as the instantiation without them (checked in tests/test_gpu_baseline_sizes.py)
  *  "env_is"          1: every scattering vertex also draws one direction from the sky's importance distribution
  *                    (pt_env_distribution) and the sky light reaching it is estimated by multiple importance sampling (balance
@@ -213,8 +214,8 @@ const float *pt_get_hdr_sum(pt_context *ctx);
  *                    multiple importance sampling (balance heuristic) of that point and the BSDF's own direction.  The same integral as
  *                    the reference's estimator (emission added where a path segment hits an emitter) - the image converges to the same
  *                    picture, with less variance per sample in scenes lit by small emitters; one more ray per vertex.  A scene without
- *                    emitters renders as without the option.  Not combinable with "env_is", the parity aids or a non-default "variant"
- *                    (pt_render returns PT_E_INVALID).  Default 0 (trace.cu:136-151).
+ *                    emitters renders as without the option.  Not combinable with "env_is" or the parity aids (pt_render returns
+ *                    PT_E_INVALID).  Default 0 (trace.cu:136-151).
  *  "tex_unit"        1 (default): texture taps through CUDA texture objects, as the reference (Pathtracer.cpp:259-288);
  *                    0: fp32 bilinear filter in software over the packed texels */
 int pt_set_option(pt_context *ctx, const char *key, double value);

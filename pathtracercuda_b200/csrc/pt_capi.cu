@@ -562,11 +562,11 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.seedHi = uint32_t(c->seed >> 32);
 		for (uint32_t i = 0; i < 10; ++i) { p.philoxKeys[2 * i] = p.seedLo + i * 0x9E3779B9u; p.philoxKeys[2 * i + 1] = p.seedHi + i * 0xBB67AE85u; }
 		p.maxBounces = c->maxBounces;
-		p.regenLow = c->launch.regenLow > 0 ? uint32_t(c->launch.regenLow) : (c->launch.variant == 8 || c->launch.variant == 9 || c->launch.variant == 10 ? 8u : 16u);
+		p.regenLow = c->launch.regenLow > 0 ? uint32_t(c->launch.regenLow) : 16u;
 		// first-bounce stratification (RenderParams::strataPer): 2^k cells, k <= 8, at least 16 samples per cell - the lanes of a
 		// pass of the one-pixel-per-warp kernel then hold samples of one or two neighbouring cells
 		const int v = c->launch.variant;
-		const bool perWarpKernel = v == 0 ? spp >= 64u : (v == 8 || v == 9 || v == 10 || v == 12 || v == 13); // launchTrace's choice
+		const bool perWarpKernel = v == 0 ? spp >= 64u : v == 12; // launchTrace's choice
 		const bool wantStrata = perWarpKernel && (c->launch.stratify < 0 ? spp >= 128u : c->launch.stratify != 0) && spp >= 4u && spp < (1u << 21);
 		if (wantStrata)
 		{
@@ -582,7 +582,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.beam = c->launch.beam < 0 ? (spp >= 128u ? 1u : 0u) : uint32_t(c->launch.beam != 0);
 		p.alpha = c->alpha;
 		c->launch.envIS = 0;
-		if (c->envIS && p.scene.skybox != 0 && (v == 0 || v == 4 || v == 12))
+		if (c->envIS && p.scene.skybox != 0)
 		{
 			const int rc = ensureEnvDistribution(c, p.scene.skybox);
 			if (rc != PT_OK) return rc;
@@ -610,15 +610,12 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.firstHitIndex = c->firstHit ? c->firstHitIndex : nullptr;
 		p.firstHitT = c->firstHit ? c->firstHitT : nullptr;
 		if (c->firstHit) p.aids |= kAidFirstHit;
-		if (p.aids && !(v == 0 || v == 4 || v == 12))
-			return setError(PT_E_INVALID, "pt_render: the parity aids (jitter = 0, first_hit = 1) are built into the default kernels only (variant 0, 4 or 12)");
 		if (p.aids && c->launch.envIS) return setError(PT_E_INVALID, "pt_render: the parity aids and env_is cannot be combined");
 		c->launch.lightIS = 0;
 		if (c->lightIS)
 		{
 			if (c->envIS) return setError(PT_E_INVALID, "pt_render: light_is and env_is cannot be combined (one sampled light source per kernel)");
 			if (c->noJitter || c->firstHit) return setError(PT_E_INVALID, "pt_render: light_is and the parity aids (jitter = 0, first_hit = 1) cannot be combined");
-			if (!(v == 0 || v == 4 || v == 12)) return setError(PT_E_INVALID, "pt_render: light_is is built into the default kernels only (variant 0, 4 or 12)");
 			// a scene without emitters renders with the plain kernel: the same bits as without the option
 			if (c->lightCount != 0)
 			{
@@ -929,7 +926,11 @@ static int setOptionOne(pt_context *c, const char *key, double value)
 	else if (k == "smem_scene") c->launch.smemScene = value != 0;
 	else if (k == "max_bounces") c->maxBounces = value < 1 ? 1u : uint32_t(value);
 	else if (k == "max_leaf") c->maxLeaf = value < 1 ? 1u : uint32_t(value);
-	else if (k == "variant") c->launch.variant = int(value);
+	else if (k == "variant")
+	{
+		if (!(value == 0 || value == 4 || value == 12)) return setError(PT_E_INVALID, "pt_set_option: variant must be 0 (default), 4 (one pixel per lane) or 12 (one pixel per warp)");
+		c->launch.variant = int(value);
+	}
 	else if (k == "max_global") c->maxGlobal = uint32_t(value < 0 ? 0 : value);
 	else if (k == "bvh_builder") c->bvhBuilder = value == 1 ? kBuilderLbvh : (value == 0 ? kBuilderSah : kBuilderAuto);
 	else if (k == "regen_low") c->launch.regenLow = int(value);

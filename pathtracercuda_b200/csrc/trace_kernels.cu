@@ -6,7 +6,7 @@
 //
 //   * persistent CTAs (one wave sized to the SM count) with path regeneration, so warps stay full through all five path
 //     segments instead of idling until the longest path of the warp ends (the reference runs one thread per pixel with no
-//     compaction).  Long renders (SHARE + SPLIT, from 64 spp): ONE PIXEL PER WARP - the lanes trace samples of the same
+//     compaction).  Long renders (SHARE, from 64 spp): ONE PIXEL PER WARP - the lanes trace samples of the same
 //     pixel; the leaves its camera rays can reach are found once per pixel (pixel beams, trace_device.cuh beamLeaves); a
 //     pass of the main loop is either for camera rays or for scattered rays; the first bounce is stratified (RenderParams::
 //     strataPer).  Short renders: one pixel per lane, pixels handed out by a warp-aggregated atomic (ballot + popc prefix);
@@ -34,7 +34,7 @@ namespace ptb
 // The twin is the same template with the same arguments; tests/test_gpu_baseline_sizes.py checks that both render the same bits.
 // LIGHTIS (option "light_is"): every scattering vertex also samples a point on an emitter (light_sampling.h), combined with the BSDF
 // sample by multiple importance sampling - a twin instantiation as well
-template <bool SMEM, bool COUNT, int TRAV, bool SHARE, bool SPLIT = false, bool SSTACK = false, bool ENVIS = false, bool AIDS = false, bool LIGHTIS = false>
+template <bool SMEM, bool COUNT, bool SHARE, bool SSTACK = false, bool ENVIS = false, bool AIDS = false, bool LIGHTIS = false>
 __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_constant__ RenderParams p)
 {
 	extern __shared__ __align__(128) float4 smemScene[];
@@ -66,8 +66,8 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 	const float4 *const matTable = sv.prims + size_t(p.scene.primCount) * 4;
 
 	// SHARE: the leaves the camera rays of the warp's pixel can reach (beamLeaves), nearest first
-	__shared__ BeamEntry beamList[SHARE && TRAV >= 1 ? kTraceThreads / 32 : 1][kBeamMax];
-	__shared__ BeamBox beamBoxes[SHARE && TRAV >= 1 && !SMEM ? kTraceThreads / 32 : 1][kBeamMax]; // scenes in global memory: the leaves' boxes (trace_device.cuh BeamBox)
+	__shared__ BeamEntry beamList[SHARE ? kTraceThreads / 32 : 1][kBeamMax];
+	__shared__ BeamBox beamBoxes[SHARE && !SMEM ? kTraceThreads / 32 : 1][kBeamMax]; // scenes in global memory: the leaves' boxes (trace_device.cuh BeamBox)
 	int nBeam = -1;
 	__shared__ float2 pixelXY[SHARE ? kTraceThreads / 32 : 1]; // SHARE: (x, y) of the warp's pixel, once per pixel instead of once per sample
 
@@ -86,9 +86,9 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 	uint32_t rays = 0, nodeVisits = 0, primTests = 0, shades = 0, misses = 0;
 	float lastPdf = 0.0f;   // ENVIS / LIGHTIS: pdf with which the BSDF sampled the direction the lane is tracing (weights the sky at a miss, an emitter at a hit)
 	uint32_t wNext = p.spp; // SHARE: next sample of the warp's pixel to hand out (warp-uniform)
-	unsigned long long passStat[6] = { 0, 0, 0, 0, 0, 0 }; // COUNT + SPLIT (lane 0): camera passes, lanes, clocks; scattered passes, lanes, clocks
-	unsigned long long travClk[2] = { 0, 0 };               // COUNT + SPLIT: clocks up to the end of the traversal, camera / scattered passes
-	const long long kernelT0 = COUNT && SPLIT ? clock64() : 0;
+	unsigned long long passStat[6] = { 0, 0, 0, 0, 0, 0 }; // COUNT + SHARE (lane 0): camera passes, lanes, clocks; scattered passes, lanes, clocks
+	unsigned long long travClk[2] = { 0, 0 };               // COUNT + SHARE: clocks up to the end of the traversal, camera / scattered passes
+	const long long kernelT0 = COUNT && SHARE ? clock64() : 0;
 
 	while (true)
 	{
@@ -155,17 +155,14 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 						if (lane == 0) pixelXY[(threadIdx.x >> 5)] = make_float2(float(px), float(py));
 						__syncwarp();
 					}
-					if constexpr (TRAV >= 1)
+					if (p.beam)
 					{
-						if (p.beam)
-						{
-							uint32_t px, py;
-							pixelToXY(pixel, p.width, p.height, px, py);
-							const float m = 1.0f / 64.0f; // footprint widened: the jittered (s, t) are rounded products
-							nBeam = beamLeaves<SMEM>(sv.nodes, p.scene.treeNodeCount, p.scene.nodeCount, p.cam, (float(px) - m) * invW, (float(px) + 1.0f + m) * invW, (float(py) - m) * invH,
-							                         (float(py) + 1.0f + m) * invH, beamList[(threadIdx.x >> 5)], lane == 0, SMEM ? nullptr : beamBoxes[(threadIdx.x >> 5)]);
-							__syncwarp();
-						}
+						uint32_t px, py;
+						pixelToXY(pixel, p.width, p.height, px, py);
+						const float m = 1.0f / 64.0f; // footprint widened: the jittered (s, t) are rounded products
+						nBeam = beamLeaves<SMEM>(sv.nodes, p.scene.treeNodeCount, p.scene.nodeCount, p.cam, (float(px) - m) * invW, (float(px) + 1.0f + m) * invW, (float(py) - m) * invH,
+						                         (float(py) + 1.0f + m) * invH, beamList[(threadIdx.x >> 5)], lane == 0, SMEM ? nullptr : beamBoxes[(threadIdx.x >> 5)]);
+						__syncwarp();
 					}
 					continue;
 				}
@@ -204,17 +201,17 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 		}
 
 		bool takePart = SHARE ? (alive || generate) : active;
-		if constexpr (SPLIT)
+		if constexpr (SHARE)
 		{
-			// SPLIT: a pass is EITHER for the camera rays just generated (coherent: same pixel, leaves from the pixel's beam list,
+			// a pass is EITHER for the camera rays just generated (coherent: same pixel, leaves from the pixel's beam list,
 			// no tree walk, usually the same material) OR for the scattered rays, where every live lane then walks the tree
 			// together.  Mixed passes kept ~11 of 32 lanes in the node loop: the lanes with camera rays had nothing to walk.
-			if (SHARE ? nGen != 0u : __any_sync(0xffffffffu, generate)) takePart = generate;
+			if (nGen != 0u) takePart = generate;
 		}
-		// COUNT + SPLIT: passes, participating lanes and clocks per pass kind (tools/exp.py prints them)
+		// COUNT + SHARE: passes, participating lanes and clocks per pass kind (tools/exp.py prints them)
 		long long passT0 = 0;
 		bool camPassNow = false;
-		if constexpr (COUNT && SPLIT)
+		if constexpr (COUNT && SHARE)
 		{
 			camPassNow = __any_sync(0xffffffffu, generate);
 			const uint32_t part = __popc(__ballot_sync(0xffffffffu, takePart));
@@ -270,11 +267,8 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 
 			// ---- traverse + intersect (trace.cu:112) ----
 			++rays;
-			const Hit h = TRAV == 0 ? closestHit<SMEM, COUNT, kHotExact>(sv, ro, rd, 0.001f, nodeVisits, primTests)
-			              : TRAV == 1 ? closestHitWW<SMEM, COUNT, false, kHotExact, SSTACK>(sv, ro, rd, 0.001f, nodeVisits, primTests, beamList[SHARE ? (threadIdx.x >> 5) : 0],
-			                                                                                SHARE && bounce == 0 ? nBeam : -1, stackColumn, SMEM ? nullptr : beamBoxes[SHARE ? (threadIdx.x >> 5) : 0])
-			                          : closestHitWW<SMEM, COUNT, true, kHotExact, SSTACK>(sv, ro, rd, 0.001f, nodeVisits, primTests, beamList[SHARE ? (threadIdx.x >> 5) : 0],
-			                                                                               SHARE && bounce == 0 ? nBeam : -1, stackColumn, SMEM ? nullptr : beamBoxes[SHARE ? (threadIdx.x >> 5) : 0]);
+			const Hit h = closestHitWW<SMEM, COUNT, kHotExact, SSTACK>(sv, ro, rd, 0.001f, nodeVisits, primTests, beamList[SHARE ? (threadIdx.x >> 5) : 0],
+			                                                           SHARE && bounce == 0 ? nBeam : -1, stackColumn, SMEM ? nullptr : beamBoxes[SHARE ? (threadIdx.x >> 5) : 0]);
 			if constexpr (AIDS)
 			{
 				// parity aid: what THIS kernel's traversal found for the camera ray (scene-order index, t), per pixel
@@ -285,7 +279,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				}
 			}
 
-			if constexpr (COUNT && SPLIT)
+			if constexpr (COUNT && SHARE)
 			{
 				// clocks of the traversal part of the pass, as seen by the first participating lane (debug statistics)
 				if (lane == uint32_t(__ffs(__activemask()) - 1)) travClk[camPassNow ? 0 : 1] += (unsigned long long)(clock64() - passT0);
@@ -391,7 +385,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 						{
 							++rays;
 							uint32_t nv = 0, pt = 0;
-							const Hit hs = closestHitWW<SMEM, false, false, kHotExact, SSTACK, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr);
+							const Hit hs = closestHitWW<SMEM, false, kHotExact, SSTACK, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr);
 							if (hs.prim < 0)
 							{
 								if constexpr (SHARE) color = color + contrib;
@@ -426,8 +420,8 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 						{
 							++rays;
 							uint32_t nv = 0, pt = 0;
-							const Hit hs = closestHitWW<SMEM, false, false, kHotExact, SSTACK, true, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr,
-							                                                                             dist * (1.0f - 1e-4f));
+							const Hit hs = closestHitWW<SMEM, false, kHotExact, SSTACK, true, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr,
+							                                                                      dist * (1.0f - 1e-4f));
 							if (hs.prim < 0)
 							{
 								if constexpr (SHARE) color = color + contrib;
@@ -453,7 +447,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				alive = false;
 			}
 		}
-		if constexpr (COUNT && SPLIT)
+		if constexpr (COUNT && SHARE)
 		{
 			__syncwarp();
 			if (lane == 0) passStat[camPassNow ? 2 : 5] += (unsigned long long)(clock64() - passT0);
@@ -465,7 +459,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 #pragma unroll
 	for (int o = 16; o > 0; o >>= 1) r64 += __shfl_xor_sync(0xffffffffu, r64, o);
 	if (lane == 0) atomicAdd(&p.counters[kCtrRays], r64);
-	if constexpr (COUNT && SPLIT)
+	if constexpr (COUNT && SHARE)
 	{
 		if (lane == 0)
 		{
@@ -612,14 +606,12 @@ int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t s
 	// default: one pixel per warp (camera passes / scattered passes) for renders long enough to amortise the drain at the end of
 	// every pixel (the last paths of a pixel run with the other lanes idle: ~half a path per spp/32 samples), one pixel per lane otherwise
 	if (variant == 0) variant = p.spp >= 64 ? 12 : 4; // measured crossover on generated_scene: 32 spp 15.0 vs 15.2, 64 spp 15.7 vs 15.2, 128 spp 17.8 vs 15.2 Grays/s
-	if ((cfg.envIS || cfg.lightIS || p.aids) && variant != 12 && variant != 4) return -1; // "env_is", "light_is" and the parity aids are built into the two default kernels only
-	if (int(cfg.envIS != 0) + int(cfg.lightIS != 0) + int(p.aids != 0) > 1) return -1;   // (and not into one twin together)
-	const bool stackVariant = variant == 12 || variant == 4; // the two default kernels have shared-memory-stack instantiations
+	if (int(cfg.envIS != 0) + int(cfg.lightIS != 0) + int(p.aids != 0) > 1) return -1; // "env_is", "light_is" and the parity aids are not built into one twin together
 	const size_t stackBytes = size_t(cfg.stackLevels) * kStackStride;
 	// what goes into shared memory: the scene when it fits (a scene larger than the opt-in limit stays in L2/HBM), the traversal
 	// stack when it fits beside it
 	bool smem = cfg.smemScene && sceneBytes + kStaticSmemBound <= cfg.maxSmemOptin;
-	bool sstack = stackVariant && cfg.smemStack != 0 && cfg.stackLevels > 0 && (smem ? sceneBytes : 0) + stackBytes + kStaticSmemBound <= cfg.maxSmemOptin;
+	bool sstack = cfg.smemStack != 0 && cfg.stackLevels > 0 && (smem ? sceneBytes : 0) + stackBytes + kStaticSmemBound <= cfg.maxSmemOptin;
 #define PT_PICK(KERN, ...)                                                                                                        \
 	(smem ? (cfg.countWork ? launchKernel(KERN<true, true __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<true, false __VA_ARGS__>, p, cfg, sb, stream)) \
 	      : (cfg.countWork ? launchKernel(KERN<false, true __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<false, false __VA_ARGS__>, p, cfg, sb, stream)))
@@ -633,23 +625,17 @@ int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t s
 		int n;
 		switch (variant)
 		{
-		case 1: n = PT_PICK(traceKernel, , 0, false); break;      // per-lane if/else traversal
-		case 5: n = PT_PICK(traceKernel, , 2, false); break;      // while-while + speculative leaf parking
-		case 8: n = PT_PICK(traceKernel, , 1, true); break;       // one pixel per WARP (lanes = samples), while-while
-		case 9: n = PT_PICK(traceKernel, , 2, true); break;       // one pixel per warp, while-while + leaf parking
-		case 10: n = PT_PICK(traceKernel, , 0, true); break;      // one pixel per warp, if/else traversal
 		case 12: // one pixel per warp, camera passes and scattered passes alternate
-			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, true, true, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, true, true, false, false, true);
-			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, true, true, true, true) : PT_PICK_NOCOUNT(traceKernel, , 1, true, true, false, true);
-			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, true, true, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, true, true, false, false, false, true);
-			else n = sstack ? PT_PICK(traceKernel, , 1, true, true, true) : PT_PICK(traceKernel, , 1, true, true);
+			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , true, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , true, false, false, true);
+			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , true, true, true) : PT_PICK_NOCOUNT(traceKernel, , true, false, true);
+			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , true, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , true, false, false, false, true);
+			else n = sstack ? PT_PICK(traceKernel, , true, true) : PT_PICK(traceKernel, , true);
 			break;
-		case 13: n = PT_PICK(traceKernel, , 2, true, true); break; // 12 + leaf parking
-		default: // 4: one pixel per lane, while-while traversal
-			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, false, false, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, false, false, false, false, true);
-			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, false, false, true, true) : PT_PICK_NOCOUNT(traceKernel, , 1, false, false, false, true);
-			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , 1, false, false, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , 1, false, false, false, false, false, true);
-			else n = sstack ? PT_PICK(traceKernel, , 1, false, false, true) : PT_PICK(traceKernel, , 1, false);
+		default: // 4: one pixel per lane
+			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , false, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , false, false, false, true);
+			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , false, true, true) : PT_PICK_NOCOUNT(traceKernel, , false, false, true);
+			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , false, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , false, false, false, false, true);
+			else n = sstack ? PT_PICK(traceKernel, , false, true) : PT_PICK(traceKernel, , false);
 			break;
 		}
 		if (n != 0) return n;

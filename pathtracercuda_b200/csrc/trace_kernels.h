@@ -83,16 +83,15 @@ struct LaunchConfig
 	int smCount = 148;
 	int smemScene = 1;   // stage the scene in shared memory when it fits
 	int countWork = 0;   // node/prim/shade/miss counters
-	int variant = 0;     // kernel variant (0 = default: 12 for spp >= 64, else 4.  4: one pixel per lane, while-while traversal; 1: if/else traversal;
-	                     //  5: + leaf parking; 8: one pixel per WARP (lanes = samples), while-while; 9/10: its other traversals;
-	                     //  12: 8 with separate passes for camera rays and scattered rays)
+	int variant = 0;     // kernel variant (0 = default: 12 for spp >= 64, else 4.  4: one pixel per lane; 12: one pixel per WARP (lanes =
+	                     //  samples) with separate passes for camera rays and scattered rays; both use the while-while traversal)
 	int regenLow = 0;    // see RenderParams::regenLow (0 = default)
 	int beam = -1;       // pixel beams for the camera rays of the one-pixel-per-warp kernel: 1 on, 0 off, -1 = on from 128 spp
 	int stratify = -1;   // first-bounce stratification (RenderParams::strataPer): 1 on, 0 off, -1 = on from 128 spp (one-pixel-per-warp kernels)
 	int strataK = 0;     // experiments: log2 of the cell count (0 = the rule of pt_render: at least 32 samples per cell, at most 128 cells)
 	int smemStack = -1;  // traversal stack in shared memory (TravStack<true>): 1 on, 0 off, -1 = on when it fits beside the scene
 	int envIS = 0;       // next-event estimation of the sky with multiple importance sampling (RenderParams::scene.env; one-pixel-per-warp kernel)
-	int lightIS = 0;     // next-event estimation of the emitters with multiple importance sampling (RenderParams::lights; variants 4 / 12)
+	int lightIS = 0;     // next-event estimation of the emitters with multiple importance sampling (RenderParams::lights)
 	int stackLevels = 0; // BVH depth + 2: levels the shared-memory stack needs (set by pt_render from the compiled scene)
 	size_t maxSmemOptin = 0;
 };

@@ -158,7 +158,7 @@ void emu_first_hit(void *p, const pt_camera_desc *cd, uint32_t width, uint32_t h
 			const float u = (float(x) + 0.5f) / float(width), v = (float(y) + 0.5f) / float(height);
 			const V3 o = mk(cam.origin[0], cam.origin[1], cam.origin[2]);
 			const V3 d = cameraDir<2>(cam, u, v);
-			const Hit h = closestHitWW<false, true, false, kHotExact>(sv, o, d, 0.001f, nv, pt, beam, nBeam, 0, boxes);
+			const Hit h = closestHitWW<false, true, kHotExact>(sv, o, d, 0.001f, nv, pt, beam, nBeam, 0, boxes);
 			hitIndex[i] = h.prim < 0 ? -1 : int32_t(primSceneIndex(sv.prims[h.prim * 4 + 3]));
 			hitT[i] = h.prim < 0 ? 0.0f : h.t;
 		}
@@ -231,7 +231,7 @@ uint64_t emu_render(void *p, const pt_camera_desc *cd, uint32_t width, uint32_t 
 				{
 					++raysTot;
 					uint32_t nv = 0, pt = 0;
-					const Hit h = g_beam ? closestHitWW<false, true, false, kHotExact>(sv, ro, rd, 0.001f, nv, pt, beam, bounce == 0 ? nBeam : -1, 0, boxes)
+					const Hit h = g_beam ? closestHitWW<false, true, kHotExact>(sv, ro, rd, 0.001f, nv, pt, beam, bounce == 0 ? nBeam : -1, 0, boxes)
 					                     : closestHit<false, true, kHotExact>(sv, ro, rd, 0.001f, nv, pt);
 					nvTot += nv; ptTot += pt;
 					if (h.prim < 0)

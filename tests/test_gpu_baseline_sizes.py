@@ -2,7 +2,7 @@
 
 Round 1 pinned the primary-pass gate on `primaryKernel` (IEEE division, plain walk).  Here the kernel that is benchmarked - one
 pixel per warp, pixel beams, hoisted-primitive culling, MUFU reciprocals, FFMA2 box tests, shared-memory stack
-(traceKernel<.., 1, true, true, ..>) - reports the closest hit of its own camera rays (options "jitter" = 0 + "first_hit" = 1),
+(traceKernel<SMEM, false, true, ..>) - reports the closest hit of its own camera rays (options "jitter" = 0 + "first_hit" = 1),
 on both BVH builders.  It is compared with the reference's hitBVH (kernels/trace.cu:28-98) as the reference's own GPU build
 computed it (tests/golden/refgpu_primary_*.npz, tools/make_golden_gpu.py).  Config 4's 100 k / 1 M object scenes are checked
 for their ray counts against the oracle (oracle/pt_oracle.c: the reference's host arithmetic on the reference's own BVH, pinned

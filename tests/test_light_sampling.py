@@ -379,7 +379,7 @@ def test_light_is_without_emitters_is_plain():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("other", [("env_is", 1), ("jitter", 0), ("first_hit", 1), ("variant", 8)])
+@pytest.mark.parametrize("other", [("env_is", 1), ("jitter", 0), ("first_hit", 1)])
 def test_light_is_rejected_combinations(other):
     W, H = 32, 32
     objs, cam = _cornell(W, H)

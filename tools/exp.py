@@ -27,7 +27,7 @@ with pt.Pathtracer(W, H) as P:
                       "bvh_nodes": st.bvh_nodes, "smem": st.scene_in_smem}), flush=True)
     import ctypes as C
     raw = (C.c_ulonglong * 24)()
-    if variant in (0, 12, 13) and hasattr(P.L, "pt_debug_counters") and P.L.pt_debug_counters(P.h, raw, 24) == 24 and raw[8]:
+    if variant in (0, 12) and hasattr(P.L, "pt_debug_counters") and P.L.pt_debug_counters(P.h, raw, 24) == 24 and raw[8]:
         cp, cl, cc, sp_, sl, sc, tot = [raw[8 + k] for k in range(7)]
         print(json.dumps({"camera_passes_per_ksample": round(1e3 * cp / st.samples, 2), "lanes_per_camera_pass": round(cl / max(cp, 1), 2), "clocks_per_camera_pass": round(cc / max(cp, 1), 1),
                           "scattered_passes_per_ksample": round(1e3 * sp_ / st.samples, 2), "lanes_per_scattered_pass": round(sl / max(sp_, 1), 2), "clocks_per_scattered_pass": round(sc / max(sp_, 1), 1),

@@ -18,7 +18,7 @@ with pt.Pathtracer(W, H) as P:
     ei, et = P.primaryPass(cam)
     P.setOption("jitter", 0)
     P.setOption("first_hit", 1)
-    for variant, beam, sstack, strat, smem in [(0, 1, 1, 1, 1), (0, 0, 1, 1, 1), (0, 1, 0, 1, 1), (0, 1, 1, 0, 1), (0, 1, 1, 1, 0), (0, 0, 0, 0, 0), (8, 1, 1, 1, 1), (8, 0, 0, 0, 1), (4, 0, 0, 0, 1), (4, 0, 1, 0, 1), (1, 0, 0, 0, 1)]:
+    for variant, beam, sstack, strat, smem in [(0, 1, 1, 1, 1), (0, 0, 1, 1, 1), (0, 1, 0, 1, 1), (0, 1, 1, 0, 1), (0, 1, 1, 1, 0), (0, 0, 0, 0, 0), (4, 0, 0, 0, 1), (4, 0, 1, 0, 1)]:
         for k, v in (("variant", variant), ("beam", beam), ("smem_stack", sstack), ("stratify", strat), ("smem_scene", smem)):
             P.setOption(k, v)
         P.render(cam, spp, True)

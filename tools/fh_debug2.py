@@ -11,7 +11,7 @@ with pt.Pathtracer(W, H) as P:
     P.setScene(objs)
     ei, et = P.primaryPass(cam)
     P.setOption("jitter", 0); P.setOption("first_hit", 1)
-    for variant, beam, sstack in [(0, 1, 1), (0, 0, 1), (0, 1, 0), (4, 0, 0), (8, 1, 0)]:
+    for variant, beam, sstack in [(0, 1, 1), (0, 0, 1), (0, 1, 0), (4, 0, 0)]:
         P.setOption("variant", variant); P.setOption("beam", beam); P.setOption("smem_stack", sstack)
         for spp in (128, 192):
             P.render(cam, spp, True)

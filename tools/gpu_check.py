@@ -115,32 +115,18 @@ def ref_pt(scene, W, H, spp):
             "stderr": p.stderr[-300:]}
 
 
-which = sys.argv[1:] or ["parity", "variants", "perf", "ref"]
+which = sys.argv[1:] or ["parity", "perf", "ref"]
 if "parity" in which:
     out["primary"] = [primary_3way("cornell_box", 256, 256), primary_3way("generated_scene", 1920, 1080)]
     print(json.dumps(out["primary"]), flush=True)
     out["render"] = [render_parity("cornell_box", 64, 64, 64), render_parity("generated_scene", 96, 54, 64)]
     print(json.dumps(out["render"]), flush=True)
-if "variants" in which:
-    imgs = {}
-    for v in (1, 0, 2):
-        with pt.Pathtracer(480, 270) as P:
-            cam = P.loadSceneFile(f"{pt.ASSETS}/scenes/generated_scene.json", cwd=pt.ASSETS)
-            P.setOption("variant", v)
-            P.render(cam, 32, True)
-            P.render(cam, 32, False)
-            imgs[v] = P.getHDRMean()
-    out["variants_bit_identical"] = {str(v): bool(np.array_equal(imgs[1].view(np.uint32), imgs[v].view(np.uint32))) for v in imgs}
-    print(json.dumps(out["variants_bit_identical"]), flush=True)
 if "perf" in which:
     out["perf"] = []
-    for kw in [dict(variant=1), dict(variant=0), dict(variant=2), dict(variant=3), dict(variant=0, smem_scene=0), dict(variant=0, count_work=1)]:
+    for kw in [dict(variant=0), dict(variant=0, smem_scene=0), dict(variant=0, count_work=1)]:
         r = perf("generated_scene", 1920, 1080, 256, **kw)
         out["perf"].append(r)
         print(json.dumps(r), flush=True)
-    r = perf("cornell_box", 1920, 1080, 256, variant=1)
-    out["perf"].append(r)
-    print(json.dumps(r), flush=True)
     r = perf("cornell_box", 1920, 1080, 256, variant=0)
     out["perf"].append(r)
     print(json.dumps(r), flush=True)

@@ -9,7 +9,7 @@ import pathtracercuda_b200 as pt
 for scene, W, H in (("generated_scene", 96, 54), ("cornell_box", 48, 48)):
     with pt.Pathtracer(W, H) as P:
         cam = P.loadSceneFile(f"{pt.ASSETS}/scenes/{scene}.json", cwd=pt.ASSETS)
-        for variant, spp, opts in ((4, 8, {}), (12, 160, {}), (12, 160, {"beam": 0}), (12, 160, {"smem_scene": 0}), (8, 96, {}), (12, 40, {"tex_unit": 0})):
+        for variant, spp, opts in ((4, 8, {}), (12, 160, {}), (12, 160, {"beam": 0}), (12, 160, {"smem_scene": 0}), (12, 40, {"tex_unit": 0})):
             P.setOption("variant", variant)
             for k, v in {"beam": -1, "smem_scene": 1, "tex_unit": 1, **opts}.items():
                 P.setOption(k, v)
