@@ -565,9 +565,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.regenLow = c->launch.regenLow > 0 ? uint32_t(c->launch.regenLow) : 16u;
 		// first-bounce stratification (RenderParams::strataPer): 2^k cells, k <= 8, at least 16 samples per cell - the lanes of a
 		// pass of the one-pixel-per-warp kernel then hold samples of one or two neighbouring cells
-		const int v = c->launch.variant;
-		const bool perWarpKernel = v == 0 ? spp >= 64u : v == 12; // launchTrace's choice
-		const bool wantStrata = perWarpKernel && (c->launch.stratify < 0 ? spp >= 128u : c->launch.stratify != 0) && spp >= 4u && spp < (1u << 21);
+		const bool wantStrata = onePixelPerWarp(c->launch, spp) && (c->launch.stratify < 0 ? spp >= 128u : c->launch.stratify != 0) && spp >= 4u && spp < (1u << 21);
 		if (wantStrata)
 		{
 			uint32_t k = 2;
@@ -581,7 +579,8 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		}
 		p.beam = c->launch.beam < 0 ? (spp >= 128u ? 1u : 0u) : uint32_t(c->launch.beam != 0);
 		p.alpha = c->alpha;
-		c->launch.envIS = 0;
+		// which twin of the trace kernel runs: the options compiled into twins are exclusive
+		c->launch.twin = Twin::Plain;
 		if (c->envIS && p.scene.skybox != 0)
 		{
 			const int rc = ensureEnvDistribution(c, p.scene.skybox);
@@ -590,7 +589,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 			p.scene.env.density = c->envDensity;
 			p.scene.env.cols = c->envCols;
 			p.scene.env.rows = c->envRows;
-			c->launch.envIS = 1;
+			c->launch.twin = Twin::EnvIS;
 		}
 		if (c->noJitter)
 		{
@@ -610,8 +609,11 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.firstHitIndex = c->firstHit ? c->firstHitIndex : nullptr;
 		p.firstHitT = c->firstHit ? c->firstHitT : nullptr;
 		if (c->firstHit) p.aids |= kAidFirstHit;
-		if (p.aids && c->launch.envIS) return setError(PT_E_INVALID, "pt_render: the parity aids and env_is cannot be combined");
-		c->launch.lightIS = 0;
+		if (p.aids)
+		{
+			if (c->launch.twin == Twin::EnvIS) return setError(PT_E_INVALID, "pt_render: the parity aids and env_is cannot be combined");
+			c->launch.twin = Twin::Aids;
+		}
 		if (c->lightIS)
 		{
 			if (c->envIS) return setError(PT_E_INVALID, "pt_render: light_is and env_is cannot be combined (one sampled light source per kernel)");
@@ -621,7 +623,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 			{
 				p.lights.recs = c->lightRecs;
 				p.lights.count = c->lightCount;
-				c->launch.lightIS = 1;
+				c->launch.twin = Twin::LightIS;
 			}
 		}
 		c->launch.stackLevels = int(c->bvhDepth) + 2;

@@ -24,17 +24,34 @@
 namespace ptb
 {
 
+// a finished pixel: the sum of its samples into the accumulation buffer (trace.cu:196-198)
+static __device__ __forceinline__ void storePixel(const RenderParams &p, uint32_t pixel, V3 color)
+{
+	float4 out = make_float4(color.x, color.y, color.z, p.alpha);
+	if (!p.ignoreHistory)
+	{
+		const float4 prev = p.accum[pixel];
+		out.x += prev.x; out.y += prev.y; out.z += prev.z;
+	}
+	p.accum[pixel] = out;
+}
+
+// a contribution of a lane's path: the one-pixel-per-warp kernel (SHARE) adds it to the warp's partial sums of the pixel as it comes, the
+// one-pixel-per-lane kernel to the path's own sum L, which goes to the pixel's when the path ends (the two orders of the additions give
+// different bits)
+template <bool SHARE>
+static __device__ __forceinline__ void accumulate(V3 &color, V3 &L, V3 c)
+{
+	if constexpr (SHARE) color = color + c;
+	else L = L + c;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // the trace kernel
 // ---------------------------------------------------------------------------------------------------------------
-// ENVIS (option "env_is"): every scattering vertex also samples the sky directly, combined with the BSDF sample by multiple
-// importance sampling (env_sampling.h) - a twin instantiation, so the default kernel's code is untouched by it
-// AIDS: the parity aids (options "jitter" = 0, "first_hit" = 1) are compiled into a twin instantiation as well: in the kernel
-// that is benchmarked their two never-taken branches cost 1.5 % (measured: 6.5 of 435 ms; profiles/r02c_microvariants_run22.txt).
-// The twin is the same template with the same arguments; tests/test_gpu_baseline_sizes.py checks that both render the same bits.
-// LIGHTIS (option "light_is"): every scattering vertex also samples a point on an emitter (light_sampling.h), combined with the BSDF
-// sample by multiple importance sampling - a twin instantiation as well
-template <bool SMEM, bool COUNT, bool SHARE, bool SSTACK = false, bool ENVIS = false, bool AIDS = false, bool LIGHTIS = false>
+// SMEM: the scene staged in shared memory; COUNT: work counters (option "count_work"); SHARE: one pixel per warp; SSTACK: the
+// traversal stack in shared memory; TWIN: the options compiled into an instantiation of their own (trace_kernels.h Twin)
+template <bool SMEM, bool COUNT, bool SHARE, bool SSTACK, Twin TWIN>
 __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_constant__ RenderParams p)
 {
 	extern __shared__ __align__(128) float4 smemScene[];
@@ -84,7 +101,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 	V3 ro = camO, rd = mk(0.0f, 0.0f, 1.0f), thr = mk(1.0f, 1.0f, 1.0f), L = mk(0.0f, 0.0f, 0.0f);
 	uint32_t bounce = 0, rz = 0, rw = 0, sampleIdx = 0;
 	uint32_t rays = 0, nodeVisits = 0, primTests = 0, shades = 0, misses = 0;
-	float lastPdf = 0.0f;   // ENVIS / LIGHTIS: pdf with which the BSDF sampled the direction the lane is tracing (weights the sky at a miss, an emitter at a hit)
+	float lastPdf = 0.0f;   // EnvIS / LightIS: pdf with which the BSDF sampled the direction the lane is tracing (weights the sky at a miss, an emitter at a hit)
 	uint32_t wNext = p.spp; // SHARE: next sample of the warp's pixel to hand out (warp-uniform)
 	unsigned long long passStat[6] = { 0, 0, 0, 0, 0, 0 }; // COUNT + SHARE (lane 0): camera passes, lanes, clocks; scattered passes, lanes, clocks
 	unsigned long long travClk[2] = { 0, 0 };               // COUNT + SHARE: clocks up to the end of the traversal, camera / scattered passes
@@ -131,16 +148,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							color.y += __shfl_xor_sync(0xffffffffu, color.y, o);
 							color.z += __shfl_xor_sync(0xffffffffu, color.z, o);
 						}
-						if (lane == 0)
-						{
-							float4 out = make_float4(color.x, color.y, color.z, p.alpha); // trace.cu:196-198
-							if (!p.ignoreHistory)
-							{
-								const float4 prev = p.accum[pixel];
-								out.x += prev.x; out.y += prev.y; out.z += prev.z;
-							}
-							p.accum[pixel] = out;
-						}
+						if (lane == 0) storePixel(p, pixel, color);
 					}
 					color = mk(0.0f, 0.0f, 0.0f);
 					unsigned long long next = 0;
@@ -172,16 +180,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 		{
 		// ---- accumulate + fetch the next pixel (warp-aggregated atomic: ballot + popc prefix) ----
 		const bool need = active && !alive && sample == p.spp;
-		if (need && pixel != kInvalid)
-		{
-			float4 out = make_float4(color.x, color.y, color.z, p.alpha); // trace.cu:196-198
-			if (!p.ignoreHistory)
-			{
-				const float4 prev = p.accum[pixel];
-				out.x += prev.x; out.y += prev.y; out.z += prev.z;
-			}
-			p.accum[pixel] = out;
-		}
+		if (need && pixel != kInvalid) storePixel(p, pixel, color);
 		const uint32_t needMask = __ballot_sync(0xffffffffu, need);
 		if (needMask)
 		{
@@ -238,7 +237,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				// option "jitter" = 0 (parity aid): every sample through the pixel centre, u = (x + 0.5) / W with the IEEE division of the
 				// reference's primary pass - read from two small tables the host worked out (a division routine here, even out of
 				// line, cost the hot loop 2 %: its call constrains the register allocation of everything around it)
-				if constexpr (AIDS)
+				if constexpr (TWIN == Twin::Aids)
 					if (p.aids & kAidPixelCentre) { u = __ldg(p.centreU + __float2uint_rz(pxf)); v = __ldg(p.centreV + __float2uint_rz(pyf)); }
 				rz = r.z; rw = r.w;
 				if constexpr (SHARE)
@@ -269,7 +268,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 			++rays;
 			const Hit h = closestHitWW<SMEM, COUNT, kHotExact, SSTACK>(sv, ro, rd, 0.001f, nodeVisits, primTests, beamList[SHARE ? (threadIdx.x >> 5) : 0],
 			                                                           SHARE && bounce == 0 ? nBeam : -1, stackColumn, SMEM ? nullptr : beamBoxes[SHARE ? (threadIdx.x >> 5) : 0]);
-			if constexpr (AIDS)
+			if constexpr (TWIN == Twin::Aids)
 			{
 				// parity aid: what THIS kernel's traversal found for the camera ray (scene-order index, t), per pixel
 				if ((p.aids & kAidFirstHit) && bounce == 0)
@@ -295,18 +294,13 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 					// call / return pairs per miss, and the calling convention fixes registers around them)
 					const float theta = fastAcos(rd.y), phi = fastAtan2Inline(rd.z, rd.x);
 					V3 sky = texLookup(p.scene.textures, p.scene.skybox, phi * (0.5f / PT_PI), theta * (1.0f / PT_PI));
-					if constexpr (ENVIS)
+					if constexpr (TWIN == Twin::EnvIS)
 					{
 						// a scattered ray that reaches the sky: the direction could also have come from the sky's own distribution
 						// (balance heuristic; the camera ray's miss has no such rival and keeps weight 1)
-						if (bounce != 0u)
-						{
-							const float pe = envPdf(p.scene.env, phi * (0.5f / PT_PI), theta * (1.0f / PT_PI), rd.y);
-							sky = (lastPdf * rcpApprox(lastPdf + pe)) * sky;
-						}
+						if (bounce != 0u) sky = balanceWeight(lastPdf, envPdf(p.scene.env, phi * (0.5f / PT_PI), theta * (1.0f / PT_PI), rd.y)) * sky;
 					}
-					if constexpr (SHARE) color = color + thr * sky; // the warp's partial sums take every contribution as it comes
-					else L = L + thr * sky;
+					accumulate<SHARE>(color, L, thr * sky);
 				}
 				terminate = true;
 			}
@@ -315,22 +309,15 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				// ---- shade / sample (trace.cu:136-151) ----
 				const float4 *mp = matTable + h.prim * 3;
 				const float4 m1 = sv.ld(mp + 1);
-				if constexpr (LIGHTIS)
+				V3 emitted = mk(m1.x, m1.y, m1.z); // getEmitted, Material.inl:62-65
+				if constexpr (TWIN == Twin::LightIS)
 				{
 					// a scattered ray that hits an emitter: the point could also have come from the light sample of the vertex it left
 					// (balance heuristic; the camera ray's hit has no such rival and keeps weight 1).  Mat::pad[0] = emitter index + 1
-					V3 emitted = mk(m1.x, m1.y, m1.z);
 					const uint32_t emitter = __float_as_uint(sv.ld(mp + 2).z);
-					if (bounce != 0u && emitter != 0u)
-					{
-						const float pl = lightPdfHit<SMEM>(p.lights, sv, emitter - 1u, h.prim, ro, rd, h.t);
-						emitted = (lastPdf * rcpApprox(lastPdf + pl)) * emitted;
-					}
-					if constexpr (SHARE) color = color + thr * emitted;
-					else L = L + thr * emitted;
+					if (bounce != 0u && emitter != 0u) emitted = balanceWeight(lastPdf, lightPdfHit<SMEM>(p.lights, sv, emitter - 1u, h.prim, ro, rd, h.t)) * emitted;
 				}
-				else if constexpr (SHARE) color = color + thr * mk(m1.x, m1.y, m1.z); // getEmitted, Material.inl:62-65
-				else L = L + thr * mk(m1.x, m1.y, m1.z);
+				accumulate<SHARE>(color, L, thr * emitted);
 				terminate = true;
 				// The last segment of a path only contributes what it hits: the direction the reference still samples there
 				// (trace.cu:139-151 in its fifth loop trip) is never traced and its weight never reaches the image - no normal,
@@ -358,7 +345,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 					else { rnd0 = uniform01(rz); rnd1 = uniform01(rw); }
 					V3 wi, weight;
 					bool scattered;
-					if constexpr (ENVIS)
+					if constexpr (TWIN == Twin::EnvIS)
 					{
 						const Frame fr = makeFrame(s.n);
 						const V3 Vv = toTangent(fr, -rd);
@@ -386,14 +373,10 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							++rays;
 							uint32_t nv = 0, pt = 0;
 							const Hit hs = closestHitWW<SMEM, false, kHotExact, SSTACK, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr);
-							if (hs.prim < 0)
-							{
-								if constexpr (SHARE) color = color + contrib;
-								else L = L + contrib;
-							}
+							if (hs.prim < 0) accumulate<SHARE>(color, L, contrib);
 						}
 					}
-					else if constexpr (LIGHTIS)
+					else if constexpr (TWIN == Twin::LightIS)
 					{
 						const Frame fr = makeFrame(s.n);
 						const V3 Vv = toTangent(fr, -rd);
@@ -422,11 +405,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							uint32_t nv = 0, pt = 0;
 							const Hit hs = closestHitWW<SMEM, false, kHotExact, SSTACK, true, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr,
 							                                                                      dist * (1.0f - 1e-4f));
-							if (hs.prim < 0)
-							{
-								if constexpr (SHARE) color = color + contrib;
-								else L = L + contrib;
-							}
+							if (hs.prim < 0) accumulate<SHARE>(color, L, contrib);
 						}
 					}
 					else scattered = sampleMaterial(mtype, base, m0.w, m1.w, s.n, rd, rnd0, rnd1, wi, weight);
@@ -598,54 +577,53 @@ static int launchKernel(K kern, const RenderParams &p, const LaunchConfig &cfg, 
 // the global-memory instantiations) - an upper bound; launchKernel has the last word (occupancy query)
 constexpr size_t kStaticSmemBound = 8192; // (the instantiations that stage the scene carry 4.5 KB: the beam boxes belong to the global-memory ones)
 
+// the instantiation of traceKernel for one scheduling form, stack form and twin; the twins exist without work counters only
+// (count_work is ignored for them)
+template <bool SHARE, bool SSTACK, Twin TWIN>
+static int launchTraceKernel(const RenderParams &p, const LaunchConfig &cfg, bool smem, size_t smemBytes, cudaStream_t stream)
+{
+	if constexpr (TWIN == Twin::Plain)
+		if (cfg.countWork)
+			return launchKernel(smem ? traceKernel<true, true, SHARE, SSTACK, TWIN> : traceKernel<false, true, SHARE, SSTACK, TWIN>, p, cfg, smemBytes, stream);
+	return launchKernel(smem ? traceKernel<true, false, SHARE, SSTACK, TWIN> : traceKernel<false, false, SHARE, SSTACK, TWIN>, p, cfg, smemBytes, stream);
+}
+
+template <bool SHARE, bool SSTACK>
+static int launchTwin(const RenderParams &p, const LaunchConfig &cfg, bool smem, size_t smemBytes, cudaStream_t stream)
+{
+	switch (cfg.twin)
+	{
+	case Twin::Aids: return launchTraceKernel<SHARE, SSTACK, Twin::Aids>(p, cfg, smem, smemBytes, stream);
+	case Twin::EnvIS: return launchTraceKernel<SHARE, SSTACK, Twin::EnvIS>(p, cfg, smem, smemBytes, stream);
+	case Twin::LightIS: return launchTraceKernel<SHARE, SSTACK, Twin::LightIS>(p, cfg, smem, smemBytes, stream);
+	default: return launchTraceKernel<SHARE, SSTACK, Twin::Plain>(p, cfg, smem, smemBytes, stream);
+	}
+}
+
 int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t stream, int *usedSmem)
 {
 	RenderParams p = pIn;
 	const size_t sceneBytes = (size_t(p.scene.nodeCount) + p.scene.primCount) * 64 + size_t(p.scene.primCount) * sizeof(Mat); // nodes | primitives | materials
-	int variant = cfg.variant;
-	// default: one pixel per warp (camera passes / scattered passes) for renders long enough to amortise the drain at the end of
-	// every pixel (the last paths of a pixel run with the other lanes idle: ~half a path per spp/32 samples), one pixel per lane otherwise
-	if (variant == 0) variant = p.spp >= 64 ? 12 : 4; // measured crossover on generated_scene: 32 spp 15.0 vs 15.2, 64 spp 15.7 vs 15.2, 128 spp 17.8 vs 15.2 Grays/s
-	if (int(cfg.envIS != 0) + int(cfg.lightIS != 0) + int(p.aids != 0) > 1) return -1; // "env_is", "light_is" and the parity aids are not built into one twin together
+	// one pixel per warp: camera passes and scattered passes alternate
+	const bool share = onePixelPerWarp(cfg, p.spp);
 	const size_t stackBytes = size_t(cfg.stackLevels) * kStackStride;
 	// what goes into shared memory: the scene when it fits (a scene larger than the opt-in limit stays in L2/HBM), the traversal
 	// stack when it fits beside it
 	bool smem = cfg.smemScene && sceneBytes + kStaticSmemBound <= cfg.maxSmemOptin;
 	bool sstack = cfg.smemStack != 0 && cfg.stackLevels > 0 && (smem ? sceneBytes : 0) + stackBytes + kStaticSmemBound <= cfg.maxSmemOptin;
-#define PT_PICK(KERN, ...)                                                                                                        \
-	(smem ? (cfg.countWork ? launchKernel(KERN<true, true __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<true, false __VA_ARGS__>, p, cfg, sb, stream)) \
-	      : (cfg.countWork ? launchKernel(KERN<false, true __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<false, false __VA_ARGS__>, p, cfg, sb, stream)))
-	// (the "env_is" / "light_is" twins exist without work counters only)
-#define PT_PICK_NOCOUNT(KERN, ...) (smem ? launchKernel(KERN<true, false __VA_ARGS__>, p, cfg, sb, stream) : launchKernel(KERN<false, false __VA_ARGS__>, p, cfg, sb, stream))
 	for (int attempt = 0; attempt < 3; ++attempt)
 	{
 		if (usedSmem) *usedSmem = smem ? 1 : 0;
 		p.stackOffset = uint32_t(smem ? sceneBytes : 0); // records are 64 bytes: the stack starts 16-byte aligned
 		const size_t sb = (smem ? sceneBytes : 0) + (sstack ? stackBytes : 0);
-		int n;
-		switch (variant)
-		{
-		case 12: // one pixel per warp, camera passes and scattered passes alternate
-			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , true, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , true, false, false, true);
-			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , true, true, true) : PT_PICK_NOCOUNT(traceKernel, , true, false, true);
-			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , true, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , true, false, false, false, true);
-			else n = sstack ? PT_PICK(traceKernel, , true, true) : PT_PICK(traceKernel, , true);
-			break;
-		default: // 4: one pixel per lane
-			if (p.aids) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , false, true, false, true) : PT_PICK_NOCOUNT(traceKernel, , false, false, false, true);
-			else if (cfg.envIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , false, true, true) : PT_PICK_NOCOUNT(traceKernel, , false, false, true);
-			else if (cfg.lightIS) n = sstack ? PT_PICK_NOCOUNT(traceKernel, , false, true, false, false, true) : PT_PICK_NOCOUNT(traceKernel, , false, false, false, false, true);
-			else n = sstack ? PT_PICK(traceKernel, , false, true) : PT_PICK(traceKernel, , false);
-			break;
-		}
+		const int n = share ? (sstack ? launchTwin<true, true>(p, cfg, smem, sb, stream) : launchTwin<true, false>(p, cfg, smem, sb, stream))
+		                    : (sstack ? launchTwin<false, true>(p, cfg, smem, sb, stream) : launchTwin<false, false>(p, cfg, smem, sb, stream));
 		if (n != 0) return n;
 		// the instantiation does not fit with this much shared memory: first without the stack, then without the scene
 		if (sstack) sstack = false;
 		else if (smem) smem = false;
 		else return -1;
 	}
-#undef PT_PICK
-#undef PT_PICK_NOCOUNT
 	return -1;
 }
 

@@ -78,6 +78,23 @@ struct RenderParams
 
 constexpr uint32_t kAidPixelCentre = 1u, kAidFirstHit = 2u;
 
+// Which twin of the trace kernel a launch runs (traceKernel's last template parameter).  Each option below is compiled into an
+// instantiation of its own, so that the plain kernel's code is untouched by it; one launch runs one of them.
+enum class Twin
+{
+	Plain,
+	// the parity aids (options "jitter" = 0, "first_hit" = 1; RenderParams::aids says which): in the kernel that is benchmarked their
+	// two never-taken branches cost 1.5 % (measured: 6.5 of 435 ms; profiles/r02c_microvariants_run22.txt).  The twin is the same
+	// template with the same arguments; tests/test_gpu_baseline_sizes.py checks that both render the same bits
+	Aids,
+	// option "env_is": every scattering vertex also samples the sky directly, combined with the BSDF sample by multiple importance
+	// sampling (env_sampling.h)
+	EnvIS,
+	// option "light_is": every scattering vertex also samples a point on an emitter (light_sampling.h), combined with the BSDF sample
+	// by multiple importance sampling
+	LightIS,
+};
+
 struct LaunchConfig
 {
 	int smCount = 148;
@@ -90,11 +107,16 @@ struct LaunchConfig
 	int stratify = -1;   // first-bounce stratification (RenderParams::strataPer): 1 on, 0 off, -1 = on from 128 spp (one-pixel-per-warp kernels)
 	int strataK = 0;     // experiments: log2 of the cell count (0 = the rule of pt_render: at least 32 samples per cell, at most 128 cells)
 	int smemStack = -1;  // traversal stack in shared memory (TravStack<true>): 1 on, 0 off, -1 = on when it fits beside the scene
-	int envIS = 0;       // next-event estimation of the sky with multiple importance sampling (RenderParams::scene.env; one-pixel-per-warp kernel)
-	int lightIS = 0;     // next-event estimation of the emitters with multiple importance sampling (RenderParams::lights)
+	Twin twin = Twin::Plain; // set by pt_render from the options (EnvIS: RenderParams::scene.env; LightIS: RenderParams::lights)
 	int stackLevels = 0; // BVH depth + 2: levels the shared-memory stack needs (set by pt_render from the compiled scene)
 	size_t maxSmemOptin = 0;
 };
+
+// The scheduling form launchTrace runs: one pixel per warp (variant 12) or one pixel per lane (variant 4).  The default (0) takes one
+// pixel per warp for renders long enough to amortise the drain at the end of every pixel (the last paths of a pixel run with the other
+// lanes idle: ~half a path per spp/32 samples) - measured crossover on generated_scene: 32 spp 15.0 vs 15.2, 64 spp 15.7 vs 15.2,
+// 128 spp 17.8 vs 15.2 Grays/s
+inline bool onePixelPerWarp(const LaunchConfig &cfg, uint32_t spp) { return cfg.variant == 0 ? spp >= 64u : cfg.variant == 12; }
 
 // Returns the number of kernels launched; *usedSmem = 1 when the scene was staged in shared memory.
 int launchTrace(const RenderParams &p, const LaunchConfig &cfg, cudaStream_t stream, int *usedSmem);

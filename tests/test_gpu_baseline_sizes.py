@@ -70,7 +70,7 @@ def test_production_kernel_first_hit_vs_reference_hitbvh(name, builder):
         st = P.stats()
         exact_idx, exact_t = P.primaryPass(cam)
         # The parity aids live in a twin instantiation of the kernel template (same source, same template arguments otherwise;
-        # csrc/trace_kernels.cu AIDS): with the ray generation left alone ("jitter" = 1) the twin (first_hit = 1) and the
+        # csrc/trace_kernels.h Twin::Aids): with the ray generation left alone ("jitter" = 1) the twin (first_hit = 1) and the
         # instantiation that is benchmarked (first_hit = 0) must render the very same bits - the twin's traversal IS the
         # production traversal
         P.setOption("jitter", 1)
