@@ -1,7 +1,8 @@
 // device_probe.cu — TEST-ONLY: the trace kernels' per-call device routines (trace_device.cuh), one thread per input, behind
-// extern "C" host wrappers, so that tests/test_device_functions.py can compare each routine on the GPU with the reference's stored
-// outputs and with float64 statements.  Never part of libpt_b200.so: the test builds it into a temporary directory, together with
-// the product's own host code (scene_compile.cpp, light_sampling.cpp, env_sampling.cpp) that makes the records the kernels read.
+// extern "C" host wrappers, so that tests/test_device_functions.py and tests/test_texture_lookups.py can compare each routine on the
+// GPU with the reference's stored outputs and with float64 statements.  Never part of libpt_b200.so: the test builds it into a
+// temporary directory, together with the product's own host code (scene_compile.cpp, light_sampling.cpp, env_sampling.cpp) that
+// makes the records the kernels read.
 // Every wrapper allocates, copies in, launches, copies out and frees; errors come back as a negative return value.
 #include "../pathtracercuda_b200/csrc/trace_device.cuh"
 #include "../pathtracercuda_b200/csrc/env_sampling.h"
@@ -264,5 +265,93 @@ extern "C" int probe_env(uint32_t width, uint32_t height, int isHdr, const void 
 		rc = finish(out, dOut, outBytes);
 	}
 	cudaFree(dAlias); cudaFree(dDens); cudaFree(dQ); cudaFree(dOut);
+	return rc;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------------------
+// textures: texLookup on a one-entry TexDesc table (handle 1) over the caller's texels - RGBA8 words or float4, row-major.
+// unit 0: texObj = 0, the fp32 software filter (option tex_unit = 0).  unit 1: a texture object over a copy of the texels in a CUDA
+// array with the descriptor of pt_capi.cu loadTextureMemOne (wrap U, clamp V, linear filter, normalised coordinates, RGBA8 read as
+// normalised floats).  This object is the probe's own; the end-to-end tests of tests/test_texture_lookups.py are what tie the
+// product's object to it.  in: (u, v)[2 n]; out[3 n]: the tap's rgb.
+// ---------------------------------------------------------------------------------------------------------------------------------
+__global__ void texKernel(const TexDesc *table, uint32_t n, const float *uv, float *out)
+{
+	const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	const V3 r = texLookup(table, 1u, uv[2 * i], uv[2 * i + 1]);
+	out[3 * i] = r.x; out[3 * i + 1] = r.y; out[3 * i + 2] = r.z;
+}
+
+extern "C" int probe_tex(uint32_t width, uint32_t height, int isHdr, const void *texels, int unit, uint32_t n, const float *uv, float *out)
+{
+	const size_t pitch = size_t(width) * (isHdr ? 16 : 4);
+	TexDesc t;
+	memset(&t, 0, sizeof t);
+	t.texels = toDevice<char>(texels, pitch * height);
+	t.width = width;
+	t.height = height;
+	t.isHdr = isHdr ? 1u : 0u;
+	cudaArray_t arr = nullptr;
+	cudaTextureObject_t obj = 0;
+	int rc = -1;
+	if (t.texels && unit)
+	{
+		cudaChannelFormatDesc fmt = isHdr ? cudaCreateChannelDesc<float4>() : cudaCreateChannelDesc<uchar4>();
+		bool ok = cudaMallocArray(&arr, &fmt, width, height) == cudaSuccess;
+		ok = ok && cudaMemcpy2DToArray(arr, 0, 0, texels, pitch, pitch, height, cudaMemcpyHostToDevice) == cudaSuccess;
+		if (ok)
+		{
+			cudaResourceDesc rd;
+			memset(&rd, 0, sizeof rd);
+			rd.resType = cudaResourceTypeArray;
+			rd.res.array.array = arr;
+			cudaTextureDesc td;
+			memset(&td, 0, sizeof td);
+			td.addressMode[0] = cudaAddressModeWrap;
+			td.addressMode[1] = cudaAddressModeClamp;
+			td.filterMode = cudaFilterModeLinear;
+			td.readMode = isHdr ? cudaReadModeElementType : cudaReadModeNormalizedFloat;
+			td.normalizedCoords = 1;
+			ok = cudaCreateTextureObject(&obj, &rd, &td, nullptr) == cudaSuccess;
+		}
+		t.texObj = ok ? (unsigned long long)obj : 0ull;
+	}
+	TexDesc *dTab = (t.texels && (!unit || t.texObj)) ? toDevice<TexDesc>(&t, sizeof t) : nullptr;
+	float *dUV = toDevice<float>(uv, size_t(n) * 8), *dOut = nullptr;
+	if (dTab && dUV && cudaMalloc(&dOut, size_t(n) * 12) == cudaSuccess)
+	{
+		texKernel<<<gridFor(n), kBlock>>>(dTab, n, dUV, dOut);
+		rc = finish(out, dOut, size_t(n) * 12);
+	}
+	if (obj) cudaDestroyTextureObject(obj);
+	if (arr) cudaFreeArray(arr);
+	cudaFree(const_cast<void *>(t.texels)); cudaFree(dTab); cudaFree(dUV); cudaFree(dOut);
+	return rc;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------------------
+// the equirectangular angles and the gamma step.  in[4 n]: y, x, c, p.
+// out[4 n]: fastAtan2(y, x), fastAtan2Inline(y, x), fastAcos(c), fastPow(p, 2.2f)
+// ---------------------------------------------------------------------------------------------------------------------------------
+__global__ void angleKernel(uint32_t n, const float *in, float *out)
+{
+	const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	const float *a = in + 4 * size_t(i);
+	float *o = out + 4 * size_t(i);
+	o[0] = fastAtan2(a[0], a[1]); o[1] = fastAtan2Inline(a[0], a[1]); o[2] = fastAcos(a[2]); o[3] = fastPow(a[3], 2.2f);
+}
+
+extern "C" int probe_angles(uint32_t n, const float *in, float *out)
+{
+	float *dIn = toDevice<float>(in, size_t(n) * 16), *dOut = nullptr;
+	int rc = -1;
+	if (dIn && cudaMalloc(&dOut, size_t(n) * 16) == cudaSuccess)
+	{
+		angleKernel<<<gridFor(n), kBlock>>>(n, dIn, dOut);
+		rc = finish(out, dOut, size_t(n) * 16);
+	}
+	cudaFree(dIn); cudaFree(dOut);
 	return rc;
 }

@@ -52,6 +52,23 @@ class Probe:
         L.probe_hit.argtypes = [vp, C.c_int, u32, vp, vp, vp, C.c_float, vp, vp]
         L.probe_light.argtypes = [vp, u32, vp, vp, vp]
         L.probe_env.argtypes = [u32, u32, C.c_int, vp, C.c_int, u32, vp, vp]
+        L.probe_tex.argtypes = [u32, u32, C.c_int, vp, C.c_int, u32, vp, vp]
+        L.probe_angles.argtypes = [u32, vp, vp]
+
+    def tex(self, img, u, v, unit):
+        """texLookup at (u, v) on an (H, W, 4) uint8 or float32 texture; unit 1 = through a texture object -> (n, 3) rgb"""
+        img = np.ascontiguousarray(img)
+        uv = np.ascontiguousarray(np.stack([u, v], 1), np.float32)
+        out = np.zeros((len(uv), 3), np.float32)
+        assert self.L.probe_tex(img.shape[1], img.shape[0], int(img.dtype == np.float32), _p(img), int(unit), len(uv), _p(uv), _p(out)) == 0
+        return out
+
+    def angles(self, y, x, c, p):
+        """-> (n, 4): fastAtan2(y, x), fastAtan2Inline(y, x), fastAcos(c), fastPow(p, 2.2f)"""
+        inp = np.ascontiguousarray(np.stack([y, x, c, p], 1), np.float32)
+        out = np.zeros((len(inp), 4), np.float32)
+        assert self.L.probe_angles(len(inp), _p(inp), _p(out)) == 0
+        return out
 
     def material(self, inp):
         inp = np.ascontiguousarray(inp, np.float32)
@@ -115,7 +132,7 @@ def _rng(tag):
 
 def test_probe_compiles_for_sm100a_without_spills(probe):
     kernels = re.findall(r"Compiling entry function '(\w+)' for 'sm_100a'", probe.log)
-    assert len(kernels) == 8, probe.log  # material, four hit forms, light, two sky
+    assert len(kernels) == 10, probe.log  # material, four hit forms, light, two sky, texture, angles
     spills = re.findall(r"(\d+) bytes spill stores, (\d+) bytes spill loads", probe.log)
     assert len(spills) == len(kernels) and all(a == "0" and b == "0" for a, b in spills), probe.log
 
