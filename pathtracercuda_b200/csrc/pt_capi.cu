@@ -12,9 +12,11 @@
 #include <cstdio>
 #include <cstring>
 #include <dlfcn.h>
+#include <memory>
 #include <nccl.h>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 using namespace ptb;
@@ -28,6 +30,40 @@ int setError(int code, const std::string &msg)
 	return code;
 }
 constexpr uint32_t kMaxTextures = 64; // MAX_TEXTURE_COUNT, Pathtracer.cpp:15
+
+// Memory of one CUDA allocator, freed when its holder goes.  Move-only; a holder is freed or replaced only where its device is
+// current and no queued work can still use it.
+template <cudaError_t (*Alloc)(void **, size_t), cudaError_t (*Free)(void *)>
+struct Buf
+{
+	void *p = nullptr;
+	Buf() = default;
+	Buf(Buf &&o) noexcept : p(std::exchange(o.p, nullptr)) {}
+	Buf &operator=(Buf o) noexcept { std::swap(p, o.p); return *this; } // (the memory held before goes with `o`)
+	~Buf() { if (p) Free(p); }
+	cudaError_t alloc(size_t bytes) // (on an empty holder; it stays empty when the allocation fails)
+	{
+		void *q = nullptr;
+		const cudaError_t e = Alloc(&q, bytes);
+		if (e == cudaSuccess) p = q;
+		return e;
+	}
+	template <typename T> T *as() const { return static_cast<T *>(p); }
+};
+using DevBuf = Buf<cudaMalloc, cudaFree>;          // device memory
+using HostBuf = Buf<cudaMallocHost, cudaFreeHost>; // pinned host memory
+
+// one loaded texture: the linear copy (software filter, env_is tables) and the texture object over a CUDA array of the same
+// texels; freed in the order object, array, linear copy
+struct Texture
+{
+	DevBuf texels;
+	cudaArray_t array = nullptr;
+	cudaTextureObject_t object = 0;
+	Texture() = default;
+	Texture(Texture &&o) noexcept : texels(std::move(o.texels)), array(std::exchange(o.array, nullptr)), object(std::exchange(o.object, 0)) {}
+	~Texture() { if (object) cudaDestroyTextureObject(object); if (array) cudaFreeArray(array); }
+};
 } // namespace
 
 struct pt_context
@@ -38,38 +74,32 @@ struct pt_context
 	cudaEvent_t evStart = nullptr, evStop = nullptr;
 	float4 *accum = nullptr;
 	bool ownAccum = true;
-	float4 *scaledDev = nullptr;
-	uchar4 *ldrDev = nullptr;
-	float *hostHdr = nullptr;     // pinned
-	uint8_t *hostLdr = nullptr;   // pinned
-	unsigned long long *counters = nullptr;
-	int32_t *firstHitIndex = nullptr; // option "first_hit": the render kernel's own first-hit (index, t) per pixel (parity aid)
-	float *firstHitT = nullptr;
+	DevBuf scaledDev, ldrDev;    // read-back staging (float4 / uchar4 per pixel)
+	HostBuf hostHdr, hostLdr;
+	DevBuf counters;             // kCtrCount unsigned long long
+	DevBuf firstHitIndex, firstHitT; // option "first_hit": the render kernel's own first-hit (index, t) per pixel (parity aid)
 	bool firstHit = false, noJitter = false;
 	// option "env_is": the sky's importance distribution (env_sampling.h), built for texture handle envHandle on first use
 	bool envIS = false;
 	uint32_t envHandle = 0;
-	void *envAlias = nullptr;
-	float *envDensity = nullptr;
+	DevBuf envAlias, envDensity;
 	uint32_t envCols = 0, envRows = 0;
 	// option "light_is": the emitter table of the current scene (light_sampling.h), built with the compiled scene
 	bool lightIS = false;
-	float4 *lightRecs = nullptr;
+	DevBuf lightRecs;
 	uint32_t lightCount = 0;
-	float *centreUV = nullptr; // option "jitter" = 0: pixel-centre coordinates (RenderParams::centreU / centreV), made on first use
+	DevBuf centreUV; // option "jitter" = 0: pixel-centre coordinates (RenderParams::centreU / centreV), made on first use
 	// scene
-	float4 *sceneBlob = nullptr;
-	Mat *mats = nullptr;
+	DevBuf sceneBlob;
+	Mat *mats = nullptr; // (the material table at the end of sceneBlob)
 	uint32_t nodeCount = 0, treeNodeCount = 0, primCount = 0, bvhDepth = 0, globalCount = 0, maxGlobal = ptb::kMaxGlobalPrims;
 	int bvhBuilder = ptb::kBuilderAuto; // option "bvh_builder" (scene_compile.h): SAH, from 2^19 objects the LBVH
-	// textures
-	std::vector<void *> texMem;
+	// textures: handle h is textures[h - 1] and texHost[h - 1]
+	std::vector<Texture> textures;
 	TexDesc texHost[kMaxTextures];
-	std::vector<cudaArray_t> texArrays;
-	std::vector<cudaTextureObject_t> texObjects;
 	int texUnit = 1; // filter textures with the texture unit (0: in software from linear memory)
-	TexDesc *texDev = nullptr;
-	uint32_t textureCount = 0, skybox = 0;
+	DevBuf texDev;   // the device copy of texHost
+	uint32_t skybox = 0;
 	// state mirrored from the reference
 	float timingMs = 0.0f;
 	uint32_t accumulatedFrames = 0;
@@ -113,18 +143,6 @@ struct pt_context
 			return setError(PT_E_CUDA, buf);                                                                          \
 		}                                                                                                             \
 	} while (0)
-
-namespace
-{
-// device allocation freed on every return path
-struct DevBuf
-{
-	void *p = nullptr;
-	~DevBuf() { if (p) cudaFree(p); }
-	cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes); }
-	template <typename T> T *as() const { return static_cast<T *>(p); }
-};
-} // namespace
 
 // NCCL is loaded at run time (dlopen, local scope), only when a multi-GPU context first needs a reduce: the library keeps
 // no link-time dependency on it - a host process that already carries its own NCCL (PyTorch's) is left alone, and single-GPU
@@ -170,36 +188,34 @@ int pt_create(uint32_t width, uint32_t height, int device, pt_context **out)
 		return setError(PT_E_NO_DEVICE, "pt_create: no CUDA device (this library has no CPU fallback)");
 	}
 	if (device < 0 || device >= count) return setError(PT_E_INVALID, "pt_create: device ordinal out of range");
-	pt_context *c = new pt_context();
+	std::unique_ptr<pt_context, void (*)(pt_context *)> c(new pt_context(), pt_destroy); // (destroyed on every early return)
 	c->device = device;
 	c->width = width;
 	c->height = height;
 	memset(&c->stats, 0, sizeof c->stats);
 	memset(c->texHost, 0, sizeof c->texHost);
 	const size_t px = size_t(width) * height;
-#define CKC(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { char buf[512]; snprintf(buf, sizeof buf, "CUDA error = %u at %s:%d '%s' (%s)", (unsigned)e_, __FILE__, __LINE__, #expr, cudaGetErrorString(e_)); g_lastError = buf; pt_destroy(c); return PT_E_CUDA; } } while (0)
-	CKC(cudaSetDevice(device));
+	CK(cudaSetDevice(device));
 	// (two attributes, not cudaGetDeviceProperties: that call fills in everything the driver knows about the device and is one of
 	// the slower ones of a process's start)
 	int smCount = 0, smemOptin = 0;
-	CKC(cudaDeviceGetAttribute(&smCount, cudaDevAttrMultiProcessorCount, device));
-	CKC(cudaDeviceGetAttribute(&smemOptin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+	CK(cudaDeviceGetAttribute(&smCount, cudaDevAttrMultiProcessorCount, device));
+	CK(cudaDeviceGetAttribute(&smemOptin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
 	c->launch.smCount = smCount;
 	c->launch.maxSmemOptin = size_t(smemOptin);
-	CKC(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-	CKC(cudaEventCreate(&c->evStart));
-	CKC(cudaEventCreate(&c->evStop));
-	CKC(cudaMalloc(&c->accum, px * sizeof(float4)));
-	CKC(cudaMemsetAsync(c->accum, 0, px * sizeof(float4), c->stream));
+	CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+	CK(cudaEventCreate(&c->evStart));
+	CK(cudaEventCreate(&c->evStop));
+	CK(cudaMalloc(&c->accum, px * sizeof(float4)));
+	CK(cudaMemsetAsync(c->accum, 0, px * sizeof(float4), c->stream));
 	// (the read-back buffers - device staging and pinned host memory for the HDR and the LDR image - are allocated by the first
 	// getter that needs them: pinned allocations are slow, a peer context of a multi-GPU job never reads back, and a run that
 	// writes a PNG does not need the 33 MB HDR pair)
-	CKC(cudaMalloc(&c->counters, kCtrCount * sizeof(unsigned long long)));
-	CKC(cudaMalloc(&c->texDev, kMaxTextures * sizeof(TexDesc)));
-	CKC(cudaMemsetAsync(c->texDev, 0, kMaxTextures * sizeof(TexDesc), c->stream));
-	CKC(cudaStreamSynchronize(c->stream));
-#undef CKC
-	*out = c;
+	CK(c->counters.alloc(kCtrCount * sizeof(unsigned long long)));
+	CK(c->texDev.alloc(kMaxTextures * sizeof(TexDesc)));
+	CK(cudaMemsetAsync(c->texDev.p, 0, kMaxTextures * sizeof(TexDesc), c->stream));
+	CK(cudaStreamSynchronize(c->stream));
+	*out = c.release();
 	return PT_OK;
 	PT_CATCH(PT_E_LIMIT)
 }
@@ -271,51 +287,35 @@ void pt_destroy(pt_context *c)
 	if (c->reduced) cudaFree(c->reduced);
 	if (c->stream) cudaStreamSynchronize(c->stream);
 	if (c->ownAccum && c->accum) cudaFree(c->accum);
-	if (c->scaledDev) cudaFree(c->scaledDev);
-	if (c->ldrDev) cudaFree(c->ldrDev);
-	if (c->hostHdr) cudaFreeHost(c->hostHdr);
-	if (c->hostLdr) cudaFreeHost(c->hostLdr);
-	if (c->counters) cudaFree(c->counters);
-	if (c->firstHitIndex) cudaFree(c->firstHitIndex);
-	if (c->firstHitT) cudaFree(c->firstHitT);
-	if (c->centreUV) cudaFree(c->centreUV);
-	if (c->envAlias) cudaFree(c->envAlias);
-	if (c->envDensity) cudaFree(c->envDensity);
-	if (c->lightRecs) cudaFree(c->lightRecs);
-	if (c->texDev) cudaFree(c->texDev);
-	if (c->sceneBlob) cudaFree(c->sceneBlob); // (the material table lives in the same allocation)
-	for (void *p : c->texMem) cudaFree(p);
-	for (cudaTextureObject_t o : c->texObjects) cudaDestroyTextureObject(o);
-	for (cudaArray_t a : c->texArrays) cudaFreeArray(a);
 	if (c->evStart) cudaEventDestroy(c->evStart);
 	if (c->evStop) cudaEventDestroy(c->evStop);
 	if (c->stream) cudaStreamDestroy(c->stream);
-	delete c;
+	delete c; // (the holders free the rest: the device is current and the stream has finished)
 }
 
-// upload a compiled scene and its emitter table to one device (replaces the previous ones)
+// upload a compiled scene and its emitter table to one device; they replace the previous ones once they are complete
 static int uploadScene(pt_context *c, const CompiledScene &cs, const LightTable &lt)
 {
 	CK(cudaSetDevice(c->device));
-	CK(cudaStreamSynchronize(c->stream));
-	if (c->sceneBlob) { CK(cudaFree(c->sceneBlob)); c->sceneBlob = nullptr; }
-	if (c->lightRecs) { CK(cudaFree(c->lightRecs)); c->lightRecs = nullptr; }
-	c->lightCount = 0;
+	DevBuf lights;
 	if (!lt.recs.empty())
 	{
-		CK(cudaMalloc(&c->lightRecs, lt.recs.size() * sizeof(LightRec)));
-		CK(cudaMemcpyAsync(c->lightRecs, lt.recs.data(), lt.recs.size() * sizeof(LightRec), cudaMemcpyHostToDevice, c->stream));
-		c->lightCount = uint32_t(lt.recs.size());
+		CK(lights.alloc(lt.recs.size() * sizeof(LightRec)));
+		CK(cudaMemcpyAsync(lights.p, lt.recs.data(), lt.recs.size() * sizeof(LightRec), cudaMemcpyHostToDevice, c->stream));
 	}
-	c->mats = nullptr;
 	// one allocation, nodes | primitives | materials: a scene that fits is staged in shared memory whole, by one bulk copy
 	const size_t nodeBytes = cs.nodes.size() * sizeof(Node), primBytes = cs.prims.size() * sizeof(Prim), matBytes = cs.mats.size() * sizeof(Mat);
-	CK(cudaMalloc(&c->sceneBlob, nodeBytes + primBytes + matBytes));
-	c->mats = reinterpret_cast<Mat *>(reinterpret_cast<char *>(c->sceneBlob) + nodeBytes + primBytes);
-	CK(cudaMemcpyAsync(c->sceneBlob, cs.nodes.data(), nodeBytes, cudaMemcpyHostToDevice, c->stream));
-	CK(cudaMemcpyAsync(reinterpret_cast<char *>(c->sceneBlob) + nodeBytes, cs.prims.data(), primBytes, cudaMemcpyHostToDevice, c->stream));
-	CK(cudaMemcpyAsync(c->mats, cs.mats.data(), matBytes, cudaMemcpyHostToDevice, c->stream));
-	CK(cudaStreamSynchronize(c->stream));
+	DevBuf blob;
+	CK(blob.alloc(nodeBytes + primBytes + matBytes));
+	char *const b = blob.as<char>();
+	CK(cudaMemcpyAsync(b, cs.nodes.data(), nodeBytes, cudaMemcpyHostToDevice, c->stream));
+	CK(cudaMemcpyAsync(b + nodeBytes, cs.prims.data(), primBytes, cudaMemcpyHostToDevice, c->stream));
+	CK(cudaMemcpyAsync(b + nodeBytes + primBytes, cs.mats.data(), matBytes, cudaMemcpyHostToDevice, c->stream));
+	CK(cudaStreamSynchronize(c->stream)); // (also: no render still reads the scene replaced here)
+	c->sceneBlob = std::move(blob);
+	c->mats = reinterpret_cast<Mat *>(b + nodeBytes + primBytes);
+	c->lightRecs = std::move(lights);
+	c->lightCount = uint32_t(lt.recs.size());
 	c->nodeCount = uint32_t(cs.nodes.size());
 	c->primCount = uint32_t(cs.prims.size());
 	c->globalCount = cs.globalCount;
@@ -327,59 +327,57 @@ static int uploadScene(pt_context *c, const CompiledScene &cs, const LightTable 
 	return PT_OK;
 }
 
-int pt_set_scene(pt_context *c, size_t count, const pt_object_desc *objects)
+// pt_set_scene (objects) and pt_set_scene_xform (xobjects: objects given by their world-to-local transform and box)
+static int setScene(pt_context *c, const std::string &fn, size_t count, const pt_object_desc *objects, const pt_object_xform_desc *xobjects)
 {
-	PT_TRY
-	if (!c) return setError(PT_E_INVALID, "pt_set_scene: null context");
+	if (!c) return setError(PT_E_INVALID, fn + ": null context");
 	if (count == 0)
 	{
 		printf("Setting an empty scene is not allowed!\n"); // Pathtracer.cpp:115
 		return PT_OK;
 	}
-	if (!objects) return setError(PT_E_INVALID, "pt_set_scene: null objects");
+	if (!objects && !xobjects) return setError(PT_E_INVALID, fn + ": null objects");
+	std::vector<pt_object_desc> descs;
+	std::vector<ObjectXform> xf;
+	if (xobjects)
+	{
+		descs.resize(count);
+		xf.resize(count);
+		for (size_t i = 0; i < count; ++i)
+		{
+			memset(&descs[i], 0, sizeof descs[i]);
+			descs[i].type = xobjects[i].type;
+			descs[i].scale[0] = descs[i].scale[1] = descs[i].scale[2] = 1.0f;
+			descs[i].material = xobjects[i].material;
+			memset(&xf[i], 0, sizeof xf[i]);
+			memcpy(xf[i].w2l, xobjects[i].world_to_local, sizeof xf[i].w2l);
+			memcpy(xf[i].bmin, xobjects[i].aabb_min, 12);
+			memcpy(xf[i].bmax, xobjects[i].aabb_max, 12);
+		}
+		objects = descs.data();
+	}
 	CompiledScene cs;
 	std::string err;
-	if (!compileScene(count, objects, c->maxLeaf, cs, err, c->maxGlobal, nullptr, c->bvhBuilder)) return setError(PT_E_LIMIT, "pt_set_scene: " + err);
+	if (!compileScene(count, objects, c->maxLeaf, cs, err, c->maxGlobal, xobjects ? xf.data() : nullptr, c->bvhBuilder)) return setError(PT_E_LIMIT, fn + ": " + err);
 	LightTable lt;
 	buildLightTable(cs, lt);
 	// the BVH (and the emitter table) is built ONCE on the host; a multi-GPU context replicates the compiled scene on every device
 	int r = uploadScene(c, cs, lt);
 	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs, lt);
 	return r;
+}
+
+int pt_set_scene(pt_context *c, size_t count, const pt_object_desc *objects)
+{
+	PT_TRY
+	return setScene(c, "pt_set_scene", count, objects, nullptr);
 	PT_CATCH(PT_E_LIMIT)
 }
 
 int pt_set_scene_xform(pt_context *c, size_t count, const pt_object_xform_desc *objects)
 {
 	PT_TRY
-	if (!c) return setError(PT_E_INVALID, "pt_set_scene_xform: null context");
-	if (count == 0)
-	{
-		printf("Setting an empty scene is not allowed!\n"); // Pathtracer.cpp:115
-		return PT_OK;
-	}
-	if (!objects) return setError(PT_E_INVALID, "pt_set_scene_xform: null objects");
-	std::vector<pt_object_desc> descs(count);
-	std::vector<ObjectXform> xf(count);
-	for (size_t i = 0; i < count; ++i)
-	{
-		memset(&descs[i], 0, sizeof descs[i]);
-		descs[i].type = objects[i].type;
-		descs[i].scale[0] = descs[i].scale[1] = descs[i].scale[2] = 1.0f;
-		descs[i].material = objects[i].material;
-		memset(&xf[i], 0, sizeof xf[i]);
-		memcpy(xf[i].w2l, objects[i].world_to_local, sizeof xf[i].w2l);
-		memcpy(xf[i].bmin, objects[i].aabb_min, 12);
-		memcpy(xf[i].bmax, objects[i].aabb_max, 12);
-	}
-	CompiledScene cs;
-	std::string err;
-	if (!compileScene(count, descs.data(), c->maxLeaf, cs, err, c->maxGlobal, xf.data(), c->bvhBuilder)) return setError(PT_E_LIMIT, "pt_set_scene_xform: " + err);
-	LightTable lt;
-	buildLightTable(cs, lt);
-	int r = uploadScene(c, cs, lt);
-	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs, lt);
-	return r;
+	return setScene(c, "pt_set_scene_xform", count, nullptr, objects);
 	PT_CATCH(PT_E_LIMIT)
 }
 
@@ -390,7 +388,7 @@ static int uploadTextureTable(pt_context *c)
 	memcpy(tmp, c->texHost, sizeof tmp);
 	if (!c->texUnit)
 		for (TexDesc &t : tmp) t.texObj = 0;
-	if (cudaMemcpyAsync(c->texDev, tmp, sizeof tmp, cudaMemcpyHostToDevice, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
+	if (cudaMemcpyAsync(c->texDev.p, tmp, sizeof tmp, cudaMemcpyHostToDevice, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
 		return setError(PT_E_CUDA, "pt_load_texture: table upload failed");
 	return PT_OK;
 }
@@ -399,63 +397,50 @@ static uint32_t loadTextureMemOne(pt_context *c, uint32_t width, uint32_t height
 {
 	PT_TRY
 	if (!c || !rgba || width == 0 || height == 0) return 0;
-	if (c->textureCount >= kMaxTextures) return 0; // Pathtracer.cpp:236-240
+	if (c->textures.size() >= kMaxTextures) return 0; // Pathtracer.cpp:236-240
 	if (cudaSetDevice(c->device) != cudaSuccess) return 0;
 	const size_t bytes = size_t(width) * height * (is_hdr ? 16 : 4);
-	void *dev = nullptr;
-	if (cudaMalloc(&dev, bytes) != cudaSuccess) { setError(PT_E_CUDA, "pt_load_texture: cudaMalloc failed"); return 0; }
-	if (cudaMemcpyAsync(dev, rgba, bytes, cudaMemcpyHostToDevice, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
+	Texture tex;
+	if (tex.texels.alloc(bytes) != cudaSuccess) { setError(PT_E_CUDA, "pt_load_texture: cudaMalloc failed"); return 0; }
+	if (cudaMemcpyAsync(tex.texels.p, rgba, bytes, cudaMemcpyHostToDevice, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
 	{
-		cudaFree(dev);
 		setError(PT_E_CUDA, "pt_load_texture: upload failed");
 		return 0;
 	}
-	TexDesc &t = c->texHost[c->textureCount];
-	t.texels = dev;
-	t.width = width;
-	t.height = height;
-	t.isHdr = is_hdr ? 1u : 0u;
-	t.pad = 0;
-	t.texObj = 0;
-	c->texMem.push_back(dev);
 	// the same texels behind a texture object (Pathtracer.cpp:259-288: array, wrap U / clamp V, linear filter, normalised
 	// coordinates; 8-bit texels read as normalised floats)
+	cudaChannelFormatDesc fmt = is_hdr ? cudaCreateChannelDesc<float4>() : cudaCreateChannelDesc<uchar4>();
+	cudaTextureObject_t obj = 0;
+	bool ok = cudaMallocArray(&tex.array, &fmt, width, height) == cudaSuccess;
+	const size_t pitch = size_t(width) * (is_hdr ? 16 : 4);
+	ok = ok && cudaMemcpy2DToArray(tex.array, 0, 0, rgba, pitch, pitch, height, cudaMemcpyHostToDevice) == cudaSuccess;
+	if (ok)
 	{
-		cudaChannelFormatDesc fmt = is_hdr ? cudaCreateChannelDesc<float4>() : cudaCreateChannelDesc<uchar4>();
-		cudaArray_t arr = nullptr;
-		cudaTextureObject_t obj = 0;
-		bool ok = cudaMallocArray(&arr, &fmt, width, height) == cudaSuccess;
-		const size_t pitch = size_t(width) * (is_hdr ? 16 : 4);
-		ok = ok && cudaMemcpy2DToArray(arr, 0, 0, rgba, pitch, pitch, height, cudaMemcpyHostToDevice) == cudaSuccess;
-		if (ok)
-		{
-			cudaResourceDesc rd;
-			memset(&rd, 0, sizeof rd);
-			rd.resType = cudaResourceTypeArray;
-			rd.res.array.array = arr;
-			cudaTextureDesc td;
-			memset(&td, 0, sizeof td);
-			td.addressMode[0] = cudaAddressModeWrap;
-			td.addressMode[1] = cudaAddressModeClamp;
-			td.filterMode = cudaFilterModeLinear;
-			td.readMode = is_hdr ? cudaReadModeElementType : cudaReadModeNormalizedFloat;
-			td.normalizedCoords = 1;
-			ok = cudaCreateTextureObject(&obj, &rd, &td, nullptr) == cudaSuccess;
-		}
-		if (!ok)
-		{
-			if (arr) cudaFreeArray(arr);
-			cudaGetLastError();
-			setError(PT_E_CUDA, "pt_load_texture: texture object creation failed");
-			return 0;
-		}
-		t.texObj = (unsigned long long)obj;
-		c->texArrays.push_back(arr);
-		c->texObjects.push_back(obj);
+		cudaResourceDesc rd;
+		memset(&rd, 0, sizeof rd);
+		rd.resType = cudaResourceTypeArray;
+		rd.res.array.array = tex.array;
+		cudaTextureDesc td;
+		memset(&td, 0, sizeof td);
+		td.addressMode[0] = cudaAddressModeWrap;
+		td.addressMode[1] = cudaAddressModeClamp;
+		td.filterMode = cudaFilterModeLinear;
+		td.readMode = is_hdr ? cudaReadModeElementType : cudaReadModeNormalizedFloat;
+		td.normalizedCoords = 1;
+		ok = cudaCreateTextureObject(&obj, &rd, &td, nullptr) == cudaSuccess;
 	}
-	++c->textureCount;
-	if (uploadTextureTable(c) != PT_OK) { --c->textureCount; return 0; }
-	return c->textureCount;
+	if (!ok)
+	{
+		cudaGetLastError();
+		setError(PT_E_CUDA, "pt_load_texture: texture object creation failed");
+		return 0;
+	}
+	tex.object = obj;
+	// the record is complete: it becomes the next handle
+	c->texHost[c->textures.size()] = TexDesc{tex.texels.p, width, height, is_hdr ? 1u : 0u, 0u, (unsigned long long)obj};
+	c->textures.push_back(std::move(tex));
+	if (uploadTextureTable(c) != PT_OK) { c->textures.pop_back(); return 0; }
+	return uint32_t(c->textures.size());
 	PT_CATCH(0u)
 }
 
@@ -472,7 +457,7 @@ uint32_t pt_load_texture(pt_context *c, const char *path)
 {
 	PT_TRY
 	if (!c || !path) return 0;
-	if (c->textureCount >= kMaxTextures) return 0;
+	if (c->textures.size() >= kMaxTextures) return 0;
 	Image img;
 	std::string err;
 	if (!readImage(path, img, err)) { g_lastError = err; return 0; } // failed load -> handle 0, no error (Pathtracer.cpp:253-257)
@@ -491,15 +476,15 @@ int pt_set_skybox(pt_context *c, uint32_t handle)
 static SceneDev sceneDev(const pt_context *c)
 {
 	SceneDev s;
-	s.sceneBlob = c->sceneBlob;
+	s.sceneBlob = c->sceneBlob.as<float4>();
 	s.mats = c->mats;
-	s.textures = c->texDev;
+	s.textures = c->texDev.as<TexDesc>();
 	s.nodeCount = c->nodeCount;
 	s.primCount = c->primCount;
 	s.globalCount = c->globalCount;
 	s.treeNodeCount = c->treeNodeCount;
-	s.texCount = c->textureCount;
-	s.skybox = (c->skybox <= c->textureCount) ? c->skybox : 0;
+	s.texCount = uint32_t(c->textures.size());
+	s.skybox = (c->skybox <= s.texCount) ? c->skybox : 0;
 	return s;
 }
 
@@ -507,7 +492,7 @@ static SceneDev sceneDev(const pt_context *c)
 // linear device copy the loader keeps)
 static int ensureEnvDistribution(pt_context *c, uint32_t handle)
 {
-	if (c->envHandle == handle && c->envAlias) return PT_OK;
+	if (c->envHandle == handle && c->envAlias.p) return PT_OK;
 	const TexDesc &t = c->texHost[handle - 1];
 	const size_t bytes = size_t(t.width) * t.height * (t.isHdr ? 16 : 4);
 	std::vector<unsigned char> texels(bytes);
@@ -515,13 +500,15 @@ static int ensureEnvDistribution(pt_context *c, uint32_t handle)
 	CK(cudaStreamSynchronize(c->stream));
 	EnvDistribution d;
 	buildEnvDistribution(t.width, t.height, t.isHdr != 0, texels.data(), d);
-	if (c->envAlias) { CK(cudaFree(c->envAlias)); c->envAlias = nullptr; }
-	if (c->envDensity) { CK(cudaFree(c->envDensity)); c->envDensity = nullptr; }
-	CK(cudaMalloc(&c->envAlias, d.alias.size() * 4));
-	CK(cudaMalloc(&c->envDensity, d.density.size() * 4));
-	CK(cudaMemcpyAsync(c->envAlias, d.alias.data(), d.alias.size() * 4, cudaMemcpyHostToDevice, c->stream));
-	CK(cudaMemcpyAsync(c->envDensity, d.density.data(), d.density.size() * 4, cudaMemcpyHostToDevice, c->stream));
+	DevBuf alias, density;
+	CK(alias.alloc(d.alias.size() * 4));
+	CK(density.alloc(d.density.size() * 4));
+	CK(cudaMemcpyAsync(alias.p, d.alias.data(), d.alias.size() * 4, cudaMemcpyHostToDevice, c->stream));
+	CK(cudaMemcpyAsync(density.p, d.density.data(), d.density.size() * 4, cudaMemcpyHostToDevice, c->stream));
 	CK(cudaStreamSynchronize(c->stream));
+	// the tables of `handle` are complete: they replace the cached ones together with their size and handle
+	c->envAlias = std::move(alias);
+	c->envDensity = std::move(density);
 	c->envCols = d.cols;
 	c->envRows = d.rows;
 	c->envHandle = handle;
@@ -541,7 +528,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 	}
 	c->timingMs = 0.0f;
 	int launches = 0, usedSmem = 0;
-	CK(cudaMemsetAsync(c->counters, 0, kCtrCount * sizeof(unsigned long long), c->stream));
+	CK(cudaMemsetAsync(c->counters.p, 0, kCtrCount * sizeof(unsigned long long), c->stream));
 	const bool run = c->nodeCount >= 1 && c->primCount >= 1 && spp > 0; // Pathtracer.cpp:174
 	if (run)
 	{
@@ -549,7 +536,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.scene = sceneDev(c);
 		p.cam = *camera;
 		p.accum = c->accum;
-		p.counters = c->counters;
+		p.counters = c->counters.as<unsigned long long>();
 		p.width = c->width;
 		p.height = c->height;
 		p.spp = spp;
@@ -585,29 +572,31 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		{
 			const int rc = ensureEnvDistribution(c, p.scene.skybox);
 			if (rc != PT_OK) return rc;
-			p.scene.env.alias = static_cast<const uint2 *>(c->envAlias);
-			p.scene.env.density = c->envDensity;
+			p.scene.env.alias = c->envAlias.as<const uint2>();
+			p.scene.env.density = c->envDensity.as<float>();
 			p.scene.env.cols = c->envCols;
 			p.scene.env.rows = c->envRows;
 			c->launch.twin = Twin::EnvIS;
 		}
 		if (c->noJitter)
 		{
-			if (!c->centreUV)
+			if (!c->centreUV.p)
 			{
 				// (this file is compiled without FMA contraction: the division is the IEEE one of the reference's primary pass)
 				std::vector<float> uv(size_t(c->width) + c->height);
 				for (uint32_t x = 0; x < c->width; ++x) uv[x] = (float(x) + 0.5f) / float(c->width);
 				for (uint32_t y = 0; y < c->height; ++y) uv[c->width + y] = (float(y) + 0.5f) / float(c->height);
-				CK(cudaMalloc(&c->centreUV, uv.size() * sizeof(float)));
-				CK(cudaMemcpy(c->centreUV, uv.data(), uv.size() * sizeof(float), cudaMemcpyHostToDevice));
+				DevBuf centres;
+				CK(centres.alloc(uv.size() * sizeof(float)));
+				CK(cudaMemcpy(centres.p, uv.data(), uv.size() * sizeof(float), cudaMemcpyHostToDevice));
+				c->centreUV = std::move(centres);
 			}
-			p.centreU = c->centreUV;
-			p.centreV = c->centreUV + c->width;
+			p.centreU = c->centreUV.as<float>();
+			p.centreV = c->centreUV.as<float>() + c->width;
 			p.aids |= kAidPixelCentre;
 		}
-		p.firstHitIndex = c->firstHit ? c->firstHitIndex : nullptr;
-		p.firstHitT = c->firstHit ? c->firstHitT : nullptr;
+		p.firstHitIndex = c->firstHit ? c->firstHitIndex.as<int32_t>() : nullptr;
+		p.firstHitT = c->firstHit ? c->firstHitT.as<float>() : nullptr;
 		if (c->firstHit) p.aids |= kAidFirstHit;
 		if (p.aids)
 		{
@@ -621,7 +610,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 			// a scene without emitters renders with the plain kernel: the same bits as without the option
 			if (c->lightCount != 0)
 			{
-				p.lights.recs = c->lightRecs;
+				p.lights.recs = c->lightRecs.as<float4>();
 				p.lights.count = c->lightCount;
 				c->launch.twin = Twin::LightIS;
 			}
@@ -641,7 +630,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 	if (run)
 	{
 		unsigned long long h[kCtrCount];
-		CK(cudaMemcpy(h, c->counters, sizeof h, cudaMemcpyDeviceToHost));
+		CK(cudaMemcpy(h, c->counters.p, sizeof h, cudaMemcpyDeviceToHost));
 		{
 			const unsigned long long all = (unsigned long long)c->width * c->height;
 			const unsigned long long own = all > c->pixelOffset ? (all - c->pixelOffset + c->pixelStride - 1u) / c->pixelStride : 0ull;
@@ -843,65 +832,56 @@ int pt_render_vectors(pt_context *c, const pt_camera_vectors *camera, uint32_t s
 
 float pt_get_timing_ms(const pt_context *c) { return c ? c->timingMs : 0.0f; }
 
-static const float *readHdr(pt_context *c, float scale)
+// the image getters: the accumulation x scale (HDR) or tone-mapped (LDR) into device staging, copied to pinned host memory (both
+// allocated by the first call)
+static const void *readBack(pt_context *c, bool ldr, float scale)
 {
 	if (cudaSetDevice(c->device) != cudaSuccess) return nullptr;
 	const uint32_t px = c->width * c->height;
-	if ((!c->scaledDev && cudaMalloc(&c->scaledDev, size_t(px) * sizeof(float4)) != cudaSuccess) ||
-	    (!c->hostHdr && cudaMallocHost(&c->hostHdr, size_t(px) * sizeof(float4)) != cudaSuccess))
+	const size_t bytes = size_t(px) * (ldr ? sizeof(uchar4) : sizeof(float4));
+	DevBuf &dev = ldr ? c->ldrDev : c->scaledDev;
+	HostBuf &host = ldr ? c->hostLdr : c->hostHdr;
+	const std::string fn = ldr ? "pt_get_ldr: " : "pt_get_hdr: ";
+	if ((!dev.p && dev.alloc(bytes) != cudaSuccess) || (!host.p && host.alloc(bytes) != cudaSuccess))
 	{
-		setError(PT_E_CUDA, std::string("pt_get_hdr: ") + cudaGetErrorString(cudaGetLastError()));
+		setError(PT_E_CUDA, fn + cudaGetErrorString(cudaGetLastError()));
 		return nullptr;
 	}
-	launchScale(c->imageSource ? c->imageSource : c->accum, c->scaledDev, px, scale, c->stream);
-	if (cudaMemcpyAsync(c->hostHdr, c->scaledDev, size_t(px) * sizeof(float4), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
-	    cudaStreamSynchronize(c->stream) != cudaSuccess)
+	const float4 *src = c->imageSource ? c->imageSource : c->accum;
+	if (ldr) launchTonemap(src, dev.as<uchar4>(), px, scale, c->stream);
+	else launchScale(src, dev.as<float4>(), px, scale, c->stream);
+	if (cudaMemcpyAsync(host.p, dev.p, bytes, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
 	{
-		setError(PT_E_CUDA, std::string("pt_get_hdr: ") + cudaGetErrorString(cudaGetLastError()));
+		setError(PT_E_CUDA, fn + cudaGetErrorString(cudaGetLastError()));
 		return nullptr;
 	}
-	return c->hostHdr;
+	return host.p;
 }
 
 const float *pt_get_hdr(pt_context *c)
 {
 	if (!c) return nullptr;
-	return readHdr(c, 1.0f / fmaxf(float(c->accumulatedFrames), 1.0f)); // Pathtracer.cpp:307
+	return static_cast<const float *>(readBack(c, false, 1.0f / fmaxf(float(c->accumulatedFrames), 1.0f))); // Pathtracer.cpp:307
 }
 
 const float *pt_get_hdr_mean(pt_context *c)
 {
 	if (!c) return nullptr;
-	return readHdr(c, 1.0f / fmaxf(float(c->totalSamples), 1.0f));
+	return static_cast<const float *>(readBack(c, false, 1.0f / fmaxf(float(c->totalSamples), 1.0f)));
 }
 
 const float *pt_get_hdr_sum(pt_context *c)
 {
 	if (!c) return nullptr;
-	return readHdr(c, 1.0f);
+	return static_cast<const float *>(readBack(c, false, 1.0f));
 }
 
 const uint8_t *pt_get_ldr(pt_context *c)
 {
 	if (!c) return nullptr;
-	if (cudaSetDevice(c->device) != cudaSuccess) return nullptr;
-	const uint32_t px = c->width * c->height;
-	if ((!c->ldrDev && cudaMalloc(&c->ldrDev, size_t(px) * sizeof(uchar4)) != cudaSuccess) ||
-	    (!c->hostLdr && cudaMallocHost(&c->hostLdr, size_t(px) * sizeof(uchar4)) != cudaSuccess))
-	{
-		setError(PT_E_CUDA, std::string("pt_get_ldr: ") + cudaGetErrorString(cudaGetLastError()));
-		return nullptr;
-	}
 	// tonemap.cu:17 divides by float(accumulatedSampleCount) via reciprocal-multiply; 0 frames -> division by zero in the
 	// reference; here the accumulation is zero in that case and the scale is clamped like getHDRImageData's
-	launchTonemap(c->imageSource ? c->imageSource : c->accum, c->ldrDev, px, 1.0f / fmaxf(float(c->accumulatedFrames), 1.0f), c->stream);
-	if (cudaMemcpyAsync(c->hostLdr, c->ldrDev, size_t(px) * sizeof(uchar4), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
-	    cudaStreamSynchronize(c->stream) != cudaSuccess)
-	{
-		setError(PT_E_CUDA, std::string("pt_get_ldr: ") + cudaGetErrorString(cudaGetLastError()));
-		return nullptr;
-	}
-	return c->hostLdr;
+	return static_cast<const uint8_t *>(readBack(c, true, 1.0f / fmaxf(float(c->accumulatedFrames), 1.0f)));
 }
 
 static int setOptionOne(pt_context *c, const char *key, double value)
@@ -946,16 +926,19 @@ static int setOptionOne(pt_context *c, const char *key, double value)
 	else if (k == "light_is") c->lightIS = value != 0;
 	else if (k == "first_hit")
 	{
-		c->firstHit = value != 0;
-		if (c->firstHit && !c->firstHitIndex)
+		if (value != 0 && !c->firstHitIndex.p)
 		{
 			const size_t px = size_t(c->width) * c->height;
 			CK(cudaSetDevice(c->device));
-			CK(cudaMalloc(&c->firstHitIndex, px * 4));
-			CK(cudaMalloc(&c->firstHitT, px * 4));
-			CK(cudaMemset(c->firstHitIndex, 0xff, px * 4));
-			CK(cudaMemset(c->firstHitT, 0, px * 4));
+			DevBuf index, t;
+			CK(index.alloc(px * 4));
+			CK(t.alloc(px * 4));
+			CK(cudaMemset(index.p, 0xff, px * 4));
+			CK(cudaMemset(t.p, 0, px * 4));
+			c->firstHitIndex = std::move(index);
+			c->firstHitT = std::move(t);
 		}
+		c->firstHit = value != 0;
 	}
 	else if (k == "tex_unit") { c->texUnit = value != 0; return uploadTextureTable(c); }
 	else return setError(PT_E_INVALID, "pt_set_option: unknown option " + k);
@@ -1063,11 +1046,11 @@ int pt_trace_rays(pt_context *c, size_t n, const float *origins, const float *di
 int pt_get_first_hit(pt_context *c, int32_t *hit_index, float *hit_t)
 {
 	if (!c || !hit_index || !hit_t) return setError(PT_E_INVALID, "pt_get_first_hit: bad arguments");
-	if (!c->firstHitIndex) return setError(PT_E_INVALID, "pt_get_first_hit: option first_hit was not set before pt_render");
+	if (!c->firstHitIndex.p) return setError(PT_E_INVALID, "pt_get_first_hit: option first_hit was not set before pt_render");
 	const size_t px = size_t(c->width) * c->height;
 	CK(cudaSetDevice(c->device));
-	CK(cudaMemcpyAsync(hit_index, c->firstHitIndex, px * 4, cudaMemcpyDeviceToHost, c->stream));
-	CK(cudaMemcpyAsync(hit_t, c->firstHitT, px * 4, cudaMemcpyDeviceToHost, c->stream));
+	CK(cudaMemcpyAsync(hit_index, c->firstHitIndex.p, px * 4, cudaMemcpyDeviceToHost, c->stream));
+	CK(cudaMemcpyAsync(hit_t, c->firstHitT.p, px * 4, cudaMemcpyDeviceToHost, c->stream));
 	CK(cudaStreamSynchronize(c->stream));
 	return PT_OK;
 }
