@@ -55,6 +55,7 @@ class Oracle:
         L.orc_uniform.argtypes = [C.c_uint32]
         L.orc_texture_lookup.argtypes = [C.c_void_p, C.c_uint32, C.c_float, C.c_float, C.c_void_p]
         self.n = len(objects)
+        self.env_is = self.light_is = False
         self._arr = object_array(objects)
         self.s = L.orc_scene_create(self.n, C.byref(self._arr))
 
@@ -75,8 +76,11 @@ class Oracle:
 
     def set_env_is(self, on):
         """the product's option "env_is" (not the reference): sky importance sampling + multiple importance sampling"""
+        if on and self.light_is:
+            raise ValueError("env_is and light_is cannot be combined (pt_render refuses it too)")
         self.L.orc_set_env_is.argtypes = [C.c_void_p, C.c_int]
         self.L.orc_set_env_is(self.s, int(on))
+        self.env_is = bool(on)
 
     def env_tables(self):
         """(cols, rows, q, alias, density) of the sky distribution built by set_env_is(1)"""
@@ -96,6 +100,34 @@ class Oracle:
         row = np.zeros(6, np.float32)
         for i in range(r.shape[0]):
             self.L.orc_env_sample(self.s, int(r[i, 0]), int(r[i, 1]), int(r[i, 2]), _p(row))
+            out[i] = row
+        return out
+
+    def set_light_is(self, on):
+        """the product's option "light_is" (not the reference): emitter importance sampling + multiple importance sampling"""
+        if on and self.env_is:
+            raise ValueError("env_is and light_is cannot be combined (pt_render refuses it too)")
+        self.L.orc_set_light_is.argtypes = [C.c_void_p, C.c_int]
+        self.L.orc_set_light_is(self.s, int(on))
+        self.light_is = bool(on)
+
+    def light_table(self):
+        """(scene_index, prob, q, alias) of the emitter table built by set_light_is(1)"""
+        self.L.orc_light_table.argtypes = [C.c_void_p] * 5
+        self.L.orc_light_table.restype = C.c_uint32
+        n = self.L.orc_light_table(self.s, None, None, None, None)
+        idx, prob, q, alias = np.zeros(n, np.uint32), np.zeros(n, np.float32), np.zeros(n, np.float32), np.zeros(n, np.uint32)
+        self.L.orc_light_table(self.s, _p(idx), _p(prob), _p(q), _p(alias))
+        return idx, prob, q, alias
+
+    def light_sample_points(self, q):
+        """q: (n, 4) uint32 random words -> (n, 8): world point, area pdf without the selection probability, emitter, local point"""
+        self.L.orc_light_sample_point.argtypes = [C.c_void_p] * 3
+        q = np.ascontiguousarray(q, np.uint32)
+        out = np.zeros((q.shape[0], 8), np.float32)
+        row = np.zeros(8, np.float32)
+        for i in range(q.shape[0]):
+            self.L.orc_light_sample_point(self.s, _p(q[i]), _p(row))
             out[i] = row
         return out
 

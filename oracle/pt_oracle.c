@@ -39,6 +39,16 @@ typedef struct { aabb_t box; uint32_t offset; uint32_t countAxis; } node_t; /* B
 
 typedef struct { uint32_t w, h; int hdr; float *f; uint8_t *b; } tex_t;
 
+/* NOT THE REFERENCE: one emitter of the "light_is" estimator (csrc/light_sampling.h) */
+typedef struct
+{
+	float m[12];    /* local -> world rows */
+	float pdfScale; /* P_sel / (A_l |det M|) */
+	float q;        /* alias threshold */
+	uint32_t alias, scene, type;
+	float prob;
+} light_t;
+
 struct orc_scene
 {
 	size_t n;
@@ -49,6 +59,9 @@ struct orc_scene
 	tex_t tex[64]; uint32_t texCount; uint32_t skybox;
 	/* NOT THE REFERENCE: importance distribution of the sky (option "env_is" of the product, csrc/env_sampling.h) */
 	int envIS; uint32_t envCols, envRows; float *envQ; uint32_t *envAlias; float *envDensity;
+	/* NOT THE REFERENCE: emitter table (option "light_is" of the product, csrc/light_sampling.h); lightCount is 0 unless the option is
+	 * on and the scene emits.  lightOf: scene index -> emitter index, -1: not an emitter */
+	uint32_t lightCount; light_t *lights; int32_t *lightOf;
 };
 
 /* ---- vec3.inl ------------------------------------------------------------------------------------------ */
@@ -565,7 +578,7 @@ static inline v3 lerp3(v3 x, v3 y, float a) { return vadd(vscale(1.0f - a, x), v
 
 /* Material::sample  Material.inl:20-60 (+ sampleLambert :67-72, sampleGGX :74-99, sampleLambertGGX :101-144).
  * Returns attenuation; *pdf, *scatteredDir (world).  baseColor already texture-resolved by the caller. */
-/* NOT THE REFERENCE (a helper of the "env_is" estimator): attenuation and pdf of Material::sample for a GIVEN tangent-space
+/* NOT THE REFERENCE (a helper of the "env_is" and "light_is" estimators): attenuation and pdf of Material::sample for a GIVEN tangent-space
  * direction - the same expressions as in materialSample below (Material.inl:67-72, :89-98, :124-143), which are functions of the
  * view vector and the scattered direction alone. */
 static v3 materialEval(uint32_t mtype, v3 baseColor, float roughness, float metalness, v3 Vv, v3 sdir, float *pdf)
@@ -729,6 +742,227 @@ static float envPdf(const orc_scene *s, float u, float v, float dirY)
 	return s->envDensity[row * s->envCols + col] * (1.0f / sqrtf(fmaxf(1.0f - dirY * dirY, 1e-12f)));
 }
 
+/* ---- NOT THE REFERENCE: the emitters' importance distribution (the product's option "light_is"; csrc/light_sampling.h states the
+ * estimator).  Restated here so that the CUDA path can be checked path for path: one alias table over the objects with a non-zero
+ * emissive channel, weight = mean emission x world area (the same double arithmetic as the product; Vose, work lists filled in index
+ * order, used as stacks), a uniform point on the chosen emitter's surface with its solid-angle pdf, and a shadow ray through the BVH
+ * that stops just short of the point. ---- */
+static double lightLocalArea(uint32_t type)
+{
+	const double pi = 3.14159265358979323846;
+	switch (type)
+	{
+	case PT_SPHERE: return 4.0 * pi;
+	case PT_CYLINDER: return 4.0 * pi;
+	case PT_DISK: return pi;
+	case PT_CONE: return 2.0 * sqrt(2.0) * pi;
+	case PT_PARABOLOID: return pi * (5.0 * sqrt(5.0) - 1.0) / 6.0;
+	case PT_QUAD: return 4.0;
+	default: return 24.0;
+	}
+}
+static void lightBuild(orc_scene *s)
+{
+	s->lightOf = (int32_t *)malloc((s->n ? s->n : 1) * sizeof(int32_t));
+	uint32_t n = 0;
+	for (size_t i = 0; i < s->n; ++i)
+	{
+		const obj_t *o = &s->sceneObjs[i];
+		s->lightOf[i] = (o->emissive.x != 0.0f || o->emissive.y != 0.0f || o->emissive.z != 0.0f) ? (int32_t)n++ : -1;
+	}
+	s->lights = (light_t *)calloc(n ? n : 1, sizeof(light_t));
+	double *w = (double *)calloc(n ? n : 1, sizeof(double)), *det = (double *)calloc(n ? n : 1, sizeof(double)), *scaled = (double *)calloc(n ? n : 1, sizeof(double));
+	double total = 0.0;
+	for (size_t i = 0; i < s->n; ++i)
+	{
+		if (s->lightOf[i] < 0) continue;
+		const uint32_t k = (uint32_t)s->lightOf[i];
+		const obj_t *o = &s->sceneObjs[i];
+		light_t *L = &s->lights[k];
+		L->scene = (uint32_t)i;
+		L->type = o->type <= PT_CUBE ? o->type : PT_SPHERE;
+		const float *rows[3] = { o->r0, o->r1, o->r2 };
+		double W[3][3], tr[3];
+		for (int r = 0; r < 3; ++r) { for (int c = 0; c < 3; ++c) W[r][c] = rows[r][c]; tr[r] = rows[r][3]; }
+		const double dW = W[0][0] * (W[1][1] * W[2][2] - W[1][2] * W[2][1]) - W[0][1] * (W[1][0] * W[2][2] - W[1][2] * W[2][0]) +
+		                  W[0][2] * (W[1][0] * W[2][1] - W[1][1] * W[2][0]);
+		if (!(isfinite(dW) && dW != 0.0)) continue;
+		double M[3][3];
+		M[0][0] = (W[1][1] * W[2][2] - W[1][2] * W[2][1]) / dW;
+		M[0][1] = (W[0][2] * W[2][1] - W[0][1] * W[2][2]) / dW;
+		M[0][2] = (W[0][1] * W[1][2] - W[0][2] * W[1][1]) / dW;
+		M[1][0] = (W[1][2] * W[2][0] - W[1][0] * W[2][2]) / dW;
+		M[1][1] = (W[0][0] * W[2][2] - W[0][2] * W[2][0]) / dW;
+		M[1][2] = (W[0][2] * W[1][0] - W[0][0] * W[1][2]) / dW;
+		M[2][0] = (W[1][0] * W[2][1] - W[1][1] * W[2][0]) / dW;
+		M[2][1] = (W[0][1] * W[2][0] - W[0][0] * W[2][1]) / dW;
+		M[2][2] = (W[0][0] * W[1][1] - W[0][1] * W[1][0]) / dW;
+		for (int r = 0; r < 3; ++r)
+		{
+			for (int c = 0; c < 3; ++c) L->m[4 * r + c] = (float)M[r][c];
+			L->m[4 * r + 3] = (float)(-(M[r][0] * tr[0] + M[r][1] * tr[1] + M[r][2] * tr[2]));
+		}
+		const double dM = fabs(1.0 / dW);
+		double len[3];
+		for (int r = 0; r < 3; ++r) len[r] = sqrt(W[r][0] * W[r][0] + W[r][1] * W[r][1] + W[r][2] * W[r][2]);
+		double area;
+		if (L->type == PT_QUAD || L->type == PT_DISK) area = lightLocalArea(L->type) * dM * len[1];
+		else if (L->type == PT_CUBE) area = 8.0 * dM * (len[0] + len[1] + len[2]);
+		else area = lightLocalArea(L->type) * cbrt(dM * dM);
+		const double mean = ((double)o->emissive.x + (double)o->emissive.y + (double)o->emissive.z) / 3.0;
+		w[k] = mean > 0.0 && isfinite(area) ? mean * area : 0.0;
+		det[k] = dM;
+		total += w[k];
+	}
+	if (!(total > 0.0 && isfinite(total))) n = 0;
+	s->lightCount = n;
+	for (uint32_t k = 0; k < n; ++k)
+	{
+		const double P = w[k] / total;
+		s->lights[k].pdfScale = P > 0.0 ? (float)(P / (lightLocalArea(s->lights[k].type) * det[k])) : 0.0f;
+		s->lights[k].prob = (float)P;
+		scaled[k] = P * (double)n;
+	}
+	uint32_t *small = (uint32_t *)malloc((n ? n : 1) * sizeof(uint32_t)), *large = (uint32_t *)malloc((n ? n : 1) * sizeof(uint32_t));
+	size_t ns = 0, nl = 0;
+	for (uint32_t i = 0; i < n; ++i) { if (scaled[i] < 1.0) small[ns++] = i; else large[nl++] = i; }
+#define LIGHT_PUT(i, qq, other) do { double q_ = (qq); s->lights[i].q = (float)(q_ < 0.0 ? 0.0 : (q_ > 1.0 ? 1.0 : q_)); s->lights[i].alias = (other); } while (0)
+	while (ns > 0 && nl > 0)
+	{
+		const uint32_t sm = small[--ns], lg = large[nl - 1];
+		LIGHT_PUT(sm, scaled[sm], lg);
+		scaled[lg] = (scaled[lg] + scaled[sm]) - 1.0;
+		if (scaled[lg] < 1.0) { --nl; small[ns++] = lg; }
+	}
+	for (size_t i = 0; i < nl; ++i) LIGHT_PUT(large[i], 1.0, large[i]);
+	for (size_t i = 0; i < ns; ++i) LIGHT_PUT(small[i], 1.0, small[i]);
+#undef LIGHT_PUT
+	free(small); free(large); free(w); free(det); free(scaled);
+}
+static v3 lightUnitNormal(uint32_t type, v3 lp)
+{
+	v3 n;
+	switch (type)
+	{
+	case PT_SPHERE: n = lp; break;
+	case PT_CYLINDER: n = V(lp.x, 0.0f, lp.z); break;
+	case PT_CONE: n = V(lp.x, -lp.y, lp.z); break;
+	case PT_PARABOLOID: n = V(2.0f * lp.x, -1.0f, 2.0f * lp.z); break;
+	case PT_CUBE:
+	{
+		const float ax = fabsf(lp.x), ay = fabsf(lp.y), az = fabsf(lp.z);
+		if (ax > ay && ax > az) n = V(1.0f, 0.0f, 0.0f);
+		else if (ay > ax && ay > az) n = V(0.0f, 1.0f, 0.0f);
+		else n = V(0.0f, 0.0f, 1.0f);
+		break;
+	}
+	default: n = V(0.0f, 1.0f, 0.0f); break;
+	}
+	return vnorm(n);
+}
+/* W^T n_l: the (unnormalised) world normal */
+static v3 lightWorldNormal(const obj_t *o, v3 nl)
+{
+	return V(nl.x * o->r0[0] + nl.y * o->r1[0] + nl.z * o->r2[0], nl.x * o->r0[1] + nl.y * o->r1[1] + nl.z * o->r2[1], nl.x * o->r0[2] + nl.y * o->r1[2] + nl.z * o->r2[2]);
+}
+/* local point of the canonical surface from two uniforms and one word (face / nappe) */
+static v3 lightLocalPoint(uint32_t type, float u, float v, uint32_t w)
+{
+	const float ph = 2.0f * PI_F * v, cp = cosf(ph), sp = sinf(ph);
+	switch (type)
+	{
+	case PT_SPHERE: { const float y = 1.0f - 2.0f * u, r = sqrtf(fmaxf(1.0f - y * y, 0.0f)); return V(r * cp, y, r * sp); }
+	case PT_CYLINDER: return V(cp, 2.0f * u - 1.0f, sp);
+	case PT_DISK: { const float r = sqrtf(u); return V(r * cp, 0.0f, r * sp); }
+	case PT_CONE: { const float h = sqrtf(u); return V(h * cp, (w & 1u) ? h : -h, h * sp); }
+	case PT_PARABOLOID:
+	{
+		const float g = cbrtf(1.0f + u * 10.180339887498949f);
+		const float r2 = fmaxf((g * g - 1.0f) * 0.25f, 0.0f), r = sqrtf(r2);
+		return V(r * cp, r2, r * sp);
+	}
+	case PT_QUAD: return V(2.0f * u - 1.0f, 0.0f, 2.0f * v - 1.0f);
+	default:
+	{
+		const uint32_t face = (uint32_t)(((uint64_t)w * 6u) >> 32);
+		const float s = (face & 1u) ? 1.0f : -1.0f, a = 2.0f * u - 1.0f, b = 2.0f * v - 1.0f;
+		return face < 2u ? V(s, a, b) : (face < 4u ? V(a, s, b) : V(a, b, s));
+	}
+	}
+}
+/* one light sample from the four words q seen from p: emitter k, world point x, unit direction, distance, solid-angle pdf; 0 = unusable */
+static int lightSample(const orc_scene *s, const uint32_t q[4], v3 p, uint32_t *k, v3 *x, v3 *wdir, float *dist, float *pdf)
+{
+	const uint64_t xx = (uint64_t)q[0] * s->lightCount;
+	const uint32_t i = (uint32_t)(xx >> 32);
+	const float frac = (float)(uint32_t)xx * 2.3283064365386963e-10f;
+	*k = frac < s->lights[i].q ? i : s->lights[i].alias;
+	const light_t *L = &s->lights[*k];
+	const v3 lp = lightLocalPoint(L->type, orc_uniform(q[1]), orc_uniform(q[2]), q[3]);
+	*x = V(L->m[0] * lp.x + L->m[1] * lp.y + L->m[2] * lp.z + L->m[3], L->m[4] * lp.x + L->m[5] * lp.y + L->m[6] * lp.z + L->m[7],
+	       L->m[8] * lp.x + L->m[9] * lp.y + L->m[10] * lp.z + L->m[11]);
+	const v3 dv = vsub(*x, p);
+	const float d2 = vdot(dv, dv);
+	*dist = sqrtf(d2);
+	*wdir = vscale(1.0f / *dist, dv);
+	const v3 wn = lightWorldNormal(&s->sceneObjs[L->scene], lightUnitNormal(L->type, lp));
+	*pdf = L->pdfScale * d2 / fmaxf(fabsf(vdot(wn, *wdir)), 1e-30f);
+	return d2 > 0.0f && *pdf > 0.0f && *pdf < 3.0e38f;
+}
+/* solid-angle pdf of the light sampler for a BSDF-sampled ray that hit emitter L (object o) at t */
+static float lightPdf(const light_t *L, const obj_t *o, ray_t ray, float t)
+{
+	v3 lo;
+	lo.x = vdot(ray.o, V(o->r0[0], o->r0[1], o->r0[2])) + o->r0[3];
+	lo.y = vdot(ray.o, V(o->r1[0], o->r1[1], o->r1[2])) + o->r1[3];
+	lo.z = vdot(ray.o, V(o->r2[0], o->r2[1], o->r2[2])) + o->r2[3];
+	const v3 ld = V(vdot(ray.d, V(o->r0[0], o->r0[1], o->r0[2])), vdot(ray.d, V(o->r1[0], o->r1[1], o->r1[2])), vdot(ray.d, V(o->r2[0], o->r2[1], o->r2[2])));
+	const v3 lp = vadd(lo, vscale(t, ld));
+	const v3 wn = lightWorldNormal(o, lightUnitNormal(L->type, lp));
+	return L->pdfScale * t * t / fmaxf(fabsf(vdot(wn, ray.d)), 1e-30f);
+}
+/* the shadow ray of a light sample: any primitive hit in (tMin, tMax] */
+static int occludedBVH(const orc_scene *s, ray_t r, float tMin, float tMax)
+{
+	uint32_t stack[64], sp = 0, cur = 0;
+	if (s->nodeCount == 0) return 0;
+	v3 inv;
+	inv.x = 1.0f / (r.d.x != 0.0f ? r.d.x : 1e-7f);
+	inv.y = 1.0f / (r.d.y != 0.0f ? r.d.y : 1e-7f);
+	inv.z = 1.0f / (r.d.z != 0.0f ? r.d.z : 1e-7f);
+	int neg[3] = { inv.x < 0.0f, inv.y < 0.0f, inv.z < 0.0f };
+	for (;;)
+	{
+		const node_t *node = &s->nodes[cur];
+		if (aabbSlab(node->box, r, tMin, tMax, NULL))
+		{
+			const uint32_t pc = node->countAxis >> 16;
+			if (pc > 0)
+			{
+				for (uint32_t i = 0; i < pc; ++i)
+				{
+					hit_t rec;
+					if (hitObject(&s->objs[node->offset + i], r, tMin, tMax, &rec) && rec.t <= tMax) return 1;
+				}
+				if (sp == 0) break;
+				cur = stack[--sp];
+			}
+			else
+			{
+				int isNeg = neg[(node->countAxis >> 8) & 0xFF];
+				stack[sp++] = isNeg ? (cur + 1) : node->offset;
+				cur = isNeg ? node->offset : (cur + 1);
+			}
+		}
+		else
+		{
+			if (sp == 0) break;
+			cur = stack[--sp];
+		}
+	}
+	return 0;
+}
+
 /* getColor  kernels/trace.cu:101-156 */
 static v3 getColor(const orc_scene *s, ray_t ray, uint32_t pixel, uint32_t sample, uint32_t k0, uint32_t k1, const uint32_t rng0[4], int maxBounces, uint64_t *rays)
 {
@@ -760,7 +994,11 @@ static v3 getColor(const orc_scene *s, ray_t ray, uint32_t pixel, uint32_t sampl
 			break;
 		}
 		const obj_t *o = &s->objs[elem];
-		L = vadd(L, vmul(throughput, o->emissive));
+		v3 em = o->emissive;
+		const int32_t ek = s->lightCount ? s->lightOf[s->toScene[elem]] : -1;
+		if (it > 0 && ek >= 0) /* NOT THE REFERENCE: balance-heuristic weight of a BSDF-sampled direction that hit an emitter */
+			em = vscale(lastPdf / (lastPdf + lightPdf(&s->lights[ek], o, ray, rec.t)), em);
+		L = vadd(L, vmul(throughput, em));
 		/* uniforms: slot 0 = (jitter x, jitter y, bounce0 r0, bounce0 r1); slot k>=1 = (bounce 2k-1 r0 r1, bounce 2k r0 r1) */
 		float rnd0, rnd1;
 		if (it == 0) { rnd0 = orc_uniform(rng[2]); rnd1 = orc_uniform(rng[3]); }
@@ -791,6 +1029,26 @@ static v3 getColor(const orc_scene *s, ray_t ray, uint32_t pixel, uint32_t sampl
 				++*rays;
 				if (!hitBVH(s, sh, 0.001f, FLT_MAX, &srec, &selem, NULL, NULL))
 					L = vadd(L, vmul(vmul(throughput, vscale(sl.z / (pe + pbL), attL)), V(tap[0], tap[1], tap[2])));
+			}
+		}
+		if (s->lightCount && it + 1 < maxBounces)
+		{
+			/* NOT THE REFERENCE: one point on an emitter per scattering vertex (Philox counter word 3 = 2, slot = bounce), weighted
+			 * against the BSDF's pdf for the same direction; the shadow ray stops just short of the point */
+			uint32_t q[4], k; v3 x, wl; float dist, pl;
+			orc_philox(pixel, sample, (uint32_t)it, 2, k0, k1, q);
+			if (lightSample(s, q, rec.p, &k, &x, &wl, &dist, &pl))
+			{
+				const v3 Vv = worldToTangent(rec.n, vneg(ray.d)), sl = worldToTangent(rec.n, wl);
+				float pbL;
+				const v3 attL = materialEval(o->mtype, base, o->roughness, o->metalness, Vv, sl, &pbL);
+				if (sl.z > 0.0f && !((attL.x == 0.0f && attL.y == 0.0f && attL.z == 0.0f) || pbL == 0.0f))
+				{
+					ray_t sh; sh.o = rec.p; sh.d = wl;
+					++*rays;
+					if (!occludedBVH(s, sh, 0.001f, dist * (1.0f - 1e-4f)))
+						L = vadd(L, vmul(vmul(throughput, vscale(sl.z / (pl + pbL), attL)), s->sceneObjs[s->lights[k].scene].emissive));
+				}
 			}
 		}
 		v3 att = materialSample(o->mtype, base, o->roughness, o->metalness, rec.n, ray.d, rnd0, rnd1, &sdir, &pdf);
@@ -828,6 +1086,7 @@ void orc_scene_destroy(orc_scene *s)
 	if (!s) return;
 	for (uint32_t i = 0; i < s->texCount; ++i) { free(s->tex[i].f); free(s->tex[i].b); }
 	free(s->envQ); free(s->envAlias); free(s->envDensity);
+	free(s->lights); free(s->lightOf);
 	free(s->objs); free(s->toScene); free(s->sceneObjs); free(s->nodes); free(s);
 }
 uint32_t orc_add_texture(orc_scene *s, uint32_t w, uint32_t h, int is_hdr, const void *rgba)
@@ -860,6 +1119,38 @@ void orc_env_sample(const orc_scene *s, uint32_t r0, uint32_t r1, uint32_t r2, f
 	float u, v, pdf;
 	const v3 d = envSample(s, r0, r1, r2, &u, &v, &pdf);
 	out6[0] = d.x; out6[1] = d.y; out6[2] = d.z; out6[3] = u; out6[4] = v; out6[5] = pdf;
+}
+/* NOT THE REFERENCE: switch the "light_is" estimator on (builds the emitter table of the scene) / off (drops it) */
+void orc_set_light_is(orc_scene *s, int on)
+{
+	free(s->lights); free(s->lightOf);
+	s->lights = NULL; s->lightOf = NULL; s->lightCount = 0;
+	if (on) lightBuild(s);
+}
+/* the table, for tests: returns the emitter count; scene / prob / q / alias may be NULL */
+uint32_t orc_light_table(const orc_scene *s, uint32_t *scene, float *prob, float *q, uint32_t *alias)
+{
+	for (uint32_t k = 0; k < s->lightCount; ++k)
+	{
+		if (scene) scene[k] = s->lights[k].scene;
+		if (prob) prob[k] = s->lights[k].prob;
+		if (q) q[k] = s->lights[k].q;
+		if (alias) alias[k] = s->lights[k].alias;
+	}
+	return s->lightCount;
+}
+/* one sample of the emitter sampler (tests): out8 = world point, area pdf without the selection probability
+ * (pdfScale / P_sel / |W^T n_l|), emitter, local point */
+void orc_light_sample_point(const orc_scene *s, const uint32_t *q, float *out8)
+{
+	uint32_t k; v3 x, wd; float dist, pdf;
+	lightSample(s, q, V(0.0f, 0.0f, 0.0f), &k, &x, &wd, &dist, &pdf);
+	const light_t *L = &s->lights[k];
+	const v3 lp = lightLocalPoint(L->type, orc_uniform(q[1]), orc_uniform(q[2]), q[3]);
+	const v3 wn = lightWorldNormal(&s->sceneObjs[L->scene], lightUnitNormal(L->type, lp));
+	out8[0] = x.x; out8[1] = x.y; out8[2] = x.z;
+	out8[3] = (float)((double)L->pdfScale / (double)L->prob / sqrt((double)wn.x * wn.x + (double)wn.y * wn.y + (double)wn.z * wn.z));
+	out8[4] = (float)k; out8[5] = lp.x; out8[6] = lp.y; out8[7] = lp.z;
 }
 void orc_bvh_info(const orc_scene *s, uint32_t *nodes, uint32_t *depth, int32_t *valid)
 {

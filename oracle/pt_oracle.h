@@ -18,6 +18,11 @@ void orc_set_skybox(orc_scene *s, uint32_t handle);
 void orc_set_env_is(orc_scene *s, int on);
 uint32_t orc_env_tables(const orc_scene *s, uint32_t *cols, uint32_t *rows, float *q, uint32_t *alias, float *density);
 void orc_env_sample(const orc_scene *s, uint32_t r0, uint32_t r1, uint32_t r2, float *out6);
+/* NOT THE REFERENCE: the product's "light_is" estimator (csrc/light_sampling.h), restated likewise.  Not to be combined with
+ * env_is, which pt_render refuses too */
+void orc_set_light_is(orc_scene *s, int on);
+uint32_t orc_light_table(const orc_scene *s, uint32_t *scene, float *prob, float *q, uint32_t *alias);
+void orc_light_sample_point(const orc_scene *s, const uint32_t *q, float *out8);
 void orc_bvh_info(const orc_scene *s, uint32_t *nodes, uint32_t *depth, int32_t *valid);
 /* per object: 12 floats world->local rows, 6 floats AABB (min, max) */
 void orc_object_info(const orc_scene *s, size_t i, float *rows12, float *aabb6);

@@ -4,8 +4,7 @@ import numpy as np
 import pytest
 
 import pathtracercuda_b200 as pt
-from tests.helpers import bits
-from tests.test_light_sampling import seven_shape_scene
+from tests.helpers import bits, seven_shape_scene
 
 W, H, SPP = 48, 36, 16
 

@@ -7,11 +7,7 @@ these look at every call.  Last, the "env_is" / "light_is" kernel twins that the
 shared memory) path for path against the restatements.
 
 Tolerances name what they absorb; "B200" is the largest value seen on one B200 (1000 W) and the bound keeps headroom over it."""
-import ctypes as C
-import os
 import re
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -19,14 +15,9 @@ from scipy import stats
 
 import pathtracercuda_b200 as pt
 from oracle import imgio, orc
-from tests.helpers import ROOT, bits, golden_objects, load_golden
-from tests.test_light_sampling import SHAPES7, LightOracle, _local_ok, _mapped_area, seven_shape_scene
+from tests.device_probe import ProbeScene, _rng, probe  # noqa: F401  (probe: the module-scoped fixture that builds device_probe.cu)
+from tests.helpers import SHAPES7, _local_ok, _mapped_area, bits, golden_objects, load_golden, seven_shape_scene
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-CSRC = os.path.join(ROOT, "pathtracercuda_b200", "csrc")
-NVCC = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")
-# the product's flags (csrc/Makefile) plus -shared; -fopenmp / -lgomp for scene_compile.cpp's parallel sort
-NVFLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-Xcompiler", "-fPIC,-fopenmp,-ffp-contract=off"]
 LAMBERT, GGX, LAMBERT_GGX = 0, 1, 2
 PI = np.pi
 
@@ -34,102 +25,6 @@ PI = np.pi
 # ---------------------------------------------------------------------------------------------------------------------------------
 # the probe
 # ---------------------------------------------------------------------------------------------------------------------------------
-def _p(a):
-    return a.ctypes.data_as(C.c_void_p)
-
-
-class Probe:
-    def __init__(self, path, ptxas_log):
-        self.log = ptxas_log
-        L = self.L = C.CDLL(path)
-        vp, u32 = C.c_void_p, C.c_uint32
-        L.probe_material.argtypes = [u32, vp, vp]
-        L.probe_scene_create.restype = vp
-        L.probe_scene_create.argtypes = [C.c_size_t, vp]
-        L.probe_scene_destroy.argtypes = [vp]
-        L.probe_scene_info.restype = u32
-        L.probe_scene_info.argtypes = [vp, vp]
-        L.probe_hit.argtypes = [vp, C.c_int, u32, vp, vp, vp, C.c_float, vp, vp]
-        L.probe_light.argtypes = [vp, u32, vp, vp, vp]
-        L.probe_env.argtypes = [u32, u32, C.c_int, vp, C.c_int, u32, vp, vp]
-        L.probe_tex.argtypes = [u32, u32, C.c_int, vp, C.c_int, u32, vp, vp]
-        L.probe_angles.argtypes = [u32, vp, vp]
-
-    def tex(self, img, u, v, unit):
-        """texLookup at (u, v) on an (H, W, 4) uint8 or float32 texture; unit 1 = through a texture object -> (n, 3) rgb"""
-        img = np.ascontiguousarray(img)
-        uv = np.ascontiguousarray(np.stack([u, v], 1), np.float32)
-        out = np.zeros((len(uv), 3), np.float32)
-        assert self.L.probe_tex(img.shape[1], img.shape[0], int(img.dtype == np.float32), _p(img), int(unit), len(uv), _p(uv), _p(out)) == 0
-        return out
-
-    def angles(self, y, x, c, p):
-        """-> (n, 4): fastAtan2(y, x), fastAtan2Inline(y, x), fastAcos(c), fastPow(p, 2.2f)"""
-        inp = np.ascontiguousarray(np.stack([y, x, c, p], 1), np.float32)
-        out = np.zeros((len(inp), 4), np.float32)
-        assert self.L.probe_angles(len(inp), _p(inp), _p(out)) == 0
-        return out
-
-    def material(self, inp):
-        inp = np.ascontiguousarray(inp, np.float32)
-        out = np.zeros((len(inp), 32), np.float32)
-        assert self.L.probe_material(len(inp), _p(inp), _p(out)) == 0
-        return out
-
-    def env(self, img, q, mode=0):
-        img = np.ascontiguousarray(img, np.float32)
-        q = np.ascontiguousarray(q, np.uint32 if mode == 0 else np.float32)
-        out = np.zeros((len(q), 8) if mode == 0 else len(q), np.float32)
-        assert self.L.probe_env(img.shape[1], img.shape[0], 1, _p(img), mode, len(q), _p(q), _p(out)) == 0
-        return out
-
-
-class ProbeScene:
-    """a scene compiled and given its emitter table by the product's host code, uploaded as the render kernels see it"""
-
-    def __init__(self, probe, objects):
-        self.L = probe.L
-        self._arr = pt.abi.object_array(objects)
-        self.h = self.L.probe_scene_create(len(objects), C.byref(self._arr))
-        assert self.h
-        self.prim_of = np.zeros(len(objects), np.int32)
-        self.emitters = self.L.probe_scene_info(self.h, _p(self.prim_of))
-        self.object_of = np.argsort(self.prim_of)
-
-    def __del__(self):
-        try:
-            self.L.probe_scene_destroy(self.h)
-        except Exception:
-            pass
-
-    def hit(self, obj, o, d, tmax, exact, clip, tmin=0.001):
-        n = len(o)
-        prim = np.ascontiguousarray(self.prim_of[np.asarray(obj)], np.int32)
-        o, d, tmax = (np.ascontiguousarray(x, np.float32) for x in (o, d, tmax))
-        out = np.zeros((n, 12), np.float32)
-        assert self.L.probe_hit(self.h, int(exact) | 2 * int(clip), n, _p(prim), _p(o), _p(d), tmin, _p(tmax), _p(out)) == 0
-        return out
-
-    def light(self, q, p):
-        q, p = np.ascontiguousarray(q, np.uint32), np.ascontiguousarray(p, np.float32)
-        out = np.zeros((len(q), 8), np.float32)
-        assert self.L.probe_light(self.h, len(q), _p(q), _p(p), _p(out)) == 0
-        return out
-
-
-@pytest.fixture(scope="module")
-def probe():
-    out = os.path.join(tempfile.mkdtemp(prefix="device_probe_"), "libdevice_probe.so")
-    srcs = [os.path.join(HERE, "device_probe.cu")] + [os.path.join(CSRC, f) for f in ("scene_compile.cpp", "light_sampling.cpp", "env_sampling.cpp")]
-    r = subprocess.run([NVCC] + NVFLAGS + ["-Xptxas", "-v", "-shared", "-o", out] + srcs + ["-lgomp"], capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout + r.stderr
-    return Probe(out, r.stdout + r.stderr)
-
-
-def _rng(tag):
-    return np.random.default_rng(sum(map(ord, tag)))
-
-
 def test_probe_compiles_for_sm100a_without_spills(probe):
     kernels = re.findall(r"Compiling entry function '(\w+)' for 'sm_100a'", probe.log)
     assert len(kernels) == 10, probe.log  # material, four hit forms, light, two sky, texture, angles
@@ -513,7 +408,7 @@ def test_sample_light_geometry_pdf_and_density(probe, shape):
     o = _emitter(shape, rng)
     S = ProbeScene(probe, [o])
     assert S.emitters == 1
-    Wt = LightOracle([o]).rows(0)  # the product's world->local rows (bit-identical to the reference's, test_transforms_boxes_bvh_camera)
+    Wt = orc.Oracle([o]).object_info(0)[0].reshape(3, 4).astype(np.float64)  # the product's world->local rows (bit-identical to the reference's, test_transforms_boxes_bvh_camera)
     n = 1 << 16
     q = rng.integers(0, 2 ** 32, (n, 4), dtype=np.uint64).astype(np.uint32)
     P = _origins(rng, n, np.array(o.position, np.float64))
@@ -604,7 +499,7 @@ def test_sample_light_grazing_never_nan(probe):
     for shape in ("QUAD", "DISK"):
         o = pt.make_object(shape, (0.5, 1.0, -0.5), (30, 40, 50), (1.0, 1.0, 0.3), emissive=(1, 1, 1))
         S = ProbeScene(probe, [o])
-        Wt = LightOracle([o]).rows(0)
+        Wt = orc.Oracle([o]).object_info(0)[0].reshape(3, 4).astype(np.float64)
         M = np.linalg.inv(Wt[:, :3])
         n = 4096
         loc = np.stack([rng.uniform(-4, 4, n), np.zeros(n), rng.uniform(-4, 4, n)], 1)
@@ -758,7 +653,9 @@ def test_light_is_twins_match_the_restatement(spp, variant, smem_scene, smem_sta
     if panel == "dark":
         objs[2].material.emissive = (0.0, 0.0, 0.0)
     if ("light", spp, panel) not in _REFS:
-        _REFS["light", spp, panel] = LightOracle(objs).render(cam, W, H, spp)
+        O = orc.Oracle(objs)
+        O.set_light_is(1)
+        _REFS["light", spp, panel] = O.render(cam, W, H, spp)
     a, ra = _REFS["light", spp, panel]
     with pt.Pathtracer(W, H) as P:
         P.setScene(objs)
@@ -793,7 +690,9 @@ def test_light_is_max_bounces_match_the_restatement(max_bounces):
     """paths of at most 1, 2, 3 segments; at 1 no vertex scatters, so no light is sampled: the plain render's image, bit for bit"""
     W, H, spp = 48, 36, 32
     objs, cam = seven_shape_scene(W, H)
-    a, ra = LightOracle(objs).render(cam, W, H, spp, max_bounces=max_bounces)
+    O = orc.Oracle(objs)
+    O.set_light_is(1)
+    a, ra = O.render(cam, W, H, spp, max_bounces=max_bounces)
     with pt.Pathtracer(W, H) as P:
         P.setScene(objs)
         b, st = _render(P, cam, spp, light_is=1, max_bounces=max_bounces)

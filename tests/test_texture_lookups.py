@@ -15,7 +15,7 @@ import pytest
 
 import pathtracercuda_b200 as pt
 from oracle import orc
-from tests.test_device_functions import _rng, probe  # noqa: F401  (probe: the module-scoped fixture that builds device_probe.cu)
+from tests.device_probe import _rng, probe  # noqa: F401  (probe: the module-scoped fixture that builds device_probe.cu)
 
 PI = np.pi
 ULP = 2.0 ** -24            # half an ulp of 1: the relative rounding of one fp32 operation
