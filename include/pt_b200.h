@@ -275,6 +275,40 @@ int pt_env_distribution(uint32_t width, uint32_t height, int is_hdr, const void 
  * alias emitter).  Host only.  Call with NULL buffers for the count; returns the emitter count (0 when nothing emits) or a negative error. */
 int pt_light_distribution(size_t count, const pt_object_desc *objects, uint32_t *scene_index, float *probability, uint32_t *alias);
 
+/* ---- denoiser: guide buffers and the edge-avoiding a-trous wavelet filter (Dammertz et al. 2010) ---- */
+
+/* Guide buffers (W*H*4 floats each), means over the camera rays of a pixel:
+ *  PT_AOV_ALBEDO    rgb: base colour of the first hit (texture tap included; a miss counts as 1, 1, 1), w: fraction of rays that hit
+ *  PT_AOV_NORMAL    xyz: unit normal of the first hit, facing the ray (a miss counts as 0), w: 0
+ *  PT_AOV_POSITION  xyz: first hit point, w: its t - means over the rays that hit (0 where none did) */
+enum { PT_AOV_ALBEDO = 0, PT_AOV_NORMAL = 1, PT_AOV_POSITION = 2 };
+/* Filter parameters: iterations K (0 ... 12; iteration i takes taps 2^i pixels apart), sigma_color (on the per-sample mean of the colour
+ * divided by the albedo; halved at every iteration), sigma_normal, sigma_position (relative to the pixel's depth t).  A sigma of 0
+ * admits equal values only. */
+typedef struct pt_denoise_params { uint32_t iterations; float sigma_color, sigma_normal, sigma_position; } pt_denoise_params;
+/* the defaults (pt_denoise with params = NULL), chosen by the sweep of tools/denoise_measure.py (DESIGN.md) */
+#define PT_DENOISE_DEFAULT_ITERATIONS 4
+#define PT_DENOISE_DEFAULT_SIGMA_COLOR 8.0f
+#define PT_DENOISE_DEFAULT_SIGMA_NORMAL 0.5f
+#define PT_DENOISE_DEFAULT_SIGMA_POSITION 0.02f
+
+/* Replaces the guide buffers with those of `spp` camera rays per pixel (spp = 0: PT_E_INVALID).  The rays are jittered within the
+ * pixel from a Philox stream of their own (option "seed"); with option "jitter" = 0 they are the pixel-centre rays of pt_primary_pass.
+ * Runs on the root device of a multi-GPU context.  pt_set_scene / pt_set_scene_xform make the guide buffers stale. */
+int pt_render_aov(pt_context *ctx, const pt_camera_desc *camera, uint32_t spp);
+/* one guide buffer (PT_AOV_*), library-owned, valid until the next call on ctx; NULL before the first pt_render_aov */
+const float *pt_get_aov(pt_context *ctx, int kind);
+/* Filters the image the getters read (on a multi-GPU context the finished image on the root) with the current guide buffers into a
+ * denoised sum buffer; params = NULL: the defaults.  PT_E_INVALID for missing or stale guide buffers, more than 12 iterations, or a
+ * negative or non-finite sigma.  Colour is divided by max(albedo, 0.01) per channel before filtering and multiplied back after;
+ * K = 0 gives the input's bits. */
+int pt_denoise(pt_context *ctx, const pt_denoise_params *params);
+/* the denoised image of the last pt_denoise, normalised as pt_get_hdr / pt_get_hdr_mean / tone-mapped as pt_get_ldr (with the counts
+ * of the image it was made from); library-owned, valid until the next call on ctx */
+const float *pt_get_denoised_hdr(pt_context *ctx);
+const float *pt_get_denoised_hdr_mean(pt_context *ctx);
+const uint8_t *pt_get_denoised_ldr(pt_context *ctx);
+
 const char *pt_last_error(void);
 const char *pt_version(void);
 

@@ -56,6 +56,12 @@ def load_library():
         "pt_write_hdr": (i32, [cp, u32, u32, vp]),
         "pt_env_distribution": (i32, [u32, u32, i32, vp, vp, vp, vp, vp]),
         "pt_light_distribution": (i32, [sz, vp, vp, vp, vp]),
+        "pt_render_aov": (i32, [vp, vp, u32]),
+        "pt_get_aov": (vp, [vp, i32]),
+        "pt_denoise": (i32, [vp, vp]),
+        "pt_get_denoised_hdr": (vp, [vp]),
+        "pt_get_denoised_hdr_mean": (vp, [vp]),
+        "pt_get_denoised_ldr": (vp, [vp]),
         "pt_read_image": (i32, [cp, vp, vp, vp, vp]),
         "pt_free": (None, [vp]),
         "pt_last_error": (cp, []),
@@ -74,7 +80,18 @@ def load_library():
 EXPORTS = ["pt_create", "pt_create_multi", "pt_get_multi_info", "pt_destroy", "pt_set_scene", "pt_set_scene_xform", "pt_render_vectors", "pt_load_texture", "pt_load_texture_mem", "pt_set_skybox", "pt_render",
            "pt_get_timing_ms", "pt_get_hdr", "pt_get_hdr_mean", "pt_get_hdr_sum", "pt_get_ldr", "pt_set_option", "pt_get_stats", "pt_camera_rotate", "pt_camera_translate", "pt_primary_pass",
            "pt_trace_rays", "pt_get_first_hit", "pt_accum_device_ptr", "pt_set_accum_device_ptr", "pt_load_scene_file", "pt_parse_scene_file",
-           "pt_write_png", "pt_write_hdr", "pt_env_distribution", "pt_light_distribution", "pt_read_image", "pt_free", "pt_last_error", "pt_version"]
+           "pt_write_png", "pt_write_hdr", "pt_env_distribution", "pt_light_distribution", "pt_read_image", "pt_free", "pt_last_error", "pt_version",
+           "pt_render_aov", "pt_get_aov", "pt_denoise", "pt_get_denoised_hdr", "pt_get_denoised_hdr_mean", "pt_get_denoised_ldr"]
+
+AOV_ALBEDO, AOV_NORMAL, AOV_POSITION = 0, 1, 2  # PT_AOV_*
+AOV_KINDS = {"albedo": AOV_ALBEDO, "normal": AOV_NORMAL, "position": AOV_POSITION}
+# PT_DENOISE_DEFAULT_* of include/pt_b200.h (tests/test_denoise.py checks that the two agree)
+DENOISE_DEFAULTS = {"iterations": 4, "sigma_color": 8.0, "sigma_normal": 0.5, "sigma_position": 0.02}
+
+
+class DenoiseParams(C.Structure):
+    """pt_denoise_params"""
+    _fields_ = [("iterations", C.c_uint32), ("sigma_color", C.c_float), ("sigma_normal", C.c_float), ("sigma_position", C.c_float)]
 
 
 def _err(L):
@@ -303,6 +320,38 @@ class Pathtracer:
         finally:
             os.chdir(old)
         return cam
+
+    # ---- denoiser ------------------------------------------------------------------------------------------------
+    def renderAOV(self, camera, spp):
+        """pt_render_aov: replace the guide buffers with the means over `spp` camera rays per pixel"""
+        _check(self.L, self.L.pt_render_aov(self.h, C.byref(camera), int(spp)), "pt_render_aov")
+
+    def aov(self, kind, copy=True):
+        """one guide buffer, (H, W, 4) float32: kind "albedo" | "normal" | "position" or AOV_*"""
+        a = self._img(self.L.pt_get_aov(self.h, AOV_KINDS.get(kind, kind)), np.float32)
+        return a.copy() if copy else a
+
+    def denoise(self, iterations=None, sigma_color=None, sigma_normal=None, sigma_position=None):
+        """pt_denoise: filter the image with the current guide buffers; None = the library's default"""
+        given = dict(iterations=iterations, sigma_color=sigma_color, sigma_normal=sigma_normal, sigma_position=sigma_position)
+        q = DenoiseParams(**{k: (DENOISE_DEFAULTS[k] if v is None else v) for k, v in given.items()})
+        all_default = all(v is None for v in given.values())
+        _check(self.L, self.L.pt_denoise(self.h, None if all_default else C.byref(q)), "pt_denoise")
+
+    def getDenoisedHDR(self, copy=True):
+        """the denoised image normalised as getHDRImageData"""
+        a = self._img(self.L.pt_get_denoised_hdr(self.h), np.float32)
+        return a.copy() if copy else a
+
+    def getDenoisedHDRMean(self, copy=True):
+        """the denoised image normalised as getHDRMean"""
+        a = self._img(self.L.pt_get_denoised_hdr_mean(self.h), np.float32)
+        return a.copy() if copy else a
+
+    def getDenoisedImage(self, copy=True):
+        """the denoised image tone-mapped as getImageData"""
+        a = self._img(self.L.pt_get_denoised_ldr(self.h), np.uint8)
+        return a.copy() if copy else a
 
     def accumDevicePtr(self):
         return self.L.pt_accum_device_ptr(self.h)

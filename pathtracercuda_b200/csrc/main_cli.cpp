@@ -4,7 +4,8 @@
 // out of scope on a headless B200 server: the flags are parsed and reported, then refused.
 // Extra options use a double dash so they cannot collide with the reference's: --device N, --seed S, --slice N,
 // --true-mean, --stats, --env-is (sky importance sampling, pt_set_option "env_is"), --light-is (emitter importance sampling,
-// pt_set_option "light_is"), --bvh sah|lbvh|auto, and for several GPUs of one box (the reference is fixed to device 0, Pathtracer.cpp:40):
+// pt_set_option "light_is"), --bvh sah|lbvh|auto, --denoise K (after the last launch: guide buffers of --aov-spp N camera rays per
+// pixel, default 16, and K iterations of the a-trous denoiser at its default sigmas; -o / -ohdr then write the denoised image), and for several GPUs of one box (the reference is fixed to device 0, Pathtracer.cpp:40):
 // --gpus N (devices 0..N-1) or --devices MASK, --partition pixels|samples, --exchange p2p|nccl (pt_create_multi).
 #include "../../include/pt_b200.h"
 #include <algorithm>
@@ -35,6 +36,8 @@ struct Params // reference Params.h:4-14
 	unsigned int deviceMask = 0; // != 0: multi-GPU context over these CUDA ordinals
 	int partition = 0;           // 0 pixels, 1 samples
 	int exchange = -1;           // -1 auto, 0 nccl, 1 p2p
+	int denoise = -1;            // >= 0: denoiser iterations (pt_denoise); -1: no denoiser
+	unsigned int aovSpp = 16;    // camera rays per pixel of the denoiser's guide buffers (pt_render_aov)
 };
 
 static bool processArgs(int argc, char *argv[], Params &params)
@@ -80,6 +83,8 @@ static bool processArgs(int argc, char *argv[], Params &params)
 		else if (strcmp(a, "--light-is") == 0) { params.lightIS = true; ++i; }
 		else if (strcmp(a, "--bvh") == 0 && i + 1 < argc) { const char *v = argv[i + 1]; params.bvhBuilder = strcmp(v, "lbvh") == 0 ? 1 : (strcmp(v, "auto") == 0 ? 2 : 0); i += 2; }
 		else if (strcmp(a, "--stats") == 0) { params.stats = true; ++i; }
+		else if (strcmp(a, "--denoise") == 0 && i + 1 < argc) { params.denoise = atoi(argv[i + 1]); i += 2; }
+		else if (strcmp(a, "--aov-spp") == 0 && i + 1 < argc) { params.aovSpp = (unsigned int)atoi(argv[i + 1]); i += 2; }
 		else
 		{
 			printf("Can't parse argument: %s\n", a);
@@ -192,6 +197,13 @@ int main(int argc, char *argv[])
 	}
 	const double tRender = nowMs();
 	printf("Finished accumulating %d samples in %f ms GPU time\n", (int)params.m_spp, totalGpuTime);
+	if (params.denoise >= 0)
+	{
+		pt_denoise_params dp = { (uint32_t)params.denoise, PT_DENOISE_DEFAULT_SIGMA_COLOR, PT_DENOISE_DEFAULT_SIGMA_NORMAL, PT_DENOISE_DEFAULT_SIGMA_POSITION };
+		if (pt_render_aov(ctx, &camera, params.aovSpp) != PT_OK) die("pt_render_aov");
+		if (pt_denoise(ctx, &dp) != PT_OK) die("pt_denoise");
+	}
+	const bool denoised = params.denoise >= 0;
 
 	if (params.m_outputFilepath)
 	{
@@ -199,14 +211,14 @@ int main(int argc, char *argv[])
 		int r;
 		if (params.m_outputHdr)
 		{
-			const float *img = params.trueMean ? pt_get_hdr_mean(ctx) : pt_get_hdr(ctx);
+			const float *img = params.trueMean ? (denoised ? pt_get_denoised_hdr_mean(ctx) : pt_get_hdr_mean(ctx)) : (denoised ? pt_get_denoised_hdr(ctx) : pt_get_hdr(ctx));
 			if (!img) die("pt_get_hdr");
 			r = pt_write_hdr(params.m_outputFilepath, params.m_width, params.m_height, img);
 		}
 		else
 		{
 			if (params.trueMean) pt_set_option(ctx, "frames_per_spp", 1.0);
-			const uint8_t *img = pt_get_ldr(ctx);
+			const uint8_t *img = denoised ? pt_get_denoised_ldr(ctx) : pt_get_ldr(ctx);
 			if (!img) die("pt_get_ldr");
 			r = pt_write_png(params.m_outputFilepath, params.m_width, params.m_height, img);
 		}

@@ -8,6 +8,7 @@
 #include "scene_compile.h"
 #include "scene_loader.h"
 #include "trace_kernels.h"
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -130,6 +131,13 @@ struct pt_context
 	pt_stats multiStats = {};     // statistics of the last pt_render summed over the devices
 	float alpha = 1.0f;           // RenderParams::alpha
 	bool skipPartitionClear = false; // p2p: the other devices write their pixels into this very buffer - nothing to zero
+	// denoiser (pt_render_aov / pt_denoise; on the root device), allocated on first use
+	DevBuf aov[3];                // guide buffers: albedo, normal, position (PT_AOV_*)
+	bool aovValid = false;        // rendered, and no scene set since
+	DevBuf denoised, denoiseTmp;  // the filtered sum buffer, and the other side of the ping-pong
+	bool hasDenoised = false;
+	uint32_t denoisedFrames = 0;  // accumulatedFrames / totalSamples of the image pt_denoise filtered
+	unsigned long long denoisedSamples = 0;
 };
 
 #define CK(expr)                                                                                                      \
@@ -363,6 +371,7 @@ static int setScene(pt_context *c, const std::string &fn, size_t count, const pt
 	buildLightTable(cs, lt);
 	// the BVH (and the emitter table) is built ONCE on the host; a multi-GPU context replicates the compiled scene on every device
 	int r = uploadScene(c, cs, lt);
+	if (r == PT_OK) c->aovValid = false; // the guide buffers show the previous scene
 	for (size_t i = 0; r == PT_OK && i < c->peers.size(); ++i) r = uploadScene(c->peers[i], cs, lt);
 	return r;
 }
@@ -515,6 +524,28 @@ static int ensureEnvDistribution(pt_context *c, uint32_t handle)
 	return PT_OK;
 }
 
+// the ten Philox round keys of `seed` (RenderParams::philoxKeys)
+static void philoxKeys(uint64_t seed, uint32_t (&keys)[20])
+{
+	const uint32_t lo = uint32_t(seed), hi = uint32_t(seed >> 32);
+	for (uint32_t i = 0; i < 10; ++i) { keys[2 * i] = lo + i * 0x9E3779B9u; keys[2 * i + 1] = hi + i * 0xBB67AE85u; }
+}
+
+// option "jitter" = 0: the pixel-centre coordinates (RenderParams::centreU / centreV), made on first use
+static int ensureCentreTables(pt_context *c)
+{
+	if (c->centreUV.p) return PT_OK;
+	// (this file is compiled without FMA contraction: the division is the IEEE one of the reference's primary pass)
+	std::vector<float> uv(size_t(c->width) + c->height);
+	for (uint32_t x = 0; x < c->width; ++x) uv[x] = (float(x) + 0.5f) / float(c->width);
+	for (uint32_t y = 0; y < c->height; ++y) uv[c->width + y] = (float(y) + 0.5f) / float(c->height);
+	DevBuf centres;
+	CK(centres.alloc(uv.size() * sizeof(float)));
+	CK(cudaMemcpy(centres.p, uv.data(), uv.size() * sizeof(float), cudaMemcpyHostToDevice));
+	c->centreUV = std::move(centres);
+	return PT_OK;
+}
+
 static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int ignore_history)
 {
 	PT_TRY
@@ -547,7 +578,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		p.pixelStride = c->pixelStride;
 		p.seedLo = uint32_t(c->seed);
 		p.seedHi = uint32_t(c->seed >> 32);
-		for (uint32_t i = 0; i < 10; ++i) { p.philoxKeys[2 * i] = p.seedLo + i * 0x9E3779B9u; p.philoxKeys[2 * i + 1] = p.seedHi + i * 0xBB67AE85u; }
+		philoxKeys(c->seed, p.philoxKeys);
 		p.maxBounces = c->maxBounces;
 		p.regenLow = c->launch.regenLow > 0 ? uint32_t(c->launch.regenLow) : 16u;
 		// first-bounce stratification (RenderParams::strataPer): 2^k cells, k <= 8, at least 16 samples per cell - the lanes of a
@@ -580,17 +611,8 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		}
 		if (c->noJitter)
 		{
-			if (!c->centreUV.p)
-			{
-				// (this file is compiled without FMA contraction: the division is the IEEE one of the reference's primary pass)
-				std::vector<float> uv(size_t(c->width) + c->height);
-				for (uint32_t x = 0; x < c->width; ++x) uv[x] = (float(x) + 0.5f) / float(c->width);
-				for (uint32_t y = 0; y < c->height; ++y) uv[c->width + y] = (float(y) + 0.5f) / float(c->height);
-				DevBuf centres;
-				CK(centres.alloc(uv.size() * sizeof(float)));
-				CK(cudaMemcpy(centres.p, uv.data(), uv.size() * sizeof(float), cudaMemcpyHostToDevice));
-				c->centreUV = std::move(centres);
-			}
+			const int rc = ensureCentreTables(c);
+			if (rc != PT_OK) return rc;
 			p.centreU = c->centreUV.as<float>();
 			p.centreV = c->centreUV.as<float>() + c->width;
 			p.aids |= kAidPixelCentre;
@@ -833,8 +855,8 @@ int pt_render_vectors(pt_context *c, const pt_camera_vectors *camera, uint32_t s
 float pt_get_timing_ms(const pt_context *c) { return c ? c->timingMs : 0.0f; }
 
 // the image getters: the accumulation x scale (HDR) or tone-mapped (LDR) into device staging, copied to pinned host memory (both
-// allocated by the first call)
-static const void *readBack(pt_context *c, bool ldr, float scale)
+// allocated by the first call).  `src`: the float4 buffer to read, null = the image (the accumulation, or a multi-GPU job's reduce)
+static const void *readBack(pt_context *c, bool ldr, float scale, const float4 *src = nullptr)
 {
 	if (cudaSetDevice(c->device) != cudaSuccess) return nullptr;
 	const uint32_t px = c->width * c->height;
@@ -847,7 +869,7 @@ static const void *readBack(pt_context *c, bool ldr, float scale)
 		setError(PT_E_CUDA, fn + cudaGetErrorString(cudaGetLastError()));
 		return nullptr;
 	}
-	const float4 *src = c->imageSource ? c->imageSource : c->accum;
+	if (!src) src = c->imageSource ? c->imageSource : c->accum;
 	if (ldr) launchTonemap(src, dev.as<uchar4>(), px, scale, c->stream);
 	else launchScale(src, dev.as<float4>(), px, scale, c->stream);
 	if (cudaMemcpyAsync(host.p, dev.p, bytes, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess)
@@ -883,6 +905,111 @@ const uint8_t *pt_get_ldr(pt_context *c)
 	// reference; here the accumulation is zero in that case and the scale is clamped like getHDRImageData's
 	return static_cast<const uint8_t *>(readBack(c, true, 1.0f / fmaxf(float(c->accumulatedFrames), 1.0f)));
 }
+
+int pt_render_aov(pt_context *c, const pt_camera_desc *camera, uint32_t spp)
+{
+	PT_TRY
+	if (!c || !camera) return setError(PT_E_INVALID, "pt_render_aov: bad arguments");
+	if (spp == 0) return setError(PT_E_INVALID, "pt_render_aov: spp must be at least 1");
+	if (c->nodeCount == 0) return setError(PT_E_INVALID, "pt_render_aov: no scene");
+	CK(cudaSetDevice(c->device));
+	const size_t bytes = size_t(c->width) * c->height * sizeof(float4);
+	for (DevBuf &b : c->aov)
+		if (!b.p) CK(b.alloc(bytes));
+	AovParams p;
+	p.scene = sceneDev(c);
+	computeCamera(*camera, p.cam);
+	p.width = c->width;
+	p.height = c->height;
+	p.spp = spp;
+	philoxKeys(c->seed, p.philoxKeys);
+	if (c->noJitter)
+	{
+		const int rc = ensureCentreTables(c);
+		if (rc != PT_OK) return rc;
+		p.centreU = c->centreUV.as<float>();
+		p.centreV = c->centreUV.as<float>() + c->width;
+	}
+	p.albedo = c->aov[PT_AOV_ALBEDO].as<float4>();
+	p.normal = c->aov[PT_AOV_NORMAL].as<float4>();
+	p.position = c->aov[PT_AOV_POSITION].as<float4>();
+	launchAov(p, c->stream);
+	CK(cudaGetLastError());
+	CK(cudaStreamSynchronize(c->stream));
+	c->aovValid = true;
+	return PT_OK;
+	PT_CATCH(PT_E_LIMIT)
+}
+
+const float *pt_get_aov(pt_context *c, int kind)
+{
+	if (!c || kind < PT_AOV_ALBEDO || kind > PT_AOV_POSITION) { setError(PT_E_INVALID, "pt_get_aov: bad arguments"); return nullptr; }
+	if (!c->aov[kind].p) { setError(PT_E_INVALID, "pt_get_aov: no pt_render_aov yet"); return nullptr; }
+	return static_cast<const float *>(readBack(c, false, 1.0f, c->aov[kind].as<float4>())); // (x 1: the buffer's own bits)
+}
+
+int pt_denoise(pt_context *c, const pt_denoise_params *params)
+{
+	PT_TRY
+	if (!c) return setError(PT_E_INVALID, "pt_denoise: null context");
+	const pt_denoise_params q = params ? *params
+	                                   : pt_denoise_params{ PT_DENOISE_DEFAULT_ITERATIONS, PT_DENOISE_DEFAULT_SIGMA_COLOR, PT_DENOISE_DEFAULT_SIGMA_NORMAL,
+	                                                        PT_DENOISE_DEFAULT_SIGMA_POSITION };
+	if (q.iterations > 12) return setError(PT_E_INVALID, "pt_denoise: at most 12 iterations");
+	for (float s : { q.sigma_color, q.sigma_normal, q.sigma_position })
+		if (!(s >= 0.0f) || !std::isfinite(s)) return setError(PT_E_INVALID, "pt_denoise: every sigma must be finite and not negative");
+	if (!c->aov[0].p) return setError(PT_E_INVALID, "pt_denoise: no guide buffers (pt_render_aov first)");
+	if (!c->aovValid) return setError(PT_E_INVALID, "pt_denoise: the guide buffers are stale (the scene changed since pt_render_aov)");
+	CK(cudaSetDevice(c->device));
+	const size_t bytes = size_t(c->width) * c->height * sizeof(float4);
+	if (!c->denoised.p) CK(c->denoised.alloc(bytes));
+	if (q.iterations > 1 && !c->denoiseTmp.p) CK(c->denoiseTmp.alloc(bytes));
+	const float4 *src = c->imageSource ? c->imageSource : c->accum;
+	if (q.iterations == 0) CK(cudaMemcpyAsync(c->denoised.p, src, bytes, cudaMemcpyDeviceToDevice, c->stream));
+	// the filter runs on the sums: the colour term's sigma is scaled by the sample count, which in exact arithmetic is the filter of the
+	// per-sample mean
+	const double n = double(c->totalSamples > 0 ? c->totalSamples : 1ull);
+	auto inverseSquare = [](double s) { return float(std::fmin(1.0 / (s * s), double(FLT_MAX))); }; // (sigma 0: FLT_MAX, see denoise.cu)
+	for (uint32_t i = 0; i < q.iterations; ++i)
+	{
+		AtrousParams a;
+		a.in = src;
+		a.out = ((q.iterations - 1u - i) & 1u) ? c->denoiseTmp.as<float4>() : c->denoised.as<float4>(); // the last iteration lands in `denoised`
+		a.albedo = c->aov[PT_AOV_ALBEDO].as<float4>();
+		a.normal = c->aov[PT_AOV_NORMAL].as<float4>();
+		a.position = c->aov[PT_AOV_POSITION].as<float4>();
+		a.width = c->width;
+		a.height = c->height;
+		a.step = 1u << i;
+		a.invColor2 = inverseSquare(double(q.sigma_color) * n / double(a.step));
+		a.invNormal2 = inverseSquare(double(q.sigma_normal));
+		a.sigmaPosition = q.sigma_position;
+		a.demodulate = i == 0;
+		a.remodulate = i + 1u == q.iterations;
+		launchAtrous(a, c->stream);
+		src = a.out;
+	}
+	CK(cudaGetLastError());
+	CK(cudaStreamSynchronize(c->stream));
+	c->hasDenoised = true;
+	c->denoisedFrames = c->accumulatedFrames;
+	c->denoisedSamples = c->totalSamples;
+	return PT_OK;
+	PT_CATCH(PT_E_LIMIT)
+}
+
+// the denoised sum buffer through readBack, with the counts of the image it was made from
+static const void *readDenoised(pt_context *c, bool ldr, bool mean)
+{
+	if (!c) return nullptr;
+	if (!c->hasDenoised) { setError(PT_E_INVALID, "pt_get_denoised_*: no pt_denoise yet"); return nullptr; }
+	const float count = mean ? float(c->denoisedSamples) : float(c->denoisedFrames);
+	return readBack(c, ldr, 1.0f / fmaxf(count, 1.0f), c->denoised.as<float4>());
+}
+
+const float *pt_get_denoised_hdr(pt_context *c) { return static_cast<const float *>(readDenoised(c, false, false)); }
+const float *pt_get_denoised_hdr_mean(pt_context *c) { return static_cast<const float *>(readDenoised(c, false, true)); }
+const uint8_t *pt_get_denoised_ldr(pt_context *c) { return static_cast<const uint8_t *>(readDenoised(c, true, false)); }
 
 static int setOptionOne(pt_context *c, const char *key, double value)
 {

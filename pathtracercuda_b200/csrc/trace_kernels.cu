@@ -36,6 +36,19 @@ static __device__ __forceinline__ void storePixel(const RenderParams &p, uint32_
 	p.accum[pixel] = out;
 }
 
+// the base colour of a hit (Material.inl:26-35): the material's own, or the tap of its texture at (u, v) taken to linear by the 2.2 power;
+// one statement for the trace kernels and the guide-buffer kernel, so that the albedo guide is the colour the paths are shaded with
+static __device__ __forceinline__ V3 baseColour(const SceneDev &scene, float4 m0, uint32_t tex, float u, float v)
+{
+	V3 base = mk(m0.x, m0.y, m0.z);
+	if (tex != 0 && tex <= scene.texCount)
+	{
+		const V3 tap = texLookup(scene.textures, tex, u, v); // Material.inl:26-35
+		base = mk(fastPow(tap.x, 2.2f), fastPow(tap.y, 2.2f), fastPow(tap.z, 2.2f));
+	}
+	return base;
+}
+
 // a contribution of a lane's path: the one-pixel-per-warp kernel (SHARE) adds it to the warp's partial sums of the pixel as it comes, the
 // one-pixel-per-lane kernel to the path's own sum L, which goes to the pixel's when the path ends (the two orders of the additions give
 // different bits)
@@ -327,13 +340,8 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 					if (COUNT) ++shades;
 					const Surface s = surfaceAt<SMEM>(sv, h.prim, ro, rd, h.t);
 					const float4 m0 = sv.ld(mp), m2 = sv.ld(mp + 2);
-					V3 base = mk(m0.x, m0.y, m0.z);
 					const uint32_t tex = __float_as_uint(m2.x), mtype = __float_as_uint(m2.y);
-					if (tex != 0 && tex <= p.scene.texCount)
-					{
-						const V3 tap = texLookup(p.scene.textures, tex, s.u, s.v); // Material.inl:26-35
-						base = mk(fastPow(tap.x, 2.2f), fastPow(tap.y, 2.2f), fastPow(tap.z, 2.2f));
-					}
+					const V3 base = baseColour(p.scene, m0, tex, s.u, s.v);
 					float rnd0, rnd1;
 					if (bounce == 0) { rnd0 = uniform01(rz); rnd1 = uniform01(rw); }
 					else if (bounce & 1u)
@@ -508,6 +516,60 @@ __global__ void __launch_bounds__(kThreads) traceRaysKernel(SceneDev scene, uint
 	}
 }
 
+// the guide buffers of the denoiser (pt_render_aov): one thread per pixel, spp camera rays each, through the scene in global memory
+// (a pass this short does not pay for the shared-memory staging); the means over the pixel's samples of the first hit's base colour
+// (a miss counts as white; w = the fraction of rays that hit), its normal facing the ray (a miss counts as 0), and over the hits only
+// its position (w = t)
+__global__ void __launch_bounds__(kThreads) aovKernel(const __grid_constant__ AovParams p)
+{
+	const uint32_t pixel = blockIdx.x * blockDim.x + threadIdx.x;
+	if (pixel >= p.width * p.height) return;
+	SceneView<false> sv;
+	sv.nodes = p.scene.sceneBlob;
+	sv.prims = p.scene.sceneBlob + size_t(p.scene.nodeCount) * 4;
+	sv.globalCount = p.scene.globalCount;
+	const float4 *const matTable = sv.prims + size_t(p.scene.primCount) * 4;
+	uint32_t px, py;
+	pixelToXY(pixel, p.width, p.height, px, py);
+	const float invW = 1.0f / float(p.width), invH = 1.0f / float(p.height);
+	const V3 o = mk(p.cam.origin[0], p.cam.origin[1], p.cam.origin[2]);
+	V3 albedo = mk(0.0f, 0.0f, 0.0f), normal = mk(0.0f, 0.0f, 0.0f), position = mk(0.0f, 0.0f, 0.0f);
+	float tSum = 0.0f;
+	uint32_t hits = 0, nv = 0, pt = 0;
+	for (uint32_t sample = 0; sample < p.spp; ++sample)
+	{
+		float u, v;
+		if (p.centreU) { u = __ldg(p.centreU + px); v = __ldg(p.centreV + py); } // option "jitter" = 0: the rays of pt_primary_pass
+		else
+		{
+			// a Philox stream of its own (fourth counter word 3): no draw of a render is reused
+			const uint4 r = philox4x32_10_keyed(pixel, sample, 0u, 3u, p.philoxKeys);
+			u = (float(px) + uniform01(r.x)) * invW;
+			v = (float(py) + uniform01(r.y)) * invH;
+		}
+		const V3 d = cameraDir<2>(p.cam, u, v);
+		// (the primitive tests with IEEE division and square root, as pt_primary_pass / pt_trace_rays: the guides of pixel-centre rays are
+		// those queries' hits)
+		const Hit h = closestHitWW<false, false, true>(sv, o, d, 0.001f, nv, pt);
+		if (h.prim < 0)
+		{
+			albedo = albedo + mk(1.0f, 1.0f, 1.0f);
+			continue;
+		}
+		const Surface s = surfaceAt<false>(sv, h.prim, o, d, h.t);
+		const float4 *mp = matTable + h.prim * 3;
+		albedo = albedo + baseColour(p.scene, __ldg(mp), __float_as_uint(__ldg(mp + 2).x), s.u, s.v);
+		normal = normal + s.n;
+		position = position + s.p;
+		tSum += h.t;
+		++hits;
+	}
+	const float n = float(p.spp), k = float(hits);
+	p.albedo[pixel] = make_float4(albedo.x / n, albedo.y / n, albedo.z / n, k / n);
+	p.normal[pixel] = make_float4(normal.x / n, normal.y / n, normal.z / n, 0.0f);
+	p.position[pixel] = hits ? make_float4(position.x / k, position.y / k, position.z / k, tSum / k) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+}
+
 // debugging aid: invSqrtExact against the library routines it stands in for
 __global__ void invSqrtCheckKernel(uint32_t n, const float *x, float *fast, float *ieee)
 {
@@ -640,6 +702,13 @@ int launchTraceRays(const SceneDev &scene, size_t n, const float *origins, const
 {
 	const int grid = int((n + kThreads - 1) / kThreads);
 	traceRaysKernel<<<grid, kThreads, 0, stream>>>(scene, uint32_t(n), origins, directions, tMin, hitIndex, hitT, hitNormal);
+	return 1;
+}
+
+int launchAov(const AovParams &p, cudaStream_t stream)
+{
+	const uint32_t total = p.width * p.height;
+	aovKernel<<<int((total + kThreads - 1) / kThreads), kThreads, 0, stream>>>(p);
 	return 1;
 }
 

@@ -78,6 +78,17 @@ struct RenderParams
 
 constexpr uint32_t kAidPixelCentre = 1u, kAidFirstHit = 2u;
 
+// the guide-buffer pass of the denoiser (pt_render_aov): W x H float4 each, means over spp camera rays per pixel
+struct AovParams
+{
+	SceneDev scene;
+	CameraDev cam;
+	uint32_t width, height, spp;
+	uint32_t philoxKeys[20];                          // as RenderParams::philoxKeys; the pass draws from its own stream (fourth counter word 3)
+	const float *centreU = nullptr, *centreV = nullptr; // option "jitter" = 0: pixel-centre rays (RenderParams::centreU)
+	float4 *albedo, *normal, *position;
+};
+
 // Which twin of the trace kernel a launch runs (traceKernel's last template parameter).  Each option below is compiled into an
 // instantiation of its own, so that the plain kernel's code is untouched by it; one launch runs one of them.
 enum class Twin
@@ -123,6 +134,20 @@ int launchTrace(const RenderParams &p, const LaunchConfig &cfg, cudaStream_t str
 int launchPrimary(const SceneDev &scene, const CameraDev &cam, uint32_t width, uint32_t height, int32_t *hitIndex, float *hitT, cudaStream_t stream);
 int launchTraceRays(const SceneDev &scene, size_t n, const float *origins, const float *directions, float tMin, int32_t *hitIndex, float *hitT,
                     float *hitNormal, cudaStream_t stream);
+int launchAov(const AovParams &p, cudaStream_t stream);
+
+// one iteration of the edge-avoiding a-trous filter (denoise.cu), on W x H float4 sum buffers
+struct AtrousParams
+{
+	const float4 *in;
+	float4 *out;                              // (never `in`: the iterations ping-pong)
+	const float4 *albedo, *normal, *position; // the guide buffers (AovParams)
+	uint32_t width, height, step;             // step = 2^iteration
+	float invColor2, invNormal2;              // 1 / sigma^2 of the colour term (sigma scaled for sums and iteration) and the normal term
+	float sigmaPosition;                      // relative to the pixel's depth
+	uint32_t demodulate, remodulate;          // first iteration: `in` is divided by the albedo; last: `out` is multiplied by it
+};
+int launchAtrous(const AtrousParams &p, cudaStream_t stream);
 int launchInvSqrtCheck(uint32_t n, const float *x, float *fast, float *ieee, cudaStream_t stream); // debugging aid
 int launchTonemap(const float4 *accum, uchar4 *out, uint32_t pixels, float invSampleCount, cudaStream_t stream);
 int launchScale(const float4 *accum, float4 *out, uint32_t pixels, float scale, cudaStream_t stream);
