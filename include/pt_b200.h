@@ -65,7 +65,7 @@ typedef struct pt_camera_desc {
 
 /* counters of the last pt_render call (SURVEY.md §5 "Tracing"). */
 typedef struct pt_stats {
-	uint64_t samples;      /* paths started (= W*H*spp) */
+	uint64_t samples;      /* paths started (= W*H*spp; with option "adaptive" the sum of the pixels' sample counts) */
 	uint64_t rays;         /* closest-hit queries (camera + scattered segments, <=5 per sample) */
 	uint64_t node_visits;  /* BVH node box-pair tests (only counted when option "count_work" = 1) */
 	uint64_t prim_tests;   /* primitive intersection tests (idem) */
@@ -216,9 +216,32 @@ const float *pt_get_hdr_sum(pt_context *ctx);
  *                    picture, with less variance per sample in scenes lit by small emitters; one more ray per vertex.  A scene without
  *                    emitters renders as without the option.  Not combinable with "env_is" or the parity aids (pt_render returns
  *                    PT_E_INVALID).  Default 0 (trace.cu:136-151).
+ *  "adaptive"        tau > 0: adaptive sampling - the spp of pt_render / pt_render_vectors is the MAXIMUM, and a pixel stops at the
+ *                    first of its checkpoints c0 = min(m, spp), c_{j+1} = min(2 c_j, spp) where the standard error of the mean luminance
+ *                    (0.2126 r + 0.7152 g + 0.0722 b of each sample's path value) of its n samples of this call is small:
+ *                    sqrt(max(S2 - S1^2 / n, 0) / (n (n - 1))) <= tau x max(S1 / n, PT_ADAPTIVE_FLOOR), S1 = sum y, S2 = sum y^2.
+ *                    The pixel's sum of n samples is stored scaled by spp / n (not at all when n = spp), so the accumulation buffer
+ *                    holds mean x spp as without the option and every getter, progressive call, pt_denoise and the multi-GPU
+ *                    exchange work unchanged.  Each interval [c_j, c_{j+1}) is stratified on its own (option "stratify", decided from
+ *                    spp as without the option), so every checkpoint's samples are complete stratifications.  Stopping on the pixel's
+ *                    own samples biases slightly towards low-variance estimates (DESIGN.md has the measured size).  Combinable with
+ *                    "env_is" and "light_is"; "count_work" is ignored; pt_render returns PT_E_INVALID with the parity aids, with
+ *                    "variant" = 4 and with a multi-GPU sample partition.  pt_get_sample_counts gives the samples of each pixel,
+ *                    pt_get_stats the total.  0 (default): off, every pixel takes spp samples.  Not finite or < 0: PT_E_INVALID.
+ *                    No tau is recommended: measured on one B200 (DESIGN.md), no tau rendered a bundled scene with less error than
+ *                    uniform sampling in the same time
+ *  "adaptive_min_spp" m, the first checkpoint of option "adaptive" (default PT_ADAPTIVE_DEFAULT_MIN_SPP); < 32: PT_E_INVALID
  *  "tex_unit"        1 (default): texture taps through CUDA texture objects, as the reference (Pathtracer.cpp:259-288);
  *                    0: fp32 bilinear filter in software over the packed texels */
 int pt_set_option(pt_context *ctx, const char *key, double value);
+/* option "adaptive": the floor of the mean in the stopping test (pixels darker than this stop on an absolute error of tau x floor) and the
+ * default first checkpoint.  Of m in {64, 128, 256} the sweep of tools/adaptive_measure.py (DESIGN.md) had the least error at 256 on every
+ * scene; neither value is tuned further, since no setting beat uniform sampling at equal time */
+#define PT_ADAPTIVE_FLOOR (1.0f / 256.0f)
+#define PT_ADAPTIVE_DEFAULT_MIN_SPP 128
+/* After an adaptive pt_render (option "adaptive" > 0): the samples each pixel took in it, W*H values into a HOST buffer, bottom row first
+ * like the images (on a multi-GPU context the pixels of every device).  PT_E_INVALID when the last pt_render was not adaptive. */
+int pt_get_sample_counts(pt_context *ctx, uint32_t *counts);
 int pt_get_stats(const pt_context *ctx, pt_stats *out);
 
 /* Camera::rotate(pitch, yaw, roll) / Camera::translate(x, y, z)   Camera.h:10-11, Camera.inl:30-52 (the reference's

@@ -62,6 +62,7 @@ def load_library():
         "pt_get_denoised_hdr": (vp, [vp]),
         "pt_get_denoised_hdr_mean": (vp, [vp]),
         "pt_get_denoised_ldr": (vp, [vp]),
+        "pt_get_sample_counts": (i32, [vp, vp]),
         "pt_read_image": (i32, [cp, vp, vp, vp, vp]),
         "pt_free": (None, [vp]),
         "pt_last_error": (cp, []),
@@ -81,7 +82,8 @@ EXPORTS = ["pt_create", "pt_create_multi", "pt_get_multi_info", "pt_destroy", "p
            "pt_get_timing_ms", "pt_get_hdr", "pt_get_hdr_mean", "pt_get_hdr_sum", "pt_get_ldr", "pt_set_option", "pt_get_stats", "pt_camera_rotate", "pt_camera_translate", "pt_primary_pass",
            "pt_trace_rays", "pt_get_first_hit", "pt_accum_device_ptr", "pt_set_accum_device_ptr", "pt_load_scene_file", "pt_parse_scene_file",
            "pt_write_png", "pt_write_hdr", "pt_env_distribution", "pt_light_distribution", "pt_read_image", "pt_free", "pt_last_error", "pt_version",
-           "pt_render_aov", "pt_get_aov", "pt_denoise", "pt_get_denoised_hdr", "pt_get_denoised_hdr_mean", "pt_get_denoised_ldr"]
+           "pt_render_aov", "pt_get_aov", "pt_denoise", "pt_get_denoised_hdr", "pt_get_denoised_hdr_mean", "pt_get_denoised_ldr",
+           "pt_get_sample_counts"]
 
 AOV_ALBEDO, AOV_NORMAL, AOV_POSITION = 0, 1, 2  # PT_AOV_*
 AOV_KINDS = {"albedo": AOV_ALBEDO, "normal": AOV_NORMAL, "position": AOV_POSITION}
@@ -285,6 +287,12 @@ class Pathtracer:
         s = Stats()
         _check(self.L, self.L.pt_get_stats(self.h, C.byref(s)), "pt_get_stats")
         return s
+
+    def sampleCounts(self):
+        """(H, W) uint32: the samples each pixel took in the last render, which must have been adaptive (option "adaptive" > 0)"""
+        out = np.zeros((self.height, self.width), np.uint32)
+        _check(self.L, self.L.pt_get_sample_counts(self.h, _p(out)), "pt_get_sample_counts")
+        return out
 
     def primaryPass(self, camera):
         idx = np.zeros(self.width * self.height, np.int32)

@@ -7,6 +7,8 @@
 // pt_set_option "light_is"), --bvh sah|lbvh|auto, --denoise K (after the last launch: guide buffers of --aov-spp N camera rays per
 // pixel, default 16, and K iterations of the a-trous denoiser at its default sigmas; -o / -ohdr then write the denoised image), and for several GPUs of one box (the reference is fixed to device 0, Pathtracer.cpp:40):
 // --gpus N (devices 0..N-1) or --devices MASK, --partition pixels|samples, --exchange p2p|nccl (pt_create_multi).
+// --adaptive T [--adaptive-min N]: adaptive sampling (pt_set_option "adaptive" / "adaptive_min_spp"), -spp is then the maximum per pixel and
+// --stats reports the samples traced; not combinable with --slice (each launch would stop its pixels on its own samples).
 #include "../../include/pt_b200.h"
 #include <algorithm>
 #include <chrono>
@@ -38,6 +40,8 @@ struct Params // reference Params.h:4-14
 	int exchange = -1;           // -1 auto, 0 nccl, 1 p2p
 	int denoise = -1;            // >= 0: denoiser iterations (pt_denoise); -1: no denoiser
 	unsigned int aovSpp = 16;    // camera rays per pixel of the denoiser's guide buffers (pt_render_aov)
+	double adaptive = 0.0;       // > 0: option "adaptive"
+	unsigned int adaptiveMin = 0; // != 0: option "adaptive_min_spp"
 };
 
 static bool processArgs(int argc, char *argv[], Params &params)
@@ -85,6 +89,8 @@ static bool processArgs(int argc, char *argv[], Params &params)
 		else if (strcmp(a, "--stats") == 0) { params.stats = true; ++i; }
 		else if (strcmp(a, "--denoise") == 0 && i + 1 < argc) { params.denoise = atoi(argv[i + 1]); i += 2; }
 		else if (strcmp(a, "--aov-spp") == 0 && i + 1 < argc) { params.aovSpp = (unsigned int)atoi(argv[i + 1]); i += 2; }
+		else if (strcmp(a, "--adaptive") == 0 && i + 1 < argc) { params.adaptive = atof(argv[i + 1]); i += 2; }
+		else if (strcmp(a, "--adaptive-min") == 0 && i + 1 < argc) { params.adaptiveMin = (unsigned int)atoi(argv[i + 1]); i += 2; }
 		else
 		{
 			printf("Can't parse argument: %s\n", a);
@@ -168,6 +174,16 @@ int main(int argc, char *argv[])
 	if (params.envIS) pt_set_option(ctx, "env_is", 1.0);
 	if (params.lightIS) pt_set_option(ctx, "light_is", 1.0);
 	pt_set_option(ctx, "bvh_builder", (double)params.bvhBuilder);
+	if (params.adaptive != 0.0)
+	{
+		if (params.slice != 0)
+		{
+			fprintf(stderr, "--adaptive cannot be combined with --slice: each launch would stop its pixels on its own samples\n");
+			return EXIT_FAILURE;
+		}
+		if (pt_set_option(ctx, "adaptive", params.adaptive) != PT_OK) die("--adaptive");
+	}
+	if (params.adaptiveMin != 0 && pt_set_option(ctx, "adaptive_min_spp", (double)params.adaptiveMin) != PT_OK) die("--adaptive-min");
 
 	pt_camera_desc camera;
 	const int lr = pt_load_scene_file(ctx, params.m_inputFilepath, &camera);

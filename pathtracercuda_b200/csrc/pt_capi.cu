@@ -90,6 +90,12 @@ struct pt_context
 	DevBuf lightRecs;
 	uint32_t lightCount = 0;
 	DevBuf centreUV; // option "jitter" = 0: pixel-centre coordinates (RenderParams::centreU / centreV), made on first use
+	// option "adaptive": threshold tau (0 = off) and first checkpoint m; the samples each pixel took in the last pt_render (made on first
+	// use), valid when that render was adaptive
+	float adaptTau = 0.0f;
+	uint32_t adaptMinSpp = 128;
+	DevBuf sampleCounts;
+	bool countsValid = false;
 	// scene
 	DevBuf sceneBlob;
 	Mat *mats = nullptr; // (the material table at the end of sceneBlob)
@@ -546,6 +552,45 @@ static int ensureCentreTables(pt_context *c)
 	return PT_OK;
 }
 
+// the first-bounce stratification of `len` samples (RenderParams::strataPer): 2^k cells, k <= 8, at least 16 samples per cell - the lanes of
+// a pass of the one-pixel-per-warp kernel then hold samples of one or two neighbouring cells; fewer than 4 samples are not stratified
+static void strataRule(const LaunchConfig &cfg, uint32_t len, uint32_t &per, uint32_t &bitsA, uint32_t &bitsB, float &invPer)
+{
+	per = bitsA = bitsB = 0;
+	invPer = 0.0f;
+	if (len < 4u || len >= (1u << 21)) return;
+	uint32_t k = 2;
+	while (k < 8u && (len >> (k + 1u)) >= 16u) ++k; // measured at 4096 spp: 32 / 64 / 128 / 256 / 512 cells -> 489 / 479 / 470 / 465 / 468 ms
+	if (cfg.strataK > 0) k = uint32_t(cfg.strataK);  // (experiments: another cell count than the rule's)
+	while (k > 2u && (len >> k) == 0u) --k;
+	bitsA = (k + 1u) / 2u;
+	bitsB = k / 2u;
+	per = len >> k;
+	invPer = 1.0f / float(per);
+}
+
+// option "adaptive": the intervals of a pixel's samples, [0, c0), [c0, c1), ... with c0 = min(m, spp), c_{j+1} = min(2 c_j, spp), each
+// stratified on its own when the launch stratifies, and the constants of the stopping test and the scaling at their ends
+static void adaptIntervals(const LaunchConfig &cfg, uint32_t spp, uint32_t minSpp, bool stratify, RenderParams &p)
+{
+	uint32_t start = 0, end = minSpp < spp ? minSpp : spp, j = 0;
+	for (;; ++j)
+	{
+		AdaptInterval &iv = p.adapt[j];
+		iv.start = start;
+		iv.end = end;
+		if (stratify) strataRule(cfg, end - start, iv.strataPer, iv.strataBitsA, iv.strataBitsB, iv.strataInvPer);
+		else { iv.strataPer = iv.strataBitsA = iv.strataBitsB = 0; iv.strataInvPer = 0.0f; }
+		iv.invN = float(1.0 / double(end));
+		iv.invNN1 = end > 1u ? float(1.0 / (double(end) * double(end - 1u))) : 0.0f;
+		iv.scale = float(spp) / float(end); // (this file is compiled without FMA contraction: the IEEE quotient)
+		if (end == spp) break;
+		start = end;
+		end = end > spp / 2u ? spp : 2u * end;
+	}
+	p.adaptIntervals = j + 1u;
+}
+
 static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int ignore_history)
 {
 	PT_TRY
@@ -581,21 +626,22 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		philoxKeys(c->seed, p.philoxKeys);
 		p.maxBounces = c->maxBounces;
 		p.regenLow = c->launch.regenLow > 0 ? uint32_t(c->launch.regenLow) : 16u;
-		// first-bounce stratification (RenderParams::strataPer): 2^k cells, k <= 8, at least 16 samples per cell - the lanes of a
-		// pass of the one-pixel-per-warp kernel then hold samples of one or two neighbouring cells
-		const bool wantStrata = onePixelPerWarp(c->launch, spp) && (c->launch.stratify < 0 ? spp >= 128u : c->launch.stratify != 0) && spp >= 4u && spp < (1u << 21);
-		if (wantStrata)
-		{
-			uint32_t k = 2;
-			while (k < 8u && (spp >> (k + 1u)) >= 16u) ++k; // measured at 4096 spp: 32 / 64 / 128 / 256 / 512 cells -> 489 / 479 / 470 / 465 / 468 ms
-			if (c->launch.strataK > 0) k = uint32_t(c->launch.strataK); // (experiments: another cell count than the rule's)
-			while (k > 2u && (spp >> k) == 0u) --k;
-			p.strataBitsA = (k + 1u) / 2u;
-			p.strataBitsB = k / 2u;
-			p.strataPer = spp >> k;
-			p.strataInvPer = 1.0f / float(p.strataPer);
-		}
+		// first-bounce stratification (RenderParams::strataPer); option "adaptive" always runs the one-pixel-per-warp kernel
+		const bool adaptive = c->adaptTau > 0.0f;
+		const bool stratify = (adaptive || onePixelPerWarp(c->launch, spp)) && (c->launch.stratify < 0 ? spp >= 128u : c->launch.stratify != 0);
+		if (stratify) strataRule(c->launch, spp, p.strataPer, p.strataBitsA, p.strataBitsB, p.strataInvPer);
 		p.beam = c->launch.beam < 0 ? (spp >= 128u ? 1u : 0u) : uint32_t(c->launch.beam != 0);
+		c->launch.adaptive = adaptive;
+		if (adaptive)
+		{
+			if (c->noJitter || c->firstHit) return setError(PT_E_INVALID, "pt_render: adaptive and the parity aids (jitter = 0, first_hit = 1) cannot be combined");
+			if (c->launch.variant == 4) return setError(PT_E_INVALID, "pt_render: adaptive runs in the one-pixel-per-warp kernel only (variant 0 or 12, not 4)");
+			if (!c->sampleCounts.p) CK(c->sampleCounts.alloc(size_t(c->width) * c->height * sizeof(uint32_t)));
+			adaptIntervals(c->launch, spp, c->adaptMinSpp, stratify, p);
+			p.sampleCounts = c->sampleCounts.as<uint32_t>();
+			p.adaptTau = c->adaptTau;
+			p.adaptFloor = PT_ADAPTIVE_FLOOR;
+		}
 		p.alpha = c->alpha;
 		// which twin of the trace kernel runs: the options compiled into twins are exclusive
 		c->launch.twin = Twin::Plain;
@@ -641,6 +687,7 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		CK(cudaEventRecord(c->evStart, c->stream)); // (all allocations are behind us: the events bracket the device work alone)
 		// pixel partition: the pixels of the other ranks hold zeros, so that the sum over ranks is the image
 		if (ignore_history && c->pixelStride > 1u && !c->skipPartitionClear) CK(cudaMemsetAsync(c->accum, 0, size_t(c->width) * c->height * sizeof(float4), c->stream));
+		if (adaptive && c->pixelStride > 1u) CK(cudaMemsetAsync(c->sampleCounts.p, 0, size_t(c->width) * c->height * sizeof(uint32_t), c->stream)); // (the other ranks' pixels: 0)
 		launches = launchTrace(p, c->launch, c->stream, &usedSmem);
 		if (launches < 0) return setError(PT_E_CUDA, std::string("pt_render: kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()));
 	}
@@ -656,8 +703,9 @@ static int renderOne(pt_context *c, const CameraDev *camera, uint32_t spp, int i
 		{
 			const unsigned long long all = (unsigned long long)c->width * c->height;
 			const unsigned long long own = all > c->pixelOffset ? (all - c->pixelOffset + c->pixelStride - 1u) / c->pixelStride : 0ull;
-			c->stats.samples = own * spp;
+			c->stats.samples = c->launch.adaptive ? h[kCtrSamples] : own * spp;
 		}
+		c->countsValid = c->launch.adaptive;
 		memcpy(c->rawCounters, h, sizeof h);
 		c->stats.rays = h[kCtrRays];
 		c->stats.node_visits = h[kCtrNodes];
@@ -711,6 +759,8 @@ static int loadNccl(pt_context *c)
 // pixel, no collective at all - or by ONE ncclReduce of the float4 accumulation buffers (option "exchange").
 static int renderMulti(pt_context *c, const CameraDev *camera, uint32_t spp, int ignore_history)
 {
+	if (c->adaptTau > 0.0f && c->partition != 0)
+		return setError(PT_E_INVALID, "pt_render: adaptive and the multi-GPU sample partition cannot be combined (each device would stop a pixel on its own share of the samples)");
 	std::vector<pt_context *> all = { c };
 	all.insert(all.end(), c->peers.begin(), c->peers.end());
 	const uint32_t N = uint32_t(all.size());
@@ -1051,6 +1101,16 @@ static int setOptionOne(pt_context *c, const char *key, double value)
 	else if (k == "jitter") c->noJitter = value == 0;
 	else if (k == "env_is") c->envIS = value != 0;
 	else if (k == "light_is") c->lightIS = value != 0;
+	else if (k == "adaptive")
+	{
+		if (!(value >= 0.0) || !std::isfinite(value)) return setError(PT_E_INVALID, "pt_set_option: adaptive must be a finite threshold >= 0 (0 = off)");
+		c->adaptTau = float(value);
+	}
+	else if (k == "adaptive_min_spp")
+	{
+		if (!(value >= 32.0) || !(value <= 4294967295.0)) return setError(PT_E_INVALID, "pt_set_option: adaptive_min_spp must be at least 32");
+		c->adaptMinSpp = uint32_t(value);
+	}
 	else if (k == "first_hit")
 	{
 		if (value != 0 && !c->firstHitIndex.p)
@@ -1180,6 +1240,36 @@ int pt_get_first_hit(pt_context *c, int32_t *hit_index, float *hit_t)
 	CK(cudaMemcpyAsync(hit_t, c->firstHitT.p, px * 4, cudaMemcpyDeviceToHost, c->stream));
 	CK(cudaStreamSynchronize(c->stream));
 	return PT_OK;
+}
+
+int pt_get_sample_counts(pt_context *c, uint32_t *counts)
+{
+	PT_TRY
+	if (!c || !counts) return setError(PT_E_INVALID, "pt_get_sample_counts: bad arguments");
+	if (!c->countsValid) return setError(PT_E_INVALID, "pt_get_sample_counts: the last pt_render was not adaptive (option \"adaptive\" > 0)");
+	const size_t px = size_t(c->width) * c->height;
+	if (c->peers.empty())
+	{
+		CK(cudaSetDevice(c->device));
+		CK(cudaMemcpyAsync(counts, c->sampleCounts.p, px * 4, cudaMemcpyDeviceToHost, c->stream));
+		CK(cudaStreamSynchronize(c->stream));
+		return PT_OK;
+	}
+	// pixel partition: device i rendered the pixels i, i + N, ... and holds their counts in its own buffer
+	std::vector<pt_context *> all = { c };
+	all.insert(all.end(), c->peers.begin(), c->peers.end());
+	std::vector<uint32_t> part(px);
+	for (size_t i = 0; i < all.size(); ++i)
+	{
+		pt_context *d = all[i];
+		CK(cudaSetDevice(d->device));
+		CK(cudaMemcpyAsync(part.data(), d->sampleCounts.p, px * 4, cudaMemcpyDeviceToHost, d->stream));
+		CK(cudaStreamSynchronize(d->stream));
+		for (size_t q = i; q < px; q += all.size()) counts[q] = part[q];
+	}
+	CK(cudaSetDevice(c->device));
+	return PT_OK;
+	PT_CATCH(PT_E_LIMIT)
 }
 
 void *pt_accum_device_ptr(pt_context *c) { return c ? (void *)c->accum : nullptr; }

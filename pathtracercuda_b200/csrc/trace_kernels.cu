@@ -51,20 +51,39 @@ static __device__ __forceinline__ V3 baseColour(const SceneDev &scene, float4 m0
 
 // a contribution of a lane's path: the one-pixel-per-warp kernel (SHARE) adds it to the warp's partial sums of the pixel as it comes, the
 // one-pixel-per-lane kernel to the path's own sum L, which goes to the pixel's when the path ends (the two orders of the additions give
-// different bits)
-template <bool SHARE>
-static __device__ __forceinline__ void accumulate(V3 &color, V3 &L, V3 c)
+// different bits).  The contribution is a x b.  ADAPT: the one-pixel-per-warp kernel also sums the luminance of the path's contributions
+// (the luminance of the path's total, one register instead of three), for the stopping test of option "adaptive"; the weights are those of
+// env_sampling.cpp.  Its product is its own, never contracted (__fmul_rn): a product with two uses is not fused into the addition to
+// `color`, which would then round differently from the kernel without the option
+template <bool SHARE, bool ADAPT = false>
+static __device__ __forceinline__ void accumulate(V3 &color, V3 &L, float &y, V3 a, V3 b)
 {
-	if constexpr (SHARE) color = color + c;
-	else L = L + c;
+	if constexpr (SHARE) color = color + a * b;
+	else L = L + a * b;
+	if constexpr (ADAPT) y += 0.2126f * __fmul_rn(a.x, b.x) + 0.7152f * __fmul_rn(a.y, b.y) + 0.0722f * __fmul_rn(a.z, b.z);
+}
+
+// first-bounce stratification of the one-pixel-per-warp kernel (RenderParams::strataPer): the cell of the sample with local index m (m / per)
+// becomes the top bits of the two randoms of the first scattering direction, the Philox draw fills the bits below
+static __device__ __forceinline__ void stratify(uint32_t m, uint32_t per, uint32_t bitsA, uint32_t bitsB, float invPer, uint32_t &rz, uint32_t &rw)
+{
+	if (m < (per << (bitsA + bitsB)))
+	{
+		const uint32_t cell = __float2uint_rz((__uint2float_rn(m) + 0.5f) * invPer);
+		const uint32_t a = cell >> bitsB, bMask = (1u << bitsB) - 1u;
+		const uint32_t b = (a & 1u) ? bMask - (cell & bMask) : (cell & bMask); // snake: neighbouring cells are neighbouring directions
+		rz = (a << (32u - bitsA)) | (rz >> bitsA);
+		rw = (b << (32u - bitsB)) | (rw >> bitsB);
+	}
 }
 
 // ---------------------------------------------------------------------------------------------------------------
 // the trace kernel
 // ---------------------------------------------------------------------------------------------------------------
 // SMEM: the scene staged in shared memory; COUNT: work counters (option "count_work"); SHARE: one pixel per warp; SSTACK: the
-// traversal stack in shared memory; TWIN: the options compiled into an instantiation of their own (trace_kernels.h Twin)
-template <bool SMEM, bool COUNT, bool SHARE, bool SSTACK, Twin TWIN>
+// traversal stack in shared memory; TWIN: the options compiled into an instantiation of their own (trace_kernels.h Twin); ADAPT (SHARE only):
+// option "adaptive", a pixel's samples stop at the first checkpoint whose stopping test passes (RenderParams::adapt)
+template <bool SMEM, bool COUNT, bool SHARE, bool SSTACK, Twin TWIN, bool ADAPT = false>
 __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_constant__ RenderParams p)
 {
 	extern __shared__ __align__(128) float4 smemScene[];
@@ -116,6 +135,10 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 	uint32_t rays = 0, nodeVisits = 0, primTests = 0, shades = 0, misses = 0;
 	float lastPdf = 0.0f;   // EnvIS / LightIS: pdf with which the BSDF sampled the direction the lane is tracing (weights the sky at a miss, an emitter at a hit)
 	uint32_t wNext = p.spp; // SHARE: next sample of the warp's pixel to hand out (warp-uniform)
+	// ADAPT: the pixel's current interval (warp-uniform; it ends at the next checkpoint); the luminance y of the lane's path, the lane's sums
+	// of y and y^2
+	uint32_t ckIdx = 0;
+	float yPath = 0.0f, s1 = 0.0f, s2 = 0.0f;
 	unsigned long long passStat[6] = { 0, 0, 0, 0, 0, 0 }; // COUNT + SHARE (lane 0): camera passes, lanes, clocks; scattered passes, lanes, clocks
 	unsigned long long travClk[2] = { 0, 0 };               // COUNT + SHARE: clocks up to the end of the traversal, camera / scattered passes
 	const long long kernelT0 = COUNT && SHARE ? clock64() : 0;
@@ -138,7 +161,25 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				// rays of one group are nearly the same ray and stay in step through their first hit.  Everything here but the
 				// lane's own place in the group is warp-uniform: one vote per pass, the rest is arithmetic on its result
 				const uint32_t idle = uint32_t(__popc(needMask));
-				if (pixel != kInvalid && wNext < p.spp && (idle >= p.regenLow || needMask == 0xffffffffu || p.spp - wNext < 32u))
+				// (each form written out on its own here and at the stratification below: a shared statement moved the register allocation of
+				// the instantiations without ADAPT)
+				if constexpr (ADAPT)
+				{
+					// samples up to the pixel's next checkpoint
+					const uint32_t end = p.adapt[ckIdx].end;
+					if (pixel != kInvalid && wNext < end && (idle >= p.regenLow || needMask == 0xffffffffu || end - wNext < 32u))
+					{
+						nGen = min(idle, end - wNext);
+						const uint32_t place = __popc(needMask & ((1u << lane) - 1u));
+						if (!alive && place < nGen)
+						{
+							sample = wNext + place;
+							generate = true;
+						}
+						wNext += nGen;
+					}
+				}
+				else if (pixel != kInvalid && wNext < p.spp && (idle >= p.regenLow || needMask == 0xffffffffu || p.spp - wNext < 32u))
 				{
 					nGen = min(idle, p.spp - wNext);
 					const uint32_t place = __popc(needMask & ((1u << lane) - 1u));
@@ -154,6 +195,30 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 					// the pixel is complete: add the lanes' partial sums in a fixed order (butterfly), one lane writes
 					if (pixel != kInvalid)
 					{
+						if constexpr (ADAPT)
+						{
+							// a checkpoint below spp: the stopping test on copies of the lanes' sums (the lanes keep their own for the
+							// next checkpoint), warp-uniform.  var / n <= (tau x max(mean, floor))^2 is the test of the standard error
+							// without a square root; 1 / n and 1 / (n (n - 1)) come from the host
+							if (wNext < p.spp)
+							{
+								float a = s1, b = s2;
+#pragma unroll
+								for (int o = 16; o > 0; o >>= 1)
+								{
+									a += __shfl_xor_sync(0xffffffffu, a, o);
+									b += __shfl_xor_sync(0xffffffffu, b, o);
+								}
+								const AdaptInterval &iv = p.adapt[ckIdx];
+								const float se2 = fmaxf(b - a * a * iv.invN, 0.0f) * iv.invNN1;
+								const float bound = p.adaptTau * fmaxf(a * iv.invN, p.adaptFloor);
+								if (!(se2 <= bound * bound))
+								{
+									++ckIdx; // the same pixel: its beam list and pixelXY stay
+									continue;
+								}
+							}
+						}
 #pragma unroll
 						for (int o = 16; o > 0; o >>= 1)
 						{
@@ -161,9 +226,26 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							color.y += __shfl_xor_sync(0xffffffffu, color.y, o);
 							color.z += __shfl_xor_sync(0xffffffffu, color.z, o);
 						}
-						if (lane == 0) storePixel(p, pixel, color);
+						if constexpr (ADAPT)
+						{
+							// the sum of n samples scaled to spp (x spp / n, worked out by the host; not at all when n = spp): the
+							// accumulation buffer holds mean x spp, as without the option
+							if (lane == 0)
+							{
+								if (wNext != p.spp) color = p.adapt[ckIdx].scale * color;
+								storePixel(p, pixel, color);
+								p.sampleCounts[pixel] = wNext;
+								atomicAdd(&p.counters[kCtrSamples], (unsigned long long)wNext);
+							}
+						}
+						else if (lane == 0) storePixel(p, pixel, color);
 					}
 					color = mk(0.0f, 0.0f, 0.0f);
+					if constexpr (ADAPT)
+					{
+						s1 = s2 = 0.0f;
+						ckIdx = 0;
+					}
 					unsigned long long next = 0;
 					if (lane == 0) next = atomicAdd(&p.counters[kCtrWork], 1ull);
 					next = __shfl_sync(0xffffffffu, next, 0);
@@ -257,7 +339,13 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				{
 					// first-bounce stratification: the cell of this sample (its local index / samples per cell) becomes the top bits of
 					// the two randoms of the first scattering direction, the Philox draw fills the bits below (RenderParams::strataPer)
-					if (sample < (p.strataPer << (p.strataBitsA + p.strataBitsB)))
+					// (ADAPT: the sample's index within its interval, and the interval's own grid)
+					if constexpr (ADAPT)
+					{
+						const AdaptInterval &iv = p.adapt[ckIdx];
+						stratify(sample - iv.start, iv.strataPer, iv.strataBitsA, iv.strataBitsB, iv.strataInvPer, rz, rw);
+					}
+					else if (sample < (p.strataPer << (p.strataBitsA + p.strataBitsB)))
 					{
 						const uint32_t cell = __float2uint_rz((__uint2float_rn(sample) + 0.5f) * p.strataInvPer);
 						const uint32_t a = cell >> p.strataBitsB, bMask = (1u << p.strataBitsB) - 1u;
@@ -273,6 +361,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 				rd = cameraDir<2>(p.cam, u, v);
 				thr = mk(1.0f, 1.0f, 1.0f);
 				L = mk(0.0f, 0.0f, 0.0f);
+				if constexpr (ADAPT) yPath = 0.0f;
 				bounce = 0;
 				alive = true;
 			}
@@ -313,7 +402,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 						// (balance heuristic; the camera ray's miss has no such rival and keeps weight 1)
 						if (bounce != 0u) sky = balanceWeight(lastPdf, envPdf(p.scene.env, phi * (0.5f / PT_PI), theta * (1.0f / PT_PI), rd.y)) * sky;
 					}
-					accumulate<SHARE>(color, L, thr * sky);
+					accumulate<SHARE, ADAPT>(color, L, yPath, thr, sky);
 				}
 				terminate = true;
 			}
@@ -330,7 +419,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 					const uint32_t emitter = __float_as_uint(sv.ld(mp + 2).z);
 					if (bounce != 0u && emitter != 0u) emitted = balanceWeight(lastPdf, lightPdfHit<SMEM>(p.lights, sv, emitter - 1u, h.prim, ro, rd, h.t)) * emitted;
 				}
-				accumulate<SHARE>(color, L, thr * emitted);
+				accumulate<SHARE, ADAPT>(color, L, yPath, thr, emitted);
 				terminate = true;
 				// The last segment of a path only contributes what it hits: the direction the reference still samples there
 				// (trace.cu:139-151 in its fifth loop trip) is never traced and its weight never reaches the image - no normal,
@@ -381,7 +470,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							++rays;
 							uint32_t nv = 0, pt = 0;
 							const Hit hs = closestHitWW<SMEM, false, kHotExact, SSTACK, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr);
-							if (hs.prim < 0) accumulate<SHARE>(color, L, contrib);
+							if (hs.prim < 0) accumulate<SHARE, ADAPT>(color, L, yPath, contrib, mk(1.0f, 1.0f, 1.0f));
 						}
 					}
 					else if constexpr (TWIN == Twin::LightIS)
@@ -413,7 +502,7 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 							uint32_t nv = 0, pt = 0;
 							const Hit hs = closestHitWW<SMEM, false, kHotExact, SSTACK, true, true>(sv, s.p, wl, 0.001f, nv, pt, beamList[0], -1, stackColumn, nullptr,
 							                                                                      dist * (1.0f - 1e-4f));
-							if (hs.prim < 0) accumulate<SHARE>(color, L, contrib);
+							if (hs.prim < 0) accumulate<SHARE, ADAPT>(color, L, yPath, contrib, mk(1.0f, 1.0f, 1.0f));
 						}
 					}
 					else scattered = sampleMaterial(mtype, base, m0.w, m1.w, s.n, rd, rnd0, rnd1, wi, weight);
@@ -430,6 +519,11 @@ __global__ void __launch_bounds__(kTraceThreads, 1) traceKernel(const __grid_con
 			if (terminate)
 			{
 				if constexpr (!SHARE) color = color + L;
+				if constexpr (ADAPT)
+				{
+					s1 += yPath;
+					s2 += yPath * yPath;
+				}
 				++sample;
 				alive = false;
 			}
@@ -650,9 +744,29 @@ static int launchTraceKernel(const RenderParams &p, const LaunchConfig &cfg, boo
 	return launchKernel(smem ? traceKernel<true, false, SHARE, SSTACK, TWIN> : traceKernel<false, false, SHARE, SSTACK, TWIN>, p, cfg, smemBytes, stream);
 }
 
+// option "adaptive": the one-pixel-per-warp form without work counters, for the plain kernel and the env_is / light_is twins
+template <bool SSTACK, Twin TWIN>
+static int launchAdaptive(const RenderParams &p, const LaunchConfig &cfg, bool smem, size_t smemBytes, cudaStream_t stream)
+{
+	return launchKernel(smem ? traceKernel<true, false, true, SSTACK, TWIN, true> : traceKernel<false, false, true, SSTACK, TWIN, true>, p, cfg, smemBytes, stream);
+}
+
 template <bool SHARE, bool SSTACK>
 static int launchTwin(const RenderParams &p, const LaunchConfig &cfg, bool smem, size_t smemBytes, cudaStream_t stream)
 {
+	if constexpr (SHARE)
+	{
+		if (cfg.adaptive)
+		{
+			switch (cfg.twin)
+			{
+			case Twin::EnvIS: return launchAdaptive<SSTACK, Twin::EnvIS>(p, cfg, smem, smemBytes, stream);
+			case Twin::LightIS: return launchAdaptive<SSTACK, Twin::LightIS>(p, cfg, smem, smemBytes, stream);
+			case Twin::Plain: return launchAdaptive<SSTACK, Twin::Plain>(p, cfg, smem, smemBytes, stream);
+			default: return -1; // (pt_render refuses the parity aids with the option)
+			}
+		}
+	}
 	switch (cfg.twin)
 	{
 	case Twin::Aids: return launchTraceKernel<SHARE, SSTACK, Twin::Aids>(p, cfg, smem, smemBytes, stream);
@@ -667,7 +781,7 @@ int launchTrace(const RenderParams &pIn, const LaunchConfig &cfg, cudaStream_t s
 	RenderParams p = pIn;
 	const size_t sceneBytes = (size_t(p.scene.nodeCount) + p.scene.primCount) * 64 + size_t(p.scene.primCount) * sizeof(Mat); // nodes | primitives | materials
 	// one pixel per warp: camera passes and scattered passes alternate
-	const bool share = onePixelPerWarp(cfg, p.spp);
+	const bool share = cfg.adaptive || onePixelPerWarp(cfg, p.spp);
 	const size_t stackBytes = size_t(cfg.stackLevels) * kStackStride;
 	// what goes into shared memory: the scene when it fits (a scene larger than the opt-in limit stays in L2/HBM), the traversal
 	// stack when it fits beside it

@@ -8,6 +8,7 @@ namespace ptb
 
 // counters[] layout (device, unsigned long long)
 enum { kCtrWork = 0, kCtrRays = 1, kCtrNodes = 2, kCtrPrims = 3, kCtrShades = 4, kCtrMisses = 5,
+       kCtrSamples = 6, // option "adaptive": paths started, one atomic per pixel
        // pass statistics of the one-pixel-per-warp kernel (count_work = 1), 9 slots from kCtrPassStats: camera passes, their lanes,
        // their clocks; scattered passes, lanes, clocks; kernel clocks; traversal clocks of camera / scattered passes
        kCtrPassStats = 8, kCtrCount = 24 };
@@ -37,6 +38,19 @@ struct SceneDev
 	uint32_t treeNodeCount = 0; // nodes[treeNodeCount..nodeCount): boxes of the hoisted primitives, for the pixel-beam walk only
 	EnvDev env;                 // set (alias != nullptr) when the launch samples the sky directly (option "env_is")
 };
+
+// option "adaptive": one interval of a pixel's samples between two checkpoints, with its own first-bounce stratification
+// (RenderParams::strataPer; strataPer = 0: unstratified), and the constants of the stopping test and the scaling at its end n = `end`
+struct AdaptInterval
+{
+	uint32_t start, end;
+	uint32_t strataPer, strataBitsA, strataBitsB;
+	float strataInvPer;
+	float invN, invNN1; // 1 / n, 1 / (n (n - 1))
+	float scale;        // spp / n
+};
+// checkpoints m, 2m, 4m, ... from m >= 32 up to a 32-bit spp: at most 28
+constexpr uint32_t kAdaptMaxIntervals = 28;
 
 struct RenderParams
 {
@@ -74,6 +88,14 @@ struct RenderParams
 	// (launch parameters added from here on go at the END: the constant-bank offsets of the fields above stay where the existing
 	// kernels read them)
 	LightDev lights; // set (count != 0) when the launch samples the emitters directly (option "light_is")
+	// option "adaptive" (traceKernel<..., ADAPT = true>): a pixel's samples come in intervals [start, end) that end at its checkpoints
+	// min(m, spp), then doubling up to spp; at a checkpoint the pixel stops when the standard error of the luminance of its samples is at
+	// most adaptTau x max(mean, PT_ADAPTIVE_FLOOR).  Each interval is stratified on its own (strataPer ... as above, for the interval's
+	// length), so that every checkpoint's samples are complete stratifications
+	uint32_t *sampleCounts = nullptr; // the samples each pixel took
+	float adaptTau = 0.0f, adaptFloor = 0.0f; // (adaptFloor: PT_ADAPTIVE_FLOOR)
+	uint32_t adaptIntervals = 0;
+	AdaptInterval adapt[kAdaptMaxIntervals];
 };
 
 constexpr uint32_t kAidPixelCentre = 1u, kAidFirstHit = 2u;
@@ -119,6 +141,7 @@ struct LaunchConfig
 	int strataK = 0;     // experiments: log2 of the cell count (0 = the rule of pt_render: at least 32 samples per cell, at most 128 cells)
 	int smemStack = -1;  // traversal stack in shared memory (TravStack<true>): 1 on, 0 off, -1 = on when it fits beside the scene
 	Twin twin = Twin::Plain; // set by pt_render from the options (EnvIS: RenderParams::scene.env; LightIS: RenderParams::lights)
+	bool adaptive = false;   // set by pt_render from option "adaptive": the ADAPT instantiation of the one-pixel-per-warp kernel, whatever the spp
 	int stackLevels = 0; // BVH depth + 2: levels the shared-memory stack needs (set by pt_render from the compiled scene)
 	size_t maxSmemOptin = 0;
 };

@@ -30,8 +30,13 @@ def main():
     ap.add_argument("old")
     ap.add_argument("new")
     ap.add_argument("--match", default="traceKernel")
+    ap.add_argument("--rename", action="append", default=[], metavar="NEW=OLD",
+                    help="replace NEW by OLD in the new object's kernel names, e.g. when a template parameter with a default was added")
     a = ap.parse_args()
     old, new = kernels(a.old), kernels(a.new)
+    for r in a.rename:
+        frm, to = r.split("=", 1)
+        new = {k.replace(frm, to): v for k, v in new.items()}
     names = sorted(k for k in old if a.match in k and k in new)
     diff = [k for k in names if old[k] != new[k]]
     for k in names:
